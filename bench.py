@@ -13,6 +13,10 @@ reported under "also".  configs[1] (101 candidates) cannot occupy 148 SMs and co
 sweep; both are reported under "also".
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scaling strong|weak] [--workload cfg3|cfg2]
+                  [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step returned (every array of the `grid_posterior` result) as DIR/<name>.npy
+in float64.  The workload is seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -104,6 +108,14 @@ def cpu_sample_text(ns, M, cores):
             "thread, oracle = restated reference with Nelder-Mead g_tol=1e-6 (the reference's optimiser)" % (ns, M, cores))
 
 
+def dump_outputs(outdir, res):
+    """One .npy per array of a grid_posterior result; the integer counters (nfev, info) are widened to float64.  The cfg3
+    grid gives 11 doubles per candidate: 0.9 MB, 7 MB at 8-fold weak scaling."""
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in res.items():
+        np.save(os.path.join(outdir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 class ClockSampler:
     Q = "clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.hw_slowdown,clocks_event_reasons.hw_thermal_slowdown,clocks_event_reasons.sw_thermal_slowdown,clocks_event_reasons.sw_power_cap"
 
@@ -191,6 +203,8 @@ def run_single_process(args, out):
         t0 = time.perf_counter()
         res = problem.grid_posterior(delays, theta0, iterations=ITERATIONS, rhomin=RHOMIN, rhomax=RHOMAX)   # synchronous call
         times.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res)
     st = ctx.stats()
     ms = float(np.mean(times)) * 1e3
     line = {"metric": METRIC, "value": len(delays) / (ms * 1e-3), "unit": "candidates/s", "n_gpus": args.gpus, "steps": args.steps,
@@ -220,7 +234,10 @@ def main():
                     help="one process driving --gpus N devices through gpcc_ctx_create(ndev=N) (the layout a single Julia process uses) instead of one rank per GPU")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-also", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the library's timed step; --impl reference has none")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -322,6 +339,8 @@ def main():
         sampler.start()
     r = measure(delays, label)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, r["state"]["res"])      # every rank holds the full, all-gathered result
 
     # ---- roofline of the dominant kernel (persistent fit kernel = fused small-N evaluator), from the library's CUDA events ----
     N = int(sum(len(a) for a in t))
