@@ -52,16 +52,13 @@ int check_options(const gpcc_fit_options* o) {
     return 0;
 }
 
-// Evaluate `M` (delay, alpha, rho) triples that already sit in the pinned host mirrors of `s`.
-// Results land in s.ll.h / s.grad.h / s.info.h.
 }  // namespace
-int gpcc::launch_eval(gpcc_problem* p, int di, int slot, int M, int want_grad) {
+int gpcc::evaluate_on_device(gpcc_problem* p, int di, int M, int want_grad) {
     DeviceState& s = p->ctx->ds[di];
-    EvalSlot& q = s.slot[slot];
+    EvalSlot& q = s.slot;
     const int L = p->L;
     CUDA_TRY(cudaSetDevice(s.dev));
-    static const int one_stream = getenv("GPCC_ONE_STREAM") ? atoi(getenv("GPCC_ONE_STREAM")) : 0;
-    cudaStream_t stream = (slot == 1 && p->small_path && !one_stream) ? s.stream2 : s.stream;
+    cudaStream_t stream = s.stream;
     CUDA_TRY(cudaMemcpyAsync(q.delays.d, q.delays.h, (size_t)M * L * sizeof(double), cudaMemcpyHostToDevice, stream));
     CUDA_TRY(cudaMemcpyAsync(q.alpha.d, q.alpha.h, (size_t)M * L * sizeof(double), cudaMemcpyHostToDevice, stream));
     CUDA_TRY(cudaMemcpyAsync(q.rho.d, q.rho.h, (size_t)M * sizeof(double), cudaMemcpyHostToDevice, stream));
@@ -70,12 +67,10 @@ int gpcc::launch_eval(gpcc_problem* p, int di, int slot, int M, int want_grad) {
     b.ll = q.ll.d; b.grad = q.grad.d; b.info = q.info.d;
     b.h_delays = q.delays.h; b.h_alpha = q.alpha.h; b.h_rho = q.rho.h;
     const bool prof = p->ctx->profiling;
-    q.M = M; q.want_grad = want_grad; q.timed = false;
     if (p->small_path) {
-        if (prof) CUDA_TRY(cudaEventRecord(q.ev0, stream));
+        if (prof) CUDA_TRY(cudaEventRecord(s.ev0, stream));
         CUDA_TRY(small_sweep_launch(p->pd[di].dp, b, stream));
-        if (prof) CUDA_TRY(cudaEventRecord(q.ev1, stream));
-        q.timed = prof;
+        if (prof) CUDA_TRY(cudaEventRecord(s.ev1, stream));
         s.launches += 1;
     } else {
         LargeTimings lt;
@@ -91,38 +86,20 @@ int gpcc::launch_eval(gpcc_problem* p, int di, int slot, int M, int want_grad) {
     if (want_grad)
         CUDA_TRY(cudaMemcpyAsync(q.grad.h, q.grad.d, (size_t)M * (L + 1) * sizeof(double), cudaMemcpyDeviceToHost, stream));
     CUDA_TRY(cudaMemcpyAsync(q.info.h, q.info.d, (size_t)M * sizeof(int), cudaMemcpyDeviceToHost, stream));
-    CUDA_TRY(cudaEventRecord(q.done, stream));
-    return 0;
-}
-
-int gpcc::finish_eval(gpcc_problem* p, int di, int slot) {
-    DeviceState& s = p->ctx->ds[di];
-    EvalSlot& q = s.slot[slot];
-    CUDA_TRY(cudaSetDevice(s.dev));
-    CUDA_TRY(cudaEventSynchronize(q.done));
-    if (q.timed) {
-        // union of the launch intervals: the two slots run on two streams and overlap in their tails
-        float t0 = 0, t1 = 0;
-        CUDA_TRY(cudaEventElapsedTime(&t0, s.origin, q.ev0));
-        CUDA_TRY(cudaEventElapsedTime(&t1, s.origin, q.ev1));
-        const double from = std::max((double)t0, s.busy_end_ms);
-        if (t1 > from) s.ms_eval += t1 - from;
-        s.busy_end_ms = std::max(s.busy_end_ms, (double)t1);
+    CUDA_TRY(cudaStreamSynchronize(stream));
+    if (prof && p->small_path) {
+        float ms = 0;
+        CUDA_TRY(cudaEventElapsedTime(&ms, s.ev0, s.ev1));
+        s.ms_eval += ms;
     }
-    s.evals += q.M;
-    if (q.want_grad) s.evals_grad += q.M;
+    s.evals += M;
+    if (want_grad) s.evals_grad += M;
     return 0;
 }
 
-int gpcc::evaluate_on_device(gpcc_problem* p, int di, int M, int want_grad) {
-    int rc = launch_eval(p, di, 0, M, want_grad);
-    if (rc) return rc;
-    return finish_eval(p, di, 0);
-}
-
-int gpcc::reserve_eval(gpcc_problem* p, int di, size_t M, int slot) {
+int gpcc::reserve_eval(gpcc_problem* p, int di, size_t M) {
     DeviceState& s = p->ctx->ds[di];
-    EvalSlot& q = s.slot[slot];
+    EvalSlot& q = s.slot;
     const int L = p->L;
     CUDA_TRY(cudaSetDevice(s.dev));
     CUDA_TRY(q.delays.reserve(M * L));
@@ -139,14 +116,10 @@ void reset_stats(gpcc_ctx* ctx) {
     for (auto& s : ctx->ds) {
         s.ms_eval = s.ms_assembly = s.ms_factor = s.ms_gradreduce = 0;
         s.launches = s.evals = s.evals_grad = s.shared_prefix_evals = s.tau_cache_evals = s.assembly_bytes = 0;
-        if (s.origin) {   // new time zero (float milliseconds lose resolution far from the origin)
-            cudaSetDevice(s.dev);
-            cudaStreamSynchronize(s.stream);
-            cudaStreamSynchronize(s.stream2);
-            cudaEventRecord(s.origin, s.stream);
-            cudaEventSynchronize(s.origin);
-            s.busy_end_ms = 0;
-        }
+        // the call about to start refills the pinned staging buffers: wait for what may still read them (a call that
+        // failed midway, or the all-gather of posterior_on_devices, which synchronises device 0 only)
+        cudaSetDevice(s.dev);
+        cudaStreamSynchronize(s.stream);
     }
 }
 
@@ -245,8 +218,7 @@ int fit_shard_device(gpcc_problem* p, int di, const std::vector<int>& idx, const
             for (int l = 1; l < L; ++l) { lo = std::min(lo, dl[l]); hi = std::max(hi, dl[l]); }
             key[c] = {-(hi - lo), c};
         }
-        static const bool grid_order = getenv("GPCC_FIT_GRID_ORDER") != nullptr;      // A/B switch
-        if (!grid_order) std::stable_sort(key.begin(), key.end(), [](const std::pair<double, int>& a, const std::pair<double, int>& b) { return a.first < b.first; });
+        std::stable_sort(key.begin(), key.end(), [](const std::pair<double, int>& a, const std::pair<double, int>& b) { return a.first < b.first; });
         for (int c = 0; c < m; ++c) s.fit_order.h[c] = key[c].second;
     }
     for (int k = 0; k < 8; ++k) s.fit_counters.h[k] = 0;
@@ -261,16 +233,14 @@ int fit_shard_device(gpcc_problem* p, int di, const std::vector<int>& idx, const
     fp.rhomin = o.rhomin; fp.rhomax = o.rhomax; fp.alpha_floor = o.alpha_floor; fp.gtol = o.gtol; fp.ftol = o.ftol;
     fp.history = o.history;
     fp.optimizer = o.optimizer; fp.nm_gtol = o.nm_gtol;
-    static const bool screen_full = getenv("GPCC_SCREEN_FULL") != nullptr;     // experiment switch: screen with gradient evaluations
-    fp.screen_forward = screen_full ? 0 : 1;
     FitBuffers fb;
     fb.delays = s.fit_delays.d; fb.theta0 = s.fit_theta0.d; fb.ll = s.fit_ll.d; fb.theta = s.fit_theta.d;
     fb.iters = s.fit_iters.d; fb.nfev = s.fit_nfev.d; fb.status = s.fit_status.d; fb.counters = s.fit_counters.d;
     fb.order = s.fit_order.d;
     const bool prof = p->ctx->profiling;
-    if (prof) CUDA_TRY(cudaEventRecord(s.fit_ev0, st));
+    if (prof) CUDA_TRY(cudaEventRecord(s.ev0, st));
     CUDA_TRY(small_fit_launch(p->pd[di].dp, fp, fb, st));
-    if (prof) CUDA_TRY(cudaEventRecord(s.fit_ev1, st));
+    if (prof) CUDA_TRY(cudaEventRecord(s.ev1, st));
     CUDA_TRY(cudaMemcpyAsync(s.fit_ll.h, s.fit_ll.d, (size_t)m * sizeof(double), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaMemcpyAsync(s.fit_theta.h, s.fit_theta.d, (size_t)m * n * sizeof(double), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaMemcpyAsync(s.fit_iters.h, s.fit_iters.d, (size_t)m * sizeof(int), cudaMemcpyDeviceToHost, st));
@@ -280,7 +250,7 @@ int fit_shard_device(gpcc_problem* p, int di, const std::vector<int>& idx, const
     CUDA_TRY(cudaStreamSynchronize(st));
     if (prof) {
         float ms = 0;
-        CUDA_TRY(cudaEventElapsedTime(&ms, s.fit_ev0, s.fit_ev1));
+        CUDA_TRY(cudaEventElapsedTime(&ms, s.ev0, s.ev1));
         s.ms_eval += ms;
     }
     static const bool debug = getenv("GPCC_FIT_DEBUG") != nullptr;
@@ -302,29 +272,47 @@ int fit_shard_device(gpcc_problem* p, int di, const std::vector<int>& idx, const
     return 0;
 }
 
-// Candidates idx[0..n) (global indices) are fitted on device `di`.
+// Candidates idx[0..n) (global indices) are fitted on device `di`.  The host-driven batched L-BFGS below is the driver of
+// the tiled path; on the fused small-N path it runs only under GPCC_FIT_HOST=1, as the reference that the persistent fit
+// kernel is tested against.
 int fit_shard(gpcc_problem* p, int di, const std::vector<int>& idx, const double* delays, int P, const double* theta0,
               const gpcc_fit_options& o, const FitOutputs& out) {
     const int L = p->L, n = L + 1;
     const int m = (int)idx.size();
     if (m == 0) return 0;
-    static const bool host_loop = getenv("GPCC_FIT_HOST") != nullptr;          // A/B switch: host-driven batched L-BFGS on the small path
+    static const bool host_loop = getenv("GPCC_FIT_HOST") != nullptr;
     if (p->small_path && (!host_loop || o.optimizer == GPCC_OPT_NELDERMEAD)) return fit_shard_device(p, di, idx, delays, P, theta0, o, out);
     if (o.optimizer == GPCC_OPT_NELDERMEAD)
         return fail(-7, "the Nelder-Mead option runs on the fused small-N path only (N <= 199); use the default L-BFGS");
-    DeviceState& s = p->ctx->ds[di];
-    EvalSlot& q0 = s.slot[0];
+    EvalSlot& q = p->ctx->ds[di].slot;
     LbfgsOptions lo;
     lo.max_iter = o.max_iter; lo.gtol = o.gtol; lo.ftol = o.ftol; lo.history = o.history; lo.n_scale = L;
-    static const double dec_env = getenv("GPCC_LBFGS_DEC") ? atof(getenv("GPCC_LBFGS_DEC")) : 0.0;   // experiment switch
-    lo.dec_tol = dec_env;
 
     std::vector<LbfgsState> st(m);
-    // ---- stage 1: screening of the P start points (:207-209), batched over all candidates -----------
     std::vector<double> jac(n);
-    // screening results of the candidates `cand` (evaluations cand-major, P per candidate, in slot q) -> L-BFGS start
-    auto screen_pack = [&](EvalSlot& q, const int* cand, size_t nc) {
-        for (size_t a = 0; a < nc; ++a) {
+    // ---- stage 1: screening of the P start points (:207-209), batched over all candidates -----------
+    const int screen_grad = o.max_iter > 0 ? 1 : 0;      // iterations = 0: the fixed-theta sweep, forward-only evaluations
+    // chunked so that one batch never exceeds ~1M evaluations worth of staging
+    const size_t chunk_c = std::max<size_t>(1, std::min<size_t>(m, (size_t)(1 << 18) / std::max(1, P)));
+    int rc = reserve_eval(p, di, chunk_c * P);
+    if (rc) return rc;
+    std::vector<int> seq(m);
+    for (int c = 0; c < m; ++c) seq[c] = c;
+    if (!p->small_path && o.max_iter <= 0 && !o.theta0_per_candidate && L >= 2) {
+        // fixed-theta sweep on the tiled path (forward-only evaluations): candidates that share the delays of all bands but
+        // the last become neighbours, so that a wave factorises their common leading block once (large_path.cu)
+        std::stable_sort(seq.begin(), seq.end(), [&](int x, int y) {
+            const double* dx = delays + (size_t)idx[x] * L;
+            const double* dy = delays + (size_t)idx[y] * L;
+            bool dec;
+            for (int l = 0; l + 1 < L; ++l) { const bool lt = bits_less(dx[l], dy[l], dec); if (dec) return lt; }
+            return false;
+        });
+    }
+    for (size_t c0 = 0; c0 < (size_t)m; c0 += chunk_c) {
+        const int* cand = seq.data() + c0;
+        const size_t nc = std::min<size_t>(m, c0 + chunk_c) - c0;
+        for (size_t a = 0; a < nc; ++a) {              // evaluations cand-major, P per candidate
             const int gi = idx[cand[a]];
             for (int j = 0; j < P; ++j) {
                 const size_t e = a * P + j;
@@ -333,8 +321,8 @@ int fit_shard(gpcc_problem* p, int di, const std::vector<int>& idx, const double
                 unpack_theta(th, L, o, q.alpha.h + e * L, q.rho.h + e, nullptr);
             }
         }
-    };
-    auto screen_feed = [&](EvalSlot& q, const int* cand, size_t nc) {
+        rc = evaluate_on_device(p, di, (int)(nc * P), screen_grad);
+        if (rc) return rc;
         for (size_t a = 0; a < nc; ++a) {
             const int c = cand[a], gi = idx[c];
             int best = -1;
@@ -360,129 +348,34 @@ int fit_shard(gpcc_problem* p, int di, const std::vector<int>& idx, const double
             for (int k = 0; k < n; ++k) g_[k] = -q.grad.h[e * n + k] * jac[k];
             S.start(n, th, bestf, g_, lo);
         }
-    };
-    // Fewer active candidates than this: one batch per round instead of two half batches.  Default 2, i.e. the halves
-    // always alternate: with one stream per slot the two small kernels of a latency-bound round overlap on the GPU
-    // (measured: 176-178 ms per fitted cfg3 grid against 179-181 with the threshold at 1024, cfg2 4.3 against 4.6 ms).
-    static const size_t MERGE_BELOW = getenv("GPCC_MERGE_BELOW") ? std::max<size_t>(2, (size_t)atol(getenv("GPCC_MERGE_BELOW"))) : 2;
-    // Fused small-N path with enough candidates: the two halves of stage 2 are formed before the screening, each half is
-    // screened on its own slot / stream, and the first L-BFGS batch of half 0 is packed and launched while the screening of
-    // half 1 still runs (no idle GPU between the stages, host bookkeeping hidden).
-    const bool pipelined = p->small_path && (size_t)m >= MERGE_BELOW && (size_t)m * P <= ((size_t)1 << 18);
-    int rc = 0;
-    const int screen_grad = o.max_iter > 0 ? 1 : 0;      // iterations = 0: the fixed-theta sweep, forward-only evaluations
-    std::vector<int> half[2];
-    if (pipelined) {
-        for (int c = 0; c < m; ++c) half[c & 1].push_back(c);
-        rc = reserve_eval(p, di, std::max(half[0].size() * P, (size_t)m), 0);
-        if (rc) return rc;
-        rc = reserve_eval(p, di, half[1].size() * P, 1);
-        if (rc) return rc;
-        for (int g = 0; g < 2; ++g) {
-            screen_pack(s.slot[g], half[g].data(), half[g].size());
-            rc = launch_eval(p, di, g, (int)(half[g].size() * P), screen_grad);
-            if (rc) return rc;
-        }
-    } else {
-        // chunked so that one batch never exceeds ~1M evaluations worth of staging
-        const size_t chunk_c = std::max<size_t>(1, std::min<size_t>(m, (size_t)(1 << 18) / std::max(1, P)));
-        rc = reserve_eval(p, di, chunk_c * P);
-        if (rc) return rc;
-        std::vector<int> seq(m);
-        for (int c = 0; c < m; ++c) seq[c] = c;
-        if (!p->small_path && o.max_iter <= 0 && !o.theta0_per_candidate && L >= 2) {
-            // fixed-theta sweep on the tiled path (forward-only evaluations): candidates that share the delays of all bands but
-            // the last become neighbours, so that a wave factorises their common leading block once (large_path.cu)
-            std::stable_sort(seq.begin(), seq.end(), [&](int x, int y) {
-                const double* dx = delays + (size_t)idx[x] * L;
-                const double* dy = delays + (size_t)idx[y] * L;
-                bool dec;
-                for (int l = 0; l + 1 < L; ++l) { const bool lt = bits_less(dx[l], dy[l], dec); if (dec) return lt; }
-                return false;
-            });
-        }
-        for (size_t c0 = 0; c0 < (size_t)m; c0 += chunk_c) {
-            const size_t c1 = std::min<size_t>(m, c0 + chunk_c);
-            screen_pack(q0, seq.data() + c0, c1 - c0);
-            rc = evaluate_on_device(p, di, (int)((c1 - c0) * P), screen_grad);
-            if (rc) return rc;
-            screen_feed(q0, seq.data() + c0, c1 - c0);
-        }
     }
-    // ---- stage 2: batched L-BFGS, software-pipelined over two halves of the candidates -------------------------
-    // While the kernel of one half runs, the host feeds the results of the other half to its L-BFGS state machines
-    // and packs that half's next trial points (the fused small-N path only; one slot for the tiled path, whose
-    // workspace is shared and whose host share is negligible).
-    int G = (p->small_path && (size_t)m >= MERGE_BELOW) ? 2 : 1;
-    std::vector<int> active[2];
-    if (!pipelined)
-        for (int c = 0; c < m; ++c)
-            if (st[c].status == LbfgsState::RUNNING) active[G == 2 ? (c & 1) : 0].push_back(c);
-    bool launched[2] = {false, false};
-    auto pack_and_launch = [&](int g) -> int {
-        EvalSlot& q = s.slot[g];
-        const int na = (int)active[g].size();
+    // ---- stage 2: batched L-BFGS, one evaluation of every running candidate per round -----------------------
+    std::vector<int> active;
+    for (int c = 0; c < m; ++c)
+        if (st[c].status == LbfgsState::RUNNING) active.push_back(c);
+    rc = reserve_eval(p, di, active.size());
+    if (rc) return rc;
+    while (!active.empty()) {
+        const int na = (int)active.size();
         for (int a = 0; a < na; ++a) {
-            const int c = active[g][a];
+            const int c = active[a];
             std::memcpy(q.delays.h + (size_t)a * L, delays + (size_t)idx[c] * L, L * sizeof(double));
             unpack_theta(st[c].xt, L, o, q.alpha.h + (size_t)a * L, q.rho.h + a, nullptr);
         }
-        launched[g] = true;
-        return launch_eval(p, di, g, na, 1);
-    };
-    auto finish_and_feed = [&](int g) -> int {
-        int r = finish_eval(p, di, g);
-        if (r) return r;
-        launched[g] = false;
-        EvalSlot& q = s.slot[g];
-        const int na = (int)active[g].size();
+        rc = evaluate_on_device(p, di, na, 1);
+        if (rc) return rc;
         size_t w = 0;
         for (int a = 0; a < na; ++a) {
-            const int c = active[g][a];
+            const int c = active[a];
             LbfgsState& S = st[c];
             double a_[LBFGS_MAXN], r_, g_[LBFGS_MAXN];
             unpack_theta(S.xt, L, o, a_, &r_, jac.data());
             const bool ok = q.info.h[a] == 0 && std::isfinite(q.ll.h[a]);
             for (int k = 0; k < n; ++k) g_[k] = ok ? -q.grad.h[(size_t)a * n + k] * jac[k] : 0.0;
             S.feed(ok, -q.ll.h[a], g_, lo);
-            if (S.status == LbfgsState::RUNNING) active[g][w++] = c;
+            if (S.status == LbfgsState::RUNNING) active[w++] = c;
         }
-        active[g].resize(w);
-        return 0;
-    };
-    if (pipelined) {
-        for (int g = 0; g < 2; ++g) {
-            rc = finish_eval(p, di, g);
-            if (rc) return rc;
-            screen_feed(s.slot[g], half[g].data(), half[g].size());
-            for (int c : half[g])
-                if (st[c].status == LbfgsState::RUNNING) active[g].push_back(c);
-            if (!active[g].empty()) { rc = pack_and_launch(g); if (rc) return rc; }
-        }
-    } else {
-        rc = reserve_eval(p, di, active[0].size() + active[1].size(), 0);
-        if (rc) return rc;
-        rc = reserve_eval(p, di, active[1].size(), 1);
-        if (rc) return rc;
-        for (int g = 0; g < G; ++g)
-            if (!active[g].empty()) { rc = pack_and_launch(g); if (rc) return rc; }
-    }
-    while (launched[0] || launched[1]) {
-        for (int g = 0; g < G; ++g) {
-            if (!launched[g]) continue;
-            rc = finish_and_feed(g);
-            if (rc) return rc;
-            if (G == 2 && active[0].size() + active[1].size() < MERGE_BELOW) {
-                const int h = 1 - g;                      // drain the other half, then continue with one batch per round
-                if (launched[h]) { rc = finish_and_feed(h); if (rc) return rc; }
-                active[0].insert(active[0].end(), active[1].begin(), active[1].end());
-                active[1].clear();
-                G = 1;
-                if (!active[0].empty()) { rc = pack_and_launch(0); if (rc) return rc; }
-                break;
-            }
-            if (!active[g].empty()) { rc = pack_and_launch(g); if (rc) return rc; }
-        }
+        active.resize(w);
     }
     // ---- outputs ------------------------------------------------------------------------------------------
     for (int c = 0; c < m; ++c) write_fit_outputs(p, o, out, idx[c], st[c].f, st[c].x, st[c].iters, st[c].nfev, st[c].status);
@@ -570,17 +463,8 @@ int gpcc_ctx_create(int ndev, const int* dev_ids, gpcc_ctx** out) {
         int prio_lo = 0, prio_hi = 0;
         CUDA_TRY(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
         CUDA_TRY(cudaStreamCreateWithPriority(&s.stream, cudaStreamNonBlocking, prio_hi));
-        CUDA_TRY(cudaStreamCreateWithPriority(&s.stream2, cudaStreamNonBlocking, prio_hi));
-        CUDA_TRY(cudaEventCreate(&s.fit_ev0));
-        CUDA_TRY(cudaEventCreate(&s.fit_ev1));
-        CUDA_TRY(cudaEventCreate(&s.origin));
-        CUDA_TRY(cudaEventRecord(s.origin, s.stream));
-        CUDA_TRY(cudaEventSynchronize(s.origin));
-        for (auto& q : s.slot) {
-            CUDA_TRY(cudaEventCreate(&q.ev0));
-            CUDA_TRY(cudaEventCreate(&q.ev1));
-            CUDA_TRY(cudaEventCreateWithFlags(&q.done, cudaEventDisableTiming));
-        }
+        CUDA_TRY(cudaEventCreate(&s.ev0));
+        CUDA_TRY(cudaEventCreate(&s.ev1));
     }
     *out = ctx;
     return 0;
@@ -591,22 +475,16 @@ int gpcc_ctx_destroy(gpcc_ctx* ctx) {
     if (ctx->nccl) nccl_bridge_destroy(ctx->nccl);
     for (auto& s : ctx->ds) {
         cudaSetDevice(s.dev);
-        for (auto& q : s.slot) {
-            s.post_ll.release(); s.post_prior.release(); s.post_out.release();
-            s.gat_send.release(); s.gat_recv.release(); s.gat_post.release();
-            q.delays.release(); q.alpha.release(); q.rho.release(); q.ll.release(); q.grad.release(); q.info.release();
-            if (q.ev0) cudaEventDestroy(q.ev0);
-            if (q.ev1) cudaEventDestroy(q.ev1);
-            if (q.done) cudaEventDestroy(q.done);
-        }
+        EvalSlot& q = s.slot;
+        q.delays.release(); q.alpha.release(); q.rho.release(); q.ll.release(); q.grad.release(); q.info.release();
+        s.post_ll.release(); s.post_prior.release(); s.post_out.release();
+        s.gat_send.release(); s.gat_recv.release(); s.gat_post.release();
         s.fit_delays.release(); s.fit_theta0.release(); s.fit_ll.release(); s.fit_theta.release();
         s.fit_iters.release(); s.fit_nfev.release(); s.fit_status.release(); s.fit_counters.release(); s.fit_order.release();
-        if (s.fit_ev0) cudaEventDestroy(s.fit_ev0);
-        if (s.fit_ev1) cudaEventDestroy(s.fit_ev1);
+        if (s.ev0) cudaEventDestroy(s.ev0);
+        if (s.ev1) cudaEventDestroy(s.ev1);
         large_workspace_release(s.large);
         if (s.stream) cudaStreamDestroy(s.stream);
-        if (s.stream2) cudaStreamDestroy(s.stream2);
-        if (s.origin) cudaEventDestroy(s.origin);
     }
     delete ctx;
     return 0;
@@ -742,7 +620,7 @@ static int loglik_batch_impl(gpcc_problem* p, int M, const double* delays, const
     const int nd = (int)ctx->ds.size();
     const size_t chunk = 1 << 18;
     int rc = for_each_device(ctx, [&](int di) -> int {
-        EvalSlot& s = ctx->ds[di].slot[0];
+        EvalSlot& s = ctx->ds[di].slot;
         std::vector<int> mine;
         for (int m = di; m < M; m += nd) mine.push_back(m);
         if (!p->small_path && !want_grad && !theta && L >= 2) {

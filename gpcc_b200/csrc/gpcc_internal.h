@@ -59,7 +59,6 @@ struct FitParams {            // keyword arguments / constants of gpcc (gpccfixd
     int history = 8;
     int optimizer = 0;        // 0: L-BFGS on the analytic gradient; 1: Nelder-Mead (nm.h), forward-only evaluations
     double nm_gtol = 1e-6;    // Optim.Options(g_tol = 1e-6) (:205)
-    int screen_forward = 1;   // 1: screen with forward-only evaluations (N^3/3) and evaluate the gradient at the winner only
 };
 struct FitBuffers {           // all on the device
     const double* delays = nullptr;   // [M][L]

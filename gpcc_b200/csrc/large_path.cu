@@ -123,8 +123,8 @@ __device__ __forceinline__ void dmma(double& c0, double& c1, double a, double b)
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// 128x128x128 DMMA main loop shared by the panel and update kernels.
-// acc += sign * A B',  A and B are 128x128 panel-layout blocks in global memory (contiguous 16 KB per K slice).
+// 128x128x128 DMMA main loop of the panel kernel.
+// acc += A B',  A and B are 128x128 panel-layout blocks in global memory (contiguous 16 KB per K slice).
 // 8 warps; warp w owns rows 32*(w&3).., cols 64*(w>>2)..  -> acc[4][8][2] per lane.
 // ---------------------------------------------------------------------------------------------------------------
 struct GemmSmem {
@@ -134,7 +134,7 @@ struct GemmSmem {
 };
 
 __device__ __forceinline__ void gemm_mainloop(GemmSmem& sm, const double* __restrict__ gA, const double* __restrict__ gB,
-                                              double (&acc)[4][8][2], bool negate) {
+                                              double (&acc)[4][8][2]) {
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int ro0 = (warp & 3) * 4, co0 = (warp >> 2) * 8;
     if (tid == 0) {
@@ -159,10 +159,7 @@ __device__ __forceinline__ void gemm_mainloop(GemmSmem& sm, const double* __rest
         for (int k4 = 0; k4 < KCH / 4; ++k4) {
             double a[4], b[8];
 #pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                a[i] = sa[((k4 * 16 + ro0 + i) << 5) + lane];
-                if (negate) a[i] = -a[i];
-            }
+            for (int i = 0; i < 4; ++i) a[i] = sa[((k4 * 16 + ro0 + i) << 5) + lane];
 #pragma unroll
             for (int j = 0; j < 8; ++j) b[j] = sb[((k4 * 16 + co0 + j) << 5) + lane];
 #pragma unroll
@@ -622,7 +619,7 @@ __global__ void __launch_bounds__(256, 1) panel_kernel(LargeArgs a, int k, int I
     for (int i = 0; i < 4; ++i)
 #pragma unroll
         for (int j = 0; j < 8; ++j) acc[i][j][0] = acc[i][j][1] = 0.0;
-    gemm_mainloop(sm, gA, gB, acc, false);
+    gemm_mainloop(sm, gA, gB, acc);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int ro0 = (warp & 3) * 4, co0 = (warp >> 2) * 8;
     double* mat = a.mats + (size_t)m * a.mat_stride;
@@ -708,7 +705,7 @@ __device__ __forceinline__ void update_tile_of(const LargeArgs& a, int k, int ph
     }
 }
 
-// half-tile form (default): blockIdx.x = 2 * tile + column half
+// one 4-warp CTA per column half of a tile (GemmSmemHalf): blockIdx.x = 2 * tile + column half
 __global__ void __launch_bounds__(128, 3) update_half_kernel(LargeArgs a, int k, int phase) {
     extern __shared__ __align__(128) unsigned char smraw[];
     GemmSmemHalf& sm = *reinterpret_cast<GemmSmemHalf*>(smraw);
@@ -736,42 +733,6 @@ __global__ void __launch_bounds__(128, 3) update_half_kernel(LargeArgs a, int k,
             acc[i][j][1] = v.y;
         }
     gemm_mainloop_half(sm, gA, gB, h, acc);
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 8; ++j)
-            *reinterpret_cast<double2*>(tile + (((ro0 + i) * 16 + co0 + j) << 6) + 2 * lane) = make_double2(acc[i][j][0], acc[i][j][1]);
-}
-
-__global__ void __launch_bounds__(256, 1) update_kernel(LargeArgs a, int k, int phase) {
-    extern __shared__ __align__(128) unsigned char smraw[];
-    GemmSmem& sm = *reinterpret_cast<GemmSmem*>(smraw);
-    const int m = blockIdx.y;
-    const int T = a.T;
-    int I, J;
-    update_tile_of(a, k, phase, blockIdx.x, I, J);
-    (void)T;
-    if (a.Tp && m > 0 && I < a.Tp) return;         // tile of the shared prefix (J <= I < Tp): updated once, in matrix 0
-    if (cache_skips_row(a, k, J) || (a.cmode == 1 && I >= a.Tq && I < a.Tc)) return;
-    const bool cached = a.cmode == 2 && k < a.Tq && I >= a.Tc;   // last band, pivot in band 1: only block (3,2) is updated,
-    if (cached && J < a.Tq) return;                              // with the cached panel of the last band
-    const int mB = (a.Tp && k < a.Tp && J < a.Tp) ? 0 : m;   // panel rows inside the shared prefix exist in matrix 0 only
-    const double* xw = a.Xws + (size_t)(k & 1) * a.x_parity_stride;
-    const double* gA = cached ? xc_tile(a, m, k, I) : xw + ((size_t)m * a.T + I) * TILE_ELEMS;
-    const double* gB = xw + ((size_t)mB * a.T + J) * TILE_ELEMS;
-    double* tile = a.mats + (size_t)m * a.mat_stride + tile_index(I, J) * TILE_ELEMS;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int ro0 = (warp & 3) * 4, co0 = (warp >> 2) * 8;
-    double acc[4][8][2];
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {      // acc = C (coalesced 512 B per warp per micro tile); overlaps the pipeline fill
-            const double2 v = *reinterpret_cast<const double2*>(tile + (((ro0 + i) * 16 + co0 + j) << 6) + 2 * lane);
-            acc[i][j][0] = v.x;
-            acc[i][j][1] = v.y;
-        }
-    gemm_mainloop(sm, gA, gB, acc, true);
 #pragma unroll
     for (int i = 0; i < 4; ++i)
 #pragma unroll
@@ -1094,16 +1055,13 @@ cudaError_t run_wave(const DevProblem& p, const EvalBatch& b, int e0, int nb, in
     const size_t pivot_smem = (size_t)(BT * PLD + 3 * BT + 112 * 17 + 16 * 17) * sizeof(double);
     if (!w.attr_set) {
         cudaFuncSetAttribute(panel_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gemm_smem);
-        cudaFuncSetAttribute(update_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gemm_smem);
         cudaFuncSetAttribute(update_half_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(GemmSmemHalf) + 128));
         cudaFuncSetAttribute(pivot_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pivot_smem);
         w.attr_set = true;
     }
-    static const bool full_tiles = getenv("GPCC_LARGE_FULL_TILES") != nullptr;   // A/B switch: one 8-warp CTA per tile
     const size_t half_smem = sizeof(GemmSmemHalf) + 128;
     auto launch_update = [&](int ntile, int phase, int kk, cudaStream_t strm) {
-        if (full_tiles) update_kernel<<<dim3(ntile, nb), 256, gemm_smem, strm>>>(a, kk, phase);
-        else update_half_kernel<<<dim3(2 * ntile, nb), 128, half_smem, strm>>>(a, kk, phase);
+        update_half_kernel<<<dim3(2 * ntile, nb), 128, half_smem, strm>>>(a, kk, phase);
     };
     long long launches = 0;
     if (profile) cudaEventRecord(w.ev[0], st);

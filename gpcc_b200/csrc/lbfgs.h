@@ -31,7 +31,6 @@ struct LbfgsOptions {
     double ftol = 1e-13;
     int history = 8;
     int max_ls = 30;
-    double dec_tol = 0.0;   // > 0: stop when the quasi-Newton estimate of the remaining decrease, 0.5 g'Hg, is below it
     int n_scale = 0;        // the first n_scale coordinates are softplus scales (alpha): their step cap grows with the coordinate
     double rel_cap = 0.25;  // ... to rel_cap * theta_i once that exceeds STEP_CAP
 };
@@ -155,10 +154,6 @@ struct LbfgsState {
         else small_df = 0;
         if (iters >= o.max_iter) { status = ITER_CAP; return; }
         new_direction(false);
-        // Newton decrement: with a full set of curvature pairs (history >= n) the two-loop recursion applies a good
-        // inverse-Hessian estimate, and -g'd/2 = g'Hg/2 predicts f - f* .  Stopping there instead of at gtol / ftol saves
-        // the last few iterations of every candidate, which only polish digits 8-13 of an optimum needed to 1e-6.
-        if (o.dec_tol > 0.0 && hcount >= n && -0.5 * gd0 <= o.dec_tol) status = CONVERGED;
     }
 
     // Feed the evaluation at xt (ok=false: matrix not PD / non-finite).  Afterwards either status != RUNNING

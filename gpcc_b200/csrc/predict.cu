@@ -465,7 +465,7 @@ int create_state(gpcc_problem* p, const double* delays, const double* alpha, dou
     // ---- A = K + Sobs (no B) = Lc Lc': blocked right-looking Cholesky with DMMA trailing updates (large_path.cu) ----
     int rc = reserve_eval(p, 0, 1);
     if (rc) return rc;
-    EvalSlot& q = ds.slot[0];
+    EvalSlot& q = ds.slot;
     std::memcpy(q.delays.h, delays, L * sizeof(double));
     std::memcpy(q.alpha.h, alpha, L * sizeof(double));
     q.rho.h[0] = rho;

@@ -35,7 +35,6 @@ struct FitCtl {                 // per-CTA control block in shared memory
     double jac[LBFGS_MAXN];     // d(alpha, rho)/d theta at the evaluation in flight
     double theta_next[LBFGS_MAXN];   // unconstrained parameters of the next evaluation (unpacked by L+1 threads)
     double theta_best[LBFGS_MAXN];
-    double grad_best[LBFGS_MAXN];
     double res_ll;
     double res_grad[LBFGS_MAXN];
     double bestf;
@@ -77,15 +76,11 @@ __device__ void advance(FitCtl& c, int L, const FitParams& fp, const FitBuffers&
             if (c.res_info == 0 && lb_finite(f) && f < c.bestf) {   // first minimum wins (Julia argmin, :209)
                 c.bestf = f;
                 c.best = c.j - 1;
-                if (!fp.screen_forward)
-                    for (int k = 0; k < n; ++k) c.grad_best[k] = -c.res_grad[k] * c.jac[k];
             }
         }
         if (c.j < fp.P) {
             unpack_to_ctl(c, th0 + (size_t)c.j * n, L, fp);
-            c.want_grad = fp.screen_forward ? 0 : 1;
-            c.fwd = fp.screen_forward;
-            if (c.fwd) ++c.n_fwd; else ++c.n_grad;
+            c.want_grad = 0; c.fwd = 1; ++c.n_fwd;
             ++c.j;
             return;
         }
@@ -107,13 +102,12 @@ __device__ void advance(FitCtl& c, int L, const FitParams& fp, const FitBuffers&
                 c.want_grad = 0; c.fwd = 1; ++c.n_fwd;
                 return;
             }
-        } else if (fp.screen_forward) {                   // gradient at the winner only
+        } else {                                          // gradient at the winner only
             unpack_to_ctl(c, c.theta_best, L, fp);
             c.want_grad = 1; c.fwd = 0; ++c.n_grad;
             c.phase = PH_START;
             return;
         }
-        if (OPT != 1) c.S.start(n, c.theta_best, c.bestf, c.grad_best, lo);
     } else if (OPT == 1 && c.phase == PH_NM) {                        // result at NM.xt
         c.NM.feed(c.res_info == 0 && lb_finite(c.res_ll), -c.res_ll, fp.max_iter, fp.nm_gtol);
         if (c.NM.phase != NmState::DONE) {

@@ -30,7 +30,6 @@ cudaError_t launch_kid(const DevProblem& p, const EvalBatch& b, int T, cudaStrea
     const int ntiles = T * (T + 1) / 2;
     const int threads = (ntiles + 31) / 32 * 32;
     static const int variant_env = getenv("GPCC_SMALL_VARIANT") ? atoi(getenv("GPCC_SMALL_VARIANT")) : -1;
-    static const bool no_fwd = getenv("GPCC_SMALL_NO_FWD") != nullptr;
     static int nsm = 0;
     if (nsm == 0) {
         int dev = 0;
@@ -45,7 +44,7 @@ cudaError_t launch_kid(const DevProblem& p, const EvalBatch& b, int T, cudaStrea
     int variant = variant_env;
     if (variant < 0) variant = (threads <= 128) ? (b.M >= 3 * nsm ? 2 : 1) : (b.M <= nsm ? 0 : 1);
     // forward-only mode (N^3/3 flop) when no gradient is wanted
-    const int fwd = (!no_fwd && !b.want_grad) ? 1 : 0;
+    const int fwd = b.want_grad ? 0 : 1;
     if (threads <= 128) {
         if (variant == 2) go<KID, 128, 3>(p, b, T, threads, 15, fwd, s);
         else              go<KID, 128, 2>(p, b, T, threads, 15, fwd, s);

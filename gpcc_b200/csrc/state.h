@@ -44,34 +44,23 @@ struct DevBuf {   // growable device buffer + pinned host mirror
     }
 };
 
-// Staging of one in-flight evaluation batch.  Two slots per device let the host-side L-BFGS bookkeeping of one
-// half of the candidates overlap with the kernel of the other half.  On the fused small-N path each slot has its own
-// stream: the CTAs of the next batch start on the SMs that the tail of the running one leaves idle (a batch ends with
-// a partial wave, and there are ~200 batches per fitted grid).  Per-launch CUDA-event times therefore overlap in
-// those tails, so the kernel time reported in the statistics is the length of the UNION of the launch intervals
-// (all event times are taken relative to one origin event per device).
+// Staging of one evaluation batch (evaluate_on_device).
 struct EvalSlot {
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr, done = nullptr;
     DevBuf<double> delays, alpha, rho, ll, grad;
     DevBuf<int> info;
-    int M = 0, want_grad = 0;
-    bool timed = false;
 };
 
 struct DeviceState {
     int dev = 0;
     cudaStream_t stream = nullptr;
-    cudaStream_t stream2 = nullptr;   // slot 1 of the fused small-N path
-    cudaEvent_t origin = nullptr;     // time zero of the kernel-busy accounting (re-recorded when the statistics are reset)
-    double busy_end_ms = 0;           // end of the last kernel interval counted so far, relative to `origin`
-    EvalSlot slot[2];
+    EvalSlot slot;
     DevBuf<double> post_ll, post_prior, post_out;   // persistent staging of the posterior kernel (no cudaMalloc/cudaFree per call)
     // staging of the device-resident fit (small_fit.cu)
     DevBuf<double> fit_delays, fit_theta0, fit_ll, fit_theta;
     DevBuf<int> fit_iters, fit_nfev, fit_status, fit_order;
     DevBuf<unsigned long long> fit_counters;
     DevBuf<double> gat_send, gat_recv, gat_post;     // all-gather of the grid results (persistent: no cudaMalloc per call)
-    cudaEvent_t fit_ev0 = nullptr, fit_ev1 = nullptr;
+    cudaEvent_t ev0 = nullptr, ev1 = nullptr;        // around the small-N kernel launch of the call (profiling)
     LargeWorkspace large;     // tiled large-N path (large_path.cu)
     // per-call statistics (profiling)
     double ms_eval = 0, ms_assembly = 0, ms_factor = 0, ms_gradreduce = 0;
@@ -107,11 +96,8 @@ struct gpcc_problem {
 };
 
 namespace gpcc {
-// Evaluate M (delay, alpha, rho) triples already staged in the pinned mirrors of device `di`;
-// results land in ds[di].ll.h / grad.h / info.h.
+// Evaluate M (delay, alpha, rho) triples already staged in the pinned mirrors of ds[di].slot and wait for them;
+// results land in ds[di].slot.ll.h / grad.h / info.h.
 int evaluate_on_device(gpcc_problem* p, int di, int M, int want_grad);
-int reserve_eval(gpcc_problem* p, int di, size_t M, int slot = 0);
-// asynchronous pair: launch_eval enqueues H2D + kernel + D2H of slot `slot`; finish_eval waits for it.
-int launch_eval(gpcc_problem* p, int di, int slot, int M, int want_grad);
-int finish_eval(gpcc_problem* p, int di, int slot);
+int reserve_eval(gpcc_problem* p, int di, size_t M);
 }  // namespace gpcc

@@ -20,8 +20,8 @@ for nb, N in ((3, 150), (2, 110)):
         ll0, info0 = p.loglik_batch(delays[:, :nb], alpha[:, :nb], rho)
         st0 = ctx.stats()
     assert np.array_equal(ll0, ll), np.max(np.abs(ll0 - ll))
-    print("   logL only (fwd=%s): kernel %.3f ms  %.1f us/eval-slot  %.2f TFLOP/s (N^3/3)" % (
-        "off" if os.environ.get("GPCC_SMALL_NO_FWD") else "on", st0["ms_eval_kernels"], st0["ms_eval_kernels"] * 1e3 / (M / 148),
+    print("   logL only (forward-only): kernel %.3f ms  %.1f us/eval-slot  %.2f TFLOP/s (N^3/3)" % (
+        st0["ms_eval_kernels"], st0["ms_eval_kernels"] * 1e3 / (M / 148),
         M * float(N)**3 / 3 / st0["ms_eval_kernels"] / 1e9), flush=True)
     r = [op.loglik_grad(delays[m, :nb], alpha[m, :nb], rho[m]) for m in range(8)]
     err = max(abs(ll[m] - r[m][0]) / abs(r[m][0]) for m in range(8)); gerr = max(np.max(np.abs(g[m] - r[m][1])) for m in range(8))

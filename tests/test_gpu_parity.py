@@ -726,8 +726,6 @@ def test_prior_with_minus_infinity_and_iteration_cap_zero(ctx):
 
 @pytest.mark.parametrize("switch", [
     {"GPCC_FIT_HOST": "1"},                                    # host-driven batched L-BFGS (api.cu fit_shard) instead of the persistent fit kernel
-    {"GPCC_SCREEN_FULL": "1"},                                 # screening with gradient evaluations instead of forward-only ones
-    {"GPCC_SMALL_NO_FWD": "1"},                                # logL-only evaluations through the full sweep
     {"GPCC_SMALL_VARIANT": "0"},                               # one CTA per SM at 255 registers whatever the batch size
 ], ids=lambda d: "+".join(f"{k[5:]}={v}" for k, v in d.items()))
 def test_alternative_drivers_agree(ctx, switch):
