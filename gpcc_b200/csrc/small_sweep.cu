@@ -37,8 +37,8 @@ cudaError_t launch_kid(const DevProblem& p, const EvalBatch& b, int T, cudaStrea
         cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
     }
     // Occupancy variant by batch size (measured on B200, profiles/small_sweep_variants_r1.log).
-    //   N <= 111 (128 threads): three CTAs per SM are 8 % faster once every SM has three (32.7 vs 35.6 us per evaluation
-    //   and SM), but slower when the batch leaves SMs with one or two (82 vs 65 us at one CTA per SM);
+    //   N <= 119 (T <= 15: 120 tiles, 128 threads): three CTAs per SM are 8 % faster once every SM has three (32.7 vs
+    //   35.6 us per evaluation and SM), but slower when the batch leaves SMs with one or two (82 vs 65 us at one CTA per SM);
     //   N <= 151 (192 threads): a CTA that is alone on its SM runs faster with 255 registers and no spills (101 vs 122 us),
     //   two co-resident CTAs at 168 registers win as soon as there is more than one evaluation per SM (134 vs 188 us for two).
     int variant = variant_env;
