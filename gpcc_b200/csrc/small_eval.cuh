@@ -31,6 +31,7 @@
 #include "kernfun.cuh"
 #include <climits>
 #include <cmath>
+#include <type_traits>
 
 namespace gpcc {
 namespace small {
@@ -69,31 +70,25 @@ __host__ __device__ inline size_t eval_smem_bytes(int T, int want_grad) {
     return doubles * sizeof(double) + (size_t)Np * sizeof(int) + 16;
 }
 
-// Publish column `kn` (tile tkn, in-tile index KKN) of the symmetric matrix for the next sweep step.
-// Scalar STS.64 straight from the tile registers (no staging moves); only warps that contain an owner enter.
-template <int KKN>
-__device__ __forceinline__ void publish(const double (&A)[8][8], int ti, int tj, int tkn, int kn, double* nb, double* pslot,
-                                        double* piv, bool live, bool fwd) {
-    // forward-only mode: the row part (tiles left of the pivot tile) is never read again
-    const bool pc = live && (tj == tkn), prw = live && (ti == tkn) && (!fwd || tj == tkn);
-    if (!__any_sync(0xffffffffu, pc || prw)) return;
-    if (pc) {
-        double* dst = nb + 2 * ti;
-        if (prw) {  // diagonal tile: below the diagonal from the column, above it from the row
-#pragma unroll
-            for (int r = 0; r < 8; ++r) dst[(r >> 1) * CS + (r & 1)] = (r >= KKN) ? A[r][KKN] : A[KKN][r];
-            const double d = A[KKN][KKN];
-            piv[kn] = d;
-            *pslot = 1.0 / d;
-        } else {
-#pragma unroll
-            for (int r = 0; r < 8; ++r) dst[(r >> 1) * CS + (r & 1)] = A[r][KKN];
-        }
-    } else if (prw) {
-        double* dst = nb + 2 * tj;
-#pragma unroll
-        for (int c = 0; c < 8; ++c) dst[(c >> 1) * CS + (c & 1)] = A[KKN][c];
+// Occupancy instantiation <MAXTHREADS, MINBLOCKS> of the batch kernel (small_sweep.cu) and of the fit kernel (small_fit.cu)
+// by tile count T, batch size M and the SM count of the device (measured on B200, profiles/small_sweep_variants_r1.log):
+//   N <= 119 (T <= 15: 120 tiles, 128 threads): three CTAs per SM are 8 % faster once every SM has three (32.7 vs
+//   35.6 us per evaluation and SM), but slower when the batch leaves SMs with one or two (82 vs 65 us at one CTA per SM);
+//   N <= 151 (192 threads): a CTA that is alone on its SM runs faster with 255 registers and no spills (101 vs 122 us),
+//   two co-resident CTAs at 168 registers win as soon as there is more than one evaluation per SM (134 vs 188 us for two).
+// Returns f(std::integral_constant<int, MAXTHREADS>, std::integral_constant<int, MINBLOCKS>, threads, maxT): threads is the
+// block size for T (its tiles in whole warps), maxT the largest T the instantiation serves.
+template <class F>
+cudaError_t with_instantiation(int T, int M, int nsm, F&& f) {
+    using std::integral_constant;
+    const int threads = (T * (T + 1) / 2 + 31) / 32 * 32;
+    if (threads <= 128) {
+        if (M >= 3 * nsm) return f(integral_constant<int, 128>(), integral_constant<int, 3>(), threads, 15);
+        return f(integral_constant<int, 128>(), integral_constant<int, 2>(), threads, 15);
     }
+    if (threads <= 192 && M > nsm) return f(integral_constant<int, 192>(), integral_constant<int, 2>(), threads, 19);
+    if (threads <= 224) return f(integral_constant<int, 224>(), integral_constant<int, 1>(), threads, 20);
+    return f(integral_constant<int, 352>(), integral_constant<int, 1>(), threads, SMALL_MAX_T);
 }
 
 #ifdef GPCC_STEP_PROF   // scripts/microbench/step_prof.cu: per-warp clock() stamps of every sweep step, kept in shared memory
@@ -107,63 +102,16 @@ __device__ __forceinline__ void publish(const double (&A)[8][8], int ti, int tj,
 #define GPCC_PROF_ARG
 #endif
 
-template <int KK>
-__device__ __forceinline__ void sweep_step(double (&A)[8][8], int ti, int tj, int tk, int k, int N, double* cbuf, double* pbuf,
-                                           double* piv, bool active, bool fwd GPCC_PROF_PARAM) {
-    GPCC_STAMP(0);
-    // forward-only mode: lanes whose tile has left the elimination skip the update but stay in the (warp-wide) vote of
-    // `publish` and in the barrier below
-    const bool live = !fwd || tj >= tk;
-    if (live) {
-        const double* cb = cbuf + (k & 1) * VLEN;
-        double v[8];
-        load8(cb, tj, v);
-        const double pr = pbuf[k & 1];
-#pragma unroll
-        for (int c = 0; c < 8; ++c) v[c] *= pr;
-        // Column k of its owner tiles must become c * (1/d).  Those registers hold exactly the broadcast values c, so
-        // running the generic update with the multiplier (1 - 1/d) in that column writes c - c (1 - 1/d) = c/d without
-        // any extra instruction (relative error eps*d in entries of the inverse only; pivots, log-det and the
-        // quadratic form never read the swept region).
-        // Row k of its owner tiles must become c * (1/d) as well: there the registers hold c and the row multiplier is the
-        // pivot d itself, so using (d - 1) instead gives c - (d - 1) c/d = c/d.  Only the diagonal element needs a fix.
-        const bool own_col = (tj == tk), own_row = (ti == tk);
-        if (own_col) v[KK] = 1.0 - pr;
-#pragma unroll
-        for (int part = 0; part < 4; ++part) {   // rows two at a time: keeps only a pair of broadcast values live
-            double2 x = *reinterpret_cast<const double2*>(cb + part * CS + 2 * ti);
-            if (part == (KK >> 1) && own_row) {
-                if (KK & 1) x.y -= 1.0; else x.x -= 1.0;
-            }
-#pragma unroll
-            for (int c = 0; c < 8; ++c) {
-                A[2 * part][c] = fma(-x.x, v[c], A[2 * part][c]);
-                A[2 * part + 1][c] = fma(-x.y, v[c], A[2 * part + 1][c]);
-            }
-        }
-        if (own_col && own_row) A[KK][KK] = -pr;
-    }
-    GPCC_STAMP(1);
-    const int kn = k + 1;
-    if (kn < N) {
-        double* nb = cbuf + (kn & 1) * VLEN;
-        if (KK < 7) publish<(KK + 1) & 7>(A, ti, tj, tk, kn, nb, pbuf + (kn & 1), piv, active && live, fwd);
-        else        publish<0>(A, ti, tj, tk + 1, kn, nb, pbuf + (kn & 1), piv, active && live, fwd);
-    }
-    GPCC_STAMP(2);
-    __syncthreads();
-    GPCC_STAMP(3);
-}
-
-// ---- lean form of the step (default; -DGPCC_CLASSIC_STEP selects the form above) ----------------------------------------
-// Timeline measurements (scripts/microbench/step_prof.cu, profiles/step_prof_r2.log) show that a step is bound by the chain
-// through the warp that owns the next pivot: its tile update, then the IEEE division for the pivot reciprocal, the vote and
-// the divergent owner paths of `publish`, then the barrier (1250 cycles per step for a CTA alone on its SM, of which the 64
-// DFMAs of a warp are 144 issue cycles).  Here
+// ---- one sweep step -------------------------------------------------------------------------------------------------------
+// A step is bound by the chain through the warp that owns the next pivot: its tile update, the reciprocal of the next pivot,
+// its stores of the next column, then the barrier at which every other warp waits for it (of the ~970 cycles of a step for a
+// CTA alone on its SM, the 64 DFMAs of a warp are 144 issue cycles: per-warp timelines of scripts/microbench/step_prof.cu in
+// profiles/README.md).  So the step keeps that chain short:
 //   * the row pair that holds the next pivot row is updated first and the reciprocal of the next pivot is formed right
 //     behind it by EVERY thread, branch free (approximate reciprocal + three Newton steps, no IEEE special-case branch), so
 //     that its latency hides under the remaining 48 DFMAs instead of sitting between the update and the barrier;
-//   * `publish` has no vote and no activity flag (threads beyond the last tile get out-of-range tile coordinates);
+//   * `publish` is one branch per owner role with no warp vote and no activity flag: threads beyond the last tile have
+//     out-of-range tile coordinates and own nothing;
 //   * buffer parities are compile-time, and full tiles run eight steps without loop-exit tests.
 __device__ __forceinline__ double fast_rcp(double d) {
     double x;
@@ -177,9 +125,11 @@ __device__ __forceinline__ double fast_rcp(double d) {
     return x;
 }
 
+// Publish column k+1 (tile tkn, in-tile index KKN) of the symmetric matrix, its pivot and the pivot's reciprocal prn for the
+// next sweep step.  Scalar STS.64 straight from the tile registers (no staging moves).
 template <int KKN>
-__device__ __forceinline__ void publish_lean(const double (&A)[8][8], int ti, int tj, int tkn, double* nb, double* pslot, double* pivslot,
-                                             double prn, bool fwd) {
+__device__ __forceinline__ void publish(const double (&A)[8][8], int ti, int tj, int tkn, double* nb, double* pslot, double* pivslot,
+                                        double prn, bool fwd) {
     const bool pc = (tj == tkn), prw = (ti == tkn) && (!fwd || pc);   // forward-only mode: the row part is never read again
     if (pc) {
         double* dst = nb + 2 * ti;
@@ -200,8 +150,8 @@ __device__ __forceinline__ void publish_lean(const double (&A)[8][8], int ti, in
 }
 
 template <int KK>
-__device__ __forceinline__ void sweep_step_lean(double (&A)[8][8], int ti, int tj, int tk, int k, double* cbuf, double* pbuf,
-                                                double* piv, bool fwd GPCC_PROF_PARAM) {
+__device__ __forceinline__ void sweep_step(double (&A)[8][8], int ti, int tj, int tk, int k, double* cbuf, double* pbuf,
+                                           double* piv, bool fwd GPCC_PROF_PARAM) {
     GPCC_STAMP(0);
     constexpr int PAR = KK & 1, NPAR = PAR ^ 1;     // k = 8 tk + KK: the buffer parity is known at compile time
     constexpr int KKN = (KK + 1) & 7;
@@ -214,8 +164,14 @@ __device__ __forceinline__ void sweep_step_lean(double (&A)[8][8], int ti, int t
         const double pr = pbuf[PAR];
 #pragma unroll
         for (int c = 0; c < 8; ++c) v[c] *= pr;
+        // Column k of its owner tiles must become c * (1/d).  Those registers hold exactly the broadcast values c, so
+        // running the generic update with the multiplier (1 - 1/d) in that column writes c - c (1 - 1/d) = c/d without
+        // any extra instruction (relative error eps*d in entries of the inverse only; pivots, log-det and the
+        // quadratic form never read the swept region).
+        // Row k of its owner tiles must become c * (1/d) as well: there the registers hold c and the row multiplier is the
+        // pivot d itself, so using (d - 1) instead gives c - (d - 1) c/d = c/d.  Only the diagonal element needs a fix.
         const bool own_col = (tj == tk), own_row = (ti == tk);
-        if (own_col) v[KK] = 1.0 - pr;              // see sweep_step: column k of its owners becomes c/d
+        if (own_col) v[KK] = 1.0 - pr;
 #pragma unroll
         for (int pp = 0; pp < 4; ++pp) {
             constexpr int P0 = KKN >> 1;
@@ -234,7 +190,7 @@ __device__ __forceinline__ void sweep_step_lean(double (&A)[8][8], int ti, int t
         if (own_col && own_row) A[KK][KK] = -pr;
     }
     GPCC_STAMP(1);
-    publish_lean<KKN>(A, ti, tj, KK < 7 ? tk : tk + 1, cbuf + NPAR * VLEN, pbuf + NPAR, piv + k + 1, prn, fwd);
+    publish<KKN>(A, ti, tj, KK < 7 ? tk : tk + 1, cbuf + NPAR * VLEN, pbuf + NPAR, piv + k + 1, prn, fwd);
     GPCC_STAMP(2);
     __syncthreads();
     GPCC_STAMP(3);
@@ -270,13 +226,12 @@ __device__ __forceinline__ void eval_one(const DevProblem& p, int T, double* sme
     const int tid = threadIdx.x;
     const int ntiles = T * (T + 1) / 2;
     const bool active = tid < ntiles;
+    // Only active threads read q.  The fallback for the others is dead code, but without it ptxas allocates the registers of
+    // the 255-register fit kernels differently (spills up in four instantiations, down in four), so it stays.
     const int q = active ? tid : ntiles - 1;
     int ti, tj;
-#ifndef GPCC_CLASSIC_STEP
     if (!active) { ti = T; tj = T; }   // threads beyond the last tile: out-of-range coordinates, never owners of anything
-    else
-#endif
-    if (fwd) {   // column-major tile order (see the header comment)
+    else if (fwd) {   // column-major tile order (see the header comment)
         int c = 0, rem = q;
         while (rem >= T - c) { rem -= T - c; ++c; }
         tj = c;
@@ -321,53 +276,15 @@ __device__ __forceinline__ void eval_one(const DevProblem& p, int T, double* sme
     __syncthreads();
 
     // ---- assembly of the bordered matrix tile in registers --------------------------------------
+    // Fully unrolled, unlike the gradient below: a rolled row loop keeps all 64 accumulators live from the first row on and
+    // spills (81 against 61 us per evaluation and SM, profiles/README.md).
     double A[8][8];
-#ifndef GPCC_CLASSIC_STEP
     if (!active) {
 #pragma unroll
         for (int r = 0; r < 8; ++r)
 #pragma unroll
             for (int c = 0; c < 8; ++c) A[r][c] = 0.0;
-    } else
-#endif
-#ifdef GPCC_ROLL_ASSEMBLY   // measured slower (all 64 accumulators live from the first row on: spills); kept for the record
-    {
-        // The row loop is ROLLED and the finished row lands in its registers through a switch with static indices: one copy of
-        // the eight kernel evaluations (8 x FP64 exp) instead of 64.  The profile of the fully unrolled form showed these
-        // phases bound by instruction fetch (64 KB of straight-line code per phase, executed once per evaluation, with two
-        // CTAs per SM in different phases: stall_no_inst was 45 % of their samples and 18 % of the whole kernel).
-        double tc[8], ac[8], rc[8];
-        int bc[8];
-        load8(tsh, tj, tc);
-        load8(av, tj, ac);
-        load8(abuf, tj, rc);
-#pragma unroll
-        for (int c = 0; c < 8; ++c) bc[c] = bandv[tj * 8 + c];
-#pragma unroll 1
-        for (int r = 0; r < 8; ++r) {
-            const int i = ti * 8 + r;
-            const int ci = cidx(i);
-            const double tr = tsh[ci], ar = av[ci], sbr = sbv[ci], dr = dadd[ci];
-            const int br = bandv[i];
-            double val[8];
-#pragma unroll
-            for (int c = 0; c < 8; ++c) {
-                const int j = tj * 8 + c;
-                const double kv = kern_value<KID>(tr - tc[c], kp);
-                double v = (ar * ac[c]) * kv;            // scale[l]*scale[m]*kernel  (delayedCovariance.jl:27)
-                if (i == j) v += dr;                     // + Sobs                   (gpccfixdelay_marginaliseb.jl:135)
-                if (br == bc[c]) v += sbr;               // + B = Q Sigma_b Q'
-                if (i == N) v = rc[c];                   // border row: r = Y - bbar (corner = 0)
-                if (i > N && i == j) v = 1.0;            // padding
-                val[c] = v;
-            }
-#define GPCC_ROW_IN(R) case R: _Pragma("unroll") for (int c = 0; c < 8; ++c) A[R][c] = val[c]; break;
-            switch (r) { GPCC_ROW_IN(0) GPCC_ROW_IN(1) GPCC_ROW_IN(2) GPCC_ROW_IN(3) GPCC_ROW_IN(4) GPCC_ROW_IN(5) GPCC_ROW_IN(6) default: _Pragma("unroll") for (int c = 0; c < 8; ++c) A[7][c] = val[c]; break; }
-#undef GPCC_ROW_IN
-        }
-    }
-#else
-    {
+    } else {
         double tc[8], ac[8], rc[8];
         int bc[8];
         load8(tsh, tj, tc);
@@ -394,43 +311,25 @@ __device__ __forceinline__ void eval_one(const DevProblem& p, int T, double* sme
             }
         }
     }
-#endif
     __syncthreads();   // everyone has read abuf/tsh before cbuf traffic starts (abuf is reused later)
 
     // ---- publish column 0, then N sweep steps ----------------------------------------------------
 #ifdef GPCC_STEP_PROF
     __shared__ unsigned prof[4 * 8 * GPCC_PROF_MAXSTEPS];
 #endif
-#ifdef GPCC_CLASSIC_STEP
-    publish<0>(A, ti, tj, 0, 0, cbuf, pbuf, piv, active, fwd);
-    __syncthreads();
-    for (int tk = 0; tk < T; ++tk) {
-        const int k0 = tk * 8;
-        if (k0 >= N) break;
-        sweep_step<0>(A, ti, tj, tk, k0 + 0, N, cbuf, pbuf, piv, active, fwd GPCC_PROF_ARG); if (k0 + 1 >= N) break;
-        sweep_step<1>(A, ti, tj, tk, k0 + 1, N, cbuf, pbuf, piv, active, fwd GPCC_PROF_ARG); if (k0 + 2 >= N) break;
-        sweep_step<2>(A, ti, tj, tk, k0 + 2, N, cbuf, pbuf, piv, active, fwd GPCC_PROF_ARG); if (k0 + 3 >= N) break;
-        sweep_step<3>(A, ti, tj, tk, k0 + 3, N, cbuf, pbuf, piv, active, fwd GPCC_PROF_ARG); if (k0 + 4 >= N) break;
-        sweep_step<4>(A, ti, tj, tk, k0 + 4, N, cbuf, pbuf, piv, active, fwd GPCC_PROF_ARG); if (k0 + 5 >= N) break;
-        sweep_step<5>(A, ti, tj, tk, k0 + 5, N, cbuf, pbuf, piv, active, fwd GPCC_PROF_ARG); if (k0 + 6 >= N) break;
-        sweep_step<6>(A, ti, tj, tk, k0 + 6, N, cbuf, pbuf, piv, active, fwd GPCC_PROF_ARG); if (k0 + 7 >= N) break;
-        sweep_step<7>(A, ti, tj, tk, k0 + 7, N, cbuf, pbuf, piv, active, fwd GPCC_PROF_ARG);
-    }
-#else
-    publish_lean<0>(A, ti, tj, 0, cbuf, pbuf, piv, fast_rcp(A[0][0]), fwd);
+    publish<0>(A, ti, tj, 0, cbuf, pbuf, piv, fast_rcp(A[0][0]), fwd);
     __syncthreads();
     for (int tk = 0; 8 * tk < N; ++tk) {   // one copy of the eight specialised steps; the guards only matter in the last tile
         const int k0 = tk * 8;               // (the last step also publishes "column N", the border row: never read, harmless)
-        sweep_step_lean<0>(A, ti, tj, tk, k0 + 0, cbuf, pbuf, piv, fwd GPCC_PROF_ARG);
-        if (k0 + 1 < N) sweep_step_lean<1>(A, ti, tj, tk, k0 + 1, cbuf, pbuf, piv, fwd GPCC_PROF_ARG);
-        if (k0 + 2 < N) sweep_step_lean<2>(A, ti, tj, tk, k0 + 2, cbuf, pbuf, piv, fwd GPCC_PROF_ARG);
-        if (k0 + 3 < N) sweep_step_lean<3>(A, ti, tj, tk, k0 + 3, cbuf, pbuf, piv, fwd GPCC_PROF_ARG);
-        if (k0 + 4 < N) sweep_step_lean<4>(A, ti, tj, tk, k0 + 4, cbuf, pbuf, piv, fwd GPCC_PROF_ARG);
-        if (k0 + 5 < N) sweep_step_lean<5>(A, ti, tj, tk, k0 + 5, cbuf, pbuf, piv, fwd GPCC_PROF_ARG);
-        if (k0 + 6 < N) sweep_step_lean<6>(A, ti, tj, tk, k0 + 6, cbuf, pbuf, piv, fwd GPCC_PROF_ARG);
-        if (k0 + 7 < N) sweep_step_lean<7>(A, ti, tj, tk, k0 + 7, cbuf, pbuf, piv, fwd GPCC_PROF_ARG);
+        sweep_step<0>(A, ti, tj, tk, k0 + 0, cbuf, pbuf, piv, fwd GPCC_PROF_ARG);
+        if (k0 + 1 < N) sweep_step<1>(A, ti, tj, tk, k0 + 1, cbuf, pbuf, piv, fwd GPCC_PROF_ARG);
+        if (k0 + 2 < N) sweep_step<2>(A, ti, tj, tk, k0 + 2, cbuf, pbuf, piv, fwd GPCC_PROF_ARG);
+        if (k0 + 3 < N) sweep_step<3>(A, ti, tj, tk, k0 + 3, cbuf, pbuf, piv, fwd GPCC_PROF_ARG);
+        if (k0 + 4 < N) sweep_step<4>(A, ti, tj, tk, k0 + 4, cbuf, pbuf, piv, fwd GPCC_PROF_ARG);
+        if (k0 + 5 < N) sweep_step<5>(A, ti, tj, tk, k0 + 5, cbuf, pbuf, piv, fwd GPCC_PROF_ARG);
+        if (k0 + 6 < N) sweep_step<6>(A, ti, tj, tk, k0 + 6, cbuf, pbuf, piv, fwd GPCC_PROF_ARG);
+        if (k0 + 7 < N) sweep_step<7>(A, ti, tj, tk, k0 + 7, cbuf, pbuf, piv, fwd GPCC_PROF_ARG);
     }
-#endif
 
 #ifdef GPCC_STEP_PROF
     if (blockIdx.x == gpcc_prof_block)
@@ -484,6 +383,12 @@ __device__ __forceinline__ void eval_one(const DevProblem& p, int T, double* sme
     }
     __syncthreads();
 
+    // Two forms of the same sums, selected per translation unit.  The rolled one (GPCC_ROLL_GRADIENT, defined by small_fit.cu)
+    // takes the row of the tile out of its registers through a switch with static indices: one copy of the four kernel
+    // evaluations instead of 32.  The persistent fit kernel's CTAs drift apart, two co-resident CTAs are in different phases,
+    // and the smaller instruction footprint measured 2 % faster there (profiles/README.md).  In the batch kernel the rolled
+    // form changes the register allocation of the whole kernel, and forward-only evaluations, which never reach this code,
+    // measured 0.7 % slower at N = 150; so small_sweep.cu keeps the unrolled form.
 #ifdef GPCC_ROLL_GRADIENT
     double es = 0.0;
     const bool diag_tile = (ti == tj);
@@ -497,7 +402,7 @@ __device__ __forceinline__ void eval_one(const DevProblem& p, int T, double* sme
             tc[cc] = tsh[cj]; ac[cc] = av[cj]; wc[cc] = abuf[cj]; cols[cc] = 0.0;
         }
 #pragma unroll 1
-        for (int r = 0; r < 8; ++r) {                // rolled, like the assembly: one copy of the four kernel evaluations
+        for (int r = 0; r < 8; ++r) {
             const int ci = cidx(ti * 8 + r);
             const double tr = tsh[ci], ar = av[ci], wr = abuf[ci];
             double ain[4];

@@ -12,9 +12,7 @@
 // host synchronisations per fitted grid, the straggler tail of the batched rounds (a round ends when its slowest
 // candidate ends; here a slow candidate only occupies its own CTA) and the host threads that contend when 8 ranks share
 // one box.  Results do not depend on the schedule: candidates never interact.
-// The gradient phase is compiled in its rolled form here (one copy of the kernel evaluations instead of 32): the CTAs of the
-// persistent kernel drift apart, two co-resident CTAs are usually in different phases, and the smaller instruction footprint
-// measured 2 % faster (profiles/README.md); in the batch kernel, whose CTAs run in step, it is neutral.
+// The gradient phase is compiled in its rolled form here (small_eval.cuh says why only here).
 #define GPCC_ROLL_GRADIENT
 #include "small_eval.cuh"
 #include "lbfgs.h"
@@ -50,7 +48,7 @@ __device__ __forceinline__ double logistic(double x) { return 0.5 * (1.0 + tanh(
 // unpack (gpccfixdelay_marginaliseb.jl:112-126): alpha = makepositive(theta_l) + floor, rho = transformbetween(theta_L+1).
 // One thread per parameter: the FP64 exp / log1p / tanh chains of the L+1 transforms run side by side instead of one after
 // the other on thread 0 (the profile showed the other five warps waiting ~9 % of the kernel time for that thread).
-__device__ __forceinline__ void unpack_to_ctl(FitCtl& c, const double* theta, int, const FitParams&) {
+__device__ __forceinline__ void unpack_to_ctl(FitCtl& c, const double* theta) {
     for (int k = 0; k < c.S.n; ++k) c.theta_next[k] = theta[k];
 }
 __device__ __forceinline__ void unpack_parallel(FitCtl& c, int tid, int L, const FitParams& fp) {
@@ -79,7 +77,7 @@ __device__ void advance(FitCtl& c, int L, const FitParams& fp, const FitBuffers&
             }
         }
         if (c.j < fp.P) {
-            unpack_to_ctl(c, th0 + (size_t)c.j * n, L, fp);
+            unpack_to_ctl(c, th0 + (size_t)c.j * n);
             c.want_grad = 0; c.fwd = 1; ++c.n_fwd;
             ++c.j;
             return;
@@ -98,12 +96,12 @@ __device__ void advance(FitCtl& c, int L, const FitParams& fp, const FitBuffers&
             c.NM.start(n, c.theta_best, c.bestf, fp.max_iter, fp.nm_gtol);
             c.phase = PH_NM;
             if (c.NM.phase != NmState::DONE) {
-                unpack_to_ctl(c, c.NM.xt, L, fp);
+                unpack_to_ctl(c, c.NM.xt);
                 c.want_grad = 0; c.fwd = 1; ++c.n_fwd;
                 return;
             }
         } else {                                          // gradient at the winner only
-            unpack_to_ctl(c, c.theta_best, L, fp);
+            unpack_to_ctl(c, c.theta_best);
             c.want_grad = 1; c.fwd = 0; ++c.n_grad;
             c.phase = PH_START;
             return;
@@ -111,7 +109,7 @@ __device__ void advance(FitCtl& c, int L, const FitParams& fp, const FitBuffers&
     } else if (OPT == 1 && c.phase == PH_NM) {                        // result at NM.xt
         c.NM.feed(c.res_info == 0 && lb_finite(c.res_ll), -c.res_ll, fp.max_iter, fp.nm_gtol);
         if (c.NM.phase != NmState::DONE) {
-            unpack_to_ctl(c, c.NM.xt, L, fp);
+            unpack_to_ctl(c, c.NM.xt);
             c.want_grad = 0; c.fwd = 1; ++c.n_fwd;
             return;
         }
@@ -136,7 +134,7 @@ __device__ void advance(FitCtl& c, int L, const FitParams& fp, const FitBuffers&
     }
     if (c.S.status != LbfgsState::RUNNING) { c.phase = PH_DONE; return; }
     c.phase = PH_LBFGS;
-    unpack_to_ctl(c, c.S.xt, L, fp);
+    unpack_to_ctl(c, c.S.xt);
     c.want_grad = 1; c.fwd = 0; ++c.n_grad;
 }
 
@@ -202,7 +200,7 @@ small_fit_kernel(DevProblem p, FitParams fp, FitBuffers fb, int T, int ctl_offse
 }
 
 template <int KID, int MT, int MB, int OPT>
-cudaError_t go2(const DevProblem& p, const FitParams& fp, const FitBuffers& fb, int T, int threads, int maxT, int nsm, cudaStream_t s) {
+cudaError_t go(const DevProblem& p, const FitParams& fp, const FitBuffers& fb, int T, int threads, int maxT, int nsm, cudaStream_t s) {
     auto kfn = small_fit_kernel<KID, MT, MB, OPT>;
     const size_t ev = (eval_smem_bytes(T, 1) + 15) / 16 * 16;
     const size_t ev_max = (eval_smem_bytes(maxT, 1) + 15) / 16 * 16;
@@ -217,27 +215,16 @@ cudaError_t go2(const DevProblem& p, const FitParams& fp, const FitBuffers& fb, 
     return cudaGetLastError();
 }
 
-template <int KID, int MT, int MB>
-cudaError_t go(const DevProblem& p, const FitParams& fp, const FitBuffers& fb, int T, int threads, int maxT, int nsm, cudaStream_t s) {
-    if (fp.optimizer == 1) return go2<KID, MT, MB, 1>(p, fp, fb, T, threads, maxT, nsm, s);
-    return go2<KID, MT, MB, 0>(p, fp, fb, T, threads, maxT, nsm, s);
-}
-
 template <int KID>
 cudaError_t launch_kid(const DevProblem& p, const FitParams& fp, const FitBuffers& fb, int T, cudaStream_t s) {
-    const int ntiles = T * (T + 1) / 2;
-    const int threads = (ntiles + 31) / 32 * 32;
     int dev = 0, nsm = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
-    // occupancy variants as in small_sweep.cu: more co-resident CTAs at 168 registers once every SM gets that many
-    if (threads <= 128) {
-        if (fp.M >= 3 * nsm) return go<KID, 128, 3>(p, fp, fb, T, threads, 15, nsm, s);
-        return go<KID, 128, 2>(p, fp, fb, T, threads, 15, nsm, s);
-    }
-    if (threads <= 192 && fp.M > nsm) return go<KID, 192, 2>(p, fp, fb, T, threads, 19, nsm, s);
-    if (threads <= 224) return go<KID, 224, 1>(p, fp, fb, T, threads, 20, nsm, s);
-    return go<KID, 352, 1>(p, fp, fb, T, threads, SMALL_MAX_T, nsm, s);
+    return with_instantiation(T, fp.M, nsm, [&](auto mt, auto mb, int threads, int maxT) {
+        constexpr int MT = decltype(mt)::value, MB = decltype(mb)::value;
+        if (fp.optimizer == 1) return go<KID, MT, MB, 1>(p, fp, fb, T, threads, maxT, nsm, s);
+        return go<KID, MT, MB, 0>(p, fp, fb, T, threads, maxT, nsm, s);
+    });
 }
 
 }  // namespace

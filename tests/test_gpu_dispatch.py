@@ -1,9 +1,9 @@
 """Every kernel variant the host dispatch can select, against the oracle and against each other (run with -m gpu on a B200).
 
 The host code picks between separately compiled code paths: the fused small-N evaluator and the persistent fit kernel by
-tile count T = ceil((N+1)/8) and by batch size relative to the SM count (small_sweep.cu, small_fit.cu: <128,2>, <128,3>,
-<192,2>, <224,1>, <352,1>); the tiled path by wave size (512, 128 or 32 matrices by N), look-ahead on two streams, the shared
-leading block and the last-band cache (large_path.cu); the fitted state by tile edges of its triangular solve, Gram product
+tile count T = ceil((N+1)/8) and by batch size relative to the SM count (with_instantiation in small_eval.cuh: <128,2>,
+<128,3>, <192,2>, <224,1>, <352,1>); the tiled path by wave size (512, 128 or 32 matrices by N), look-ahead on two streams,
+the shared leading block and the last-band cache (large_path.cu); the fitted state by tile edges of its triangular solve, Gram product
 and one-CTA Cholesky (predict.cu).  A bug in one of them shows only in the calls that select it, so each is selected here
 on purpose.  Tolerances are those of test_gpu_parity.py; "bitwise" means np.array_equal.
 """
@@ -108,56 +108,33 @@ def test_every_small_size_matches_oracle(ctx):
             p.close()
 
 
-@pytest.mark.parametrize("N", [60, 119, 120, 151, 159, 199])
-def test_batch_size_dispatch_is_bitwise_stable(ctx, nsm, N):
+# (N, kernel, distinct candidates, seed of the light curves, seed of the candidates)
+DISPATCH_CASES = [pytest.param(N, oracle.KERNELS[k % 4], 3, 40 + k, k, id=str(N))
+                  for k, N in enumerate((60, 119, 120, 151, 159, 199))]
+DISPATCH_CASES += [pytest.param(N, kernel, 5, N, N, id=f"{N}-{kernel}") for N, kernel in ((60, "rbf"), (151, "matern52"))]
+
+
+@pytest.mark.parametrize("N,kernel,ncand,seed,cand_seed", DISPATCH_CASES)
+def test_batch_size_dispatch_is_bitwise_stable(ctx, nsm, N, kernel, ncand, seed, cand_seed):
     """The batch kernel's instantiation depends on M: <128,2> / <128,3> for T <= 15, <224,1> / <192,2> for T = 16-19,
-    <224,1> for T = 20, <352,1> for T >= 21.  Three distinct candidates repeated to M = 1, 3, SMs, SMs+1, 3 SMs-1 and 3 SMs:
+    <224,1> for T = 20, <352,1> for T >= 21.  A few distinct candidates repeated to M = 1, 3, SMs, SMs+1, 3 SMs-1 and 3 SMs:
     every copy must be bitwise the result of the M = 1 call, with and without gradient."""
-    k = [60, 119, 120, 151, 159, 199].index(N)
-    kernel = oracle.KERNELS[k % 4]
-    t, y, s, d = gpcc_b200.synthetic_bands(_bands(N), seed=40 + k, span=25.0)
+    t, y, s, d = gpcc_b200.synthetic_bands(_bands(N), seed=seed, span=25.0)
     p = Problem(t, y, s, kernel, ctx)
-    delays, alpha, rho = _candidates(3, 3, np.random.default_rng(k))
-    one = [p.loglik_batch(delays[j:j + 1], alpha[j:j + 1], rho[j:j + 1], want_grad=True) for j in range(3)]
-    one_f = [p.loglik_batch(delays[j:j + 1], alpha[j:j + 1], rho[j:j + 1])[0] for j in range(3)]
+    delays, alpha, rho = _candidates(3, ncand, np.random.default_rng(cand_seed))
+    one = [p.loglik_batch(delays[j:j + 1], alpha[j:j + 1], rho[j:j + 1], want_grad=True) for j in range(ncand)]
+    one_f = [p.loglik_batch(delays[j:j + 1], alpha[j:j + 1], rho[j:j + 1])[0] for j in range(ncand)]
     _check_oracle(oracle.Problem(t, y, s, kernel), delays, alpha, rho, np.array([o[0][0] for o in one]),
                   np.array([o[1][0] for o in one]), (N, kernel))
     for M in (1, 3, nsm, nsm + 1, 3 * nsm - 1, 3 * nsm):
-        rep = np.arange(M) % 3
+        rep = np.arange(M) % ncand
         ll, grad, info = p.loglik_batch(delays[rep], alpha[rep], rho[rep], want_grad=True)
         ll_f, info_f = p.loglik_batch(delays[rep], alpha[rep], rho[rep])
         assert np.all(info == 0) and np.all(info_f == 0)
-        for j in range(min(M, 3)):
+        for j in range(min(M, ncand)):
             sel = rep == j
             assert np.all(ll[sel] == one[j][0][0]) and np.all(grad[sel] == one[j][1][0]), (N, M, j)
             assert np.all(ll_f[sel] == one_f[j][0]), (N, M, j)
-
-
-def test_small_variant_switch_is_bitwise_stable(ctx):
-    """GPCC_SMALL_VARIANT = 0, 1, 2 forces an instantiation whatever the batch size: at M = 5 this reaches <128,3> (N = 60)
-    and <192,2> (N = 151), which the default only selects for large batches.  Same bits as the default."""
-    cases, ref = {}, {}
-    for N, kernel in ((60, "rbf"), (151, "matern52")):
-        t, y, s, d = gpcc_b200.synthetic_bands(_bands(N), seed=N, span=25.0)
-        delays, alpha, rho = _candidates(3, 5, np.random.default_rng(N))
-        p = Problem(t, y, s, kernel, ctx)
-        ref[N] = p.loglik_batch(delays, alpha, rho, want_grad=True)[:2] + (p.loglik_batch(delays, alpha, rho)[0],)
-        cases.update({f"{k}{N}": v for k, v in dict(delays=delays, alpha=alpha, rho=rho, **_pack(t, y, s)).items()})
-        cases[f"kernel{N}"] = np.array(kernel)
-    code = ("from test_gpu_dispatch import _unpack\n"
-            "for N in (60, 151):\n"
-            "    zz = {k: z[k + str(N)] for k in ('t', 'y', 's', 'n')}\n"
-            "    p = gpcc_b200.Problem(*_unpack(zz), str(z['kernel%d' % N]))\n"
-            "    a = (z['delays%d' % N], z['alpha%d' % N], z['rho%d' % N])\n"
-            "    ll, grad, info = p.loglik_batch(*a, want_grad=True)\n"
-            "    assert np.all(info == 0)\n"
-            "    out('ll%d' % N, ll); out('grad%d' % N, grad); out('llf%d' % N, p.loglik_batch(*a)[0])\n")
-    for variant in ("0", "1", "2"):
-        got = _run_switched({"GPCC_SMALL_VARIANT": variant}, code, **cases)
-        for N in (60, 151):
-            assert np.array_equal(got[f"ll{N}"], ref[N][0]), (variant, N)
-            assert np.array_equal(got[f"grad{N}"], ref[N][1]), (variant, N)
-            assert np.array_equal(got[f"llf{N}"], ref[N][2]), (variant, N)
 
 
 # ---- B. persistent fit kernel (small_fit.cu, lbfgs.h, nm.h) -----------------------------------------------------------------

@@ -726,7 +726,6 @@ def test_prior_with_minus_infinity_and_iteration_cap_zero(ctx):
 
 @pytest.mark.parametrize("switch", [
     {"GPCC_FIT_HOST": "1"},                                    # host-driven batched L-BFGS (api.cu fit_shard) instead of the persistent fit kernel
-    {"GPCC_SMALL_VARIANT": "0"},                               # one CTA per SM at 255 registers whatever the batch size
 ], ids=lambda d: "+".join(f"{k[5:]}={v}" for k, v in d.items()))
 def test_alternative_drivers_agree(ctx, switch):
     """The A/B switches of the fused small-N path (read once per process) must give the same answers as the default path:
