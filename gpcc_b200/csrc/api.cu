@@ -11,6 +11,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <limits>
+#include <memory>
 #include <string>
 #include <thread>
 #include <utility>
@@ -58,7 +59,7 @@ int gpcc::evaluate_on_device(gpcc_problem* p, int di, int M, int want_grad) {
     EvalSlot& q = s.slot;
     const int L = p->L;
     CUDA_TRY(cudaSetDevice(s.dev));
-    cudaStream_t stream = s.stream;
+    cudaStream_t stream = s.stream.get();
     CUDA_TRY(cudaMemcpyAsync(q.delays.d, q.delays.h, (size_t)M * L * sizeof(double), cudaMemcpyHostToDevice, stream));
     CUDA_TRY(cudaMemcpyAsync(q.alpha.d, q.alpha.h, (size_t)M * L * sizeof(double), cudaMemcpyHostToDevice, stream));
     CUDA_TRY(cudaMemcpyAsync(q.rho.d, q.rho.h, (size_t)M * sizeof(double), cudaMemcpyHostToDevice, stream));
@@ -68,9 +69,9 @@ int gpcc::evaluate_on_device(gpcc_problem* p, int di, int M, int want_grad) {
     b.h_delays = q.delays.h; b.h_alpha = q.alpha.h; b.h_rho = q.rho.h;
     const bool prof = p->ctx->profiling;
     if (p->small_path) {
-        if (prof) CUDA_TRY(cudaEventRecord(s.ev0, stream));
+        if (prof) CUDA_TRY(cudaEventRecord(s.ev0.get(), stream));
         CUDA_TRY(small_sweep_launch(p->pd[di].dp, b, stream));
-        if (prof) CUDA_TRY(cudaEventRecord(s.ev1, stream));
+        if (prof) CUDA_TRY(cudaEventRecord(s.ev1.get(), stream));
         s.launches += 1;
     } else {
         LargeTimings lt;
@@ -89,7 +90,7 @@ int gpcc::evaluate_on_device(gpcc_problem* p, int di, int M, int want_grad) {
     CUDA_TRY(cudaStreamSynchronize(stream));
     if (prof && p->small_path) {
         float ms = 0;
-        CUDA_TRY(cudaEventElapsedTime(&ms, s.ev0, s.ev1));
+        CUDA_TRY(cudaEventElapsedTime(&ms, s.ev0.get(), s.ev1.get()));
         s.ms_eval += ms;
     }
     s.evals += M;
@@ -119,7 +120,7 @@ void reset_stats(gpcc_ctx* ctx) {
         // the call about to start refills the pinned staging buffers: wait for what may still read them (a call that
         // failed midway, or the all-gather of posterior_on_devices, which synchronises device 0 only)
         cudaSetDevice(s.dev);
-        cudaStreamSynchronize(s.stream);
+        cudaStreamSynchronize(s.stream.get());
     }
 }
 
@@ -223,7 +224,7 @@ int fit_shard_device(gpcc_problem* p, int di, const std::vector<int>& idx, const
     }
     for (int k = 0; k < 8; ++k) s.fit_counters.h[k] = 0;
     s.fit_counters.h[5] = ~0ULL;
-    cudaStream_t st = s.stream;
+    cudaStream_t st = s.stream.get();
     CUDA_TRY(cudaMemcpyAsync(s.fit_delays.d, s.fit_delays.h, (size_t)m * L * sizeof(double), cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(s.fit_theta0.d, s.fit_theta0.h, nth * sizeof(double), cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(s.fit_counters.d, s.fit_counters.h, 8 * sizeof(unsigned long long), cudaMemcpyHostToDevice, st));
@@ -238,9 +239,9 @@ int fit_shard_device(gpcc_problem* p, int di, const std::vector<int>& idx, const
     fb.iters = s.fit_iters.d; fb.nfev = s.fit_nfev.d; fb.status = s.fit_status.d; fb.counters = s.fit_counters.d;
     fb.order = s.fit_order.d;
     const bool prof = p->ctx->profiling;
-    if (prof) CUDA_TRY(cudaEventRecord(s.ev0, st));
+    if (prof) CUDA_TRY(cudaEventRecord(s.ev0.get(), st));
     CUDA_TRY(small_fit_launch(p->pd[di].dp, fp, fb, st));
-    if (prof) CUDA_TRY(cudaEventRecord(s.ev1, st));
+    if (prof) CUDA_TRY(cudaEventRecord(s.ev1.get(), st));
     CUDA_TRY(cudaMemcpyAsync(s.fit_ll.h, s.fit_ll.d, (size_t)m * sizeof(double), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaMemcpyAsync(s.fit_theta.h, s.fit_theta.d, (size_t)m * n * sizeof(double), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaMemcpyAsync(s.fit_iters.h, s.fit_iters.d, (size_t)m * sizeof(int), cudaMemcpyDeviceToHost, st));
@@ -250,7 +251,7 @@ int fit_shard_device(gpcc_problem* p, int di, const std::vector<int>& idx, const
     CUDA_TRY(cudaStreamSynchronize(st));
     if (prof) {
         float ms = 0;
-        CUDA_TRY(cudaEventElapsedTime(&ms, s.ev0, s.ev1));
+        CUDA_TRY(cudaEventElapsedTime(&ms, s.ev0.get(), s.ev1.get()));
         s.ms_eval += ms;
     }
     static const bool debug = getenv("GPCC_FIT_DEBUG") != nullptr;
@@ -448,44 +449,35 @@ int gpcc_ctx_create(int ndev, const int* dev_ids, gpcc_ctx** out) {
     }
     if (ndev <= 0) ndev = 1;
     if (ndev > count) return fail(-2, "ndev exceeds the number of visible CUDA devices");
-    gpcc_ctx* ctx = new gpcc_ctx();
-    ctx->ds.resize(ndev);
+    // every id is checked before a DeviceState holds it: its destructor makes its device current
+    std::vector<int> devs(ndev);
     for (int i = 0; i < ndev; ++i) {
-        DeviceState& s = ctx->ds[i];
-        s.dev = dev_ids ? dev_ids[i] : i;
-        if (s.dev < 0 || s.dev >= count) { delete ctx; return fail(-3, "invalid device id"); }
+        devs[i] = dev_ids ? dev_ids[i] : i;
+        if (devs[i] < 0 || devs[i] >= count) return fail(-3, "invalid device id");
         cudaDeviceProp prop;
-        CUDA_TRY(cudaGetDeviceProperties(&prop, s.dev));
-        if (prop.major < 10) { delete ctx; return fail(-4, "libgpcc_b200 is built for sm_100a (Blackwell B200) only"); }
+        CUDA_TRY(cudaGetDeviceProperties(&prop, devs[i]));
+        if (prop.major < 10) return fail(-4, "libgpcc_b200 is built for sm_100a (Blackwell B200) only");
+    }
+    std::unique_ptr<gpcc_ctx> ctx(new gpcc_ctx());
+    ctx->ds = std::vector<DeviceState>(ndev);     // DeviceState owns device resources: not movable, so no resize()
+    for (int i = 0; i < ndev; ++i) ctx->ds[i].dev = devs[i];
+    for (DeviceState& s : ctx->ds) {
         CUDA_TRY(cudaSetDevice(s.dev));
         // highest priority: in the tiled path this stream carries the critical pivot/panel chain while the bulk of each
         // trailing update runs on a low-priority stream (large_path.cu), so pivot CTAs get the next free SM
         int prio_lo = 0, prio_hi = 0;
         CUDA_TRY(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
-        CUDA_TRY(cudaStreamCreateWithPriority(&s.stream, cudaStreamNonBlocking, prio_hi));
-        CUDA_TRY(cudaEventCreate(&s.ev0));
-        CUDA_TRY(cudaEventCreate(&s.ev1));
+        CUDA_TRY(create_stream(s.stream, prio_hi));
+        CUDA_TRY(create_event(s.ev0));
+        CUDA_TRY(create_event(s.ev1));
     }
-    *out = ctx;
+    *out = ctx.release();
     return 0;
 }
 
 int gpcc_ctx_destroy(gpcc_ctx* ctx) {
     if (!ctx) return 0;
     if (ctx->nccl) nccl_bridge_destroy(ctx->nccl);
-    for (auto& s : ctx->ds) {
-        cudaSetDevice(s.dev);
-        EvalSlot& q = s.slot;
-        q.delays.release(); q.alpha.release(); q.rho.release(); q.ll.release(); q.grad.release(); q.info.release();
-        s.post_ll.release(); s.post_prior.release(); s.post_out.release();
-        s.gat_send.release(); s.gat_recv.release(); s.gat_post.release();
-        s.fit_delays.release(); s.fit_theta0.release(); s.fit_ll.release(); s.fit_theta.release();
-        s.fit_iters.release(); s.fit_nfev.release(); s.fit_status.release(); s.fit_counters.release(); s.fit_order.release();
-        if (s.ev0) cudaEventDestroy(s.ev0);
-        if (s.ev1) cudaEventDestroy(s.ev1);
-        large_workspace_release(s.large);
-        if (s.stream) cudaStreamDestroy(s.stream);
-    }
     delete ctx;
     return 0;
 }
@@ -510,12 +502,12 @@ int gpcc_problem_create(gpcc_ctx* ctx, int L, const int* n_per_band, const doubl
     if (L < 1 || L > GPCC_MAX_BANDS) return fail(-2, "L must be in 1..GPCC_MAX_BANDS");
     if (kernel_id < 0 || kernel_id > 3)
         return fail(-3, "unknown kernel (expected GPCC.OU, GPCC.rbf, GPCC.matern32 or GPCC.matern52)");
-    gpcc_problem* p = new gpcc_problem();
+    std::unique_ptr<gpcc_problem> p(new gpcc_problem());
     p->ctx = ctx; p->L = L; p->kernel_id = kernel_id;
     p->n_per_band.assign(n_per_band, n_per_band + L);
     p->band_start.assign(L + 1, 0);
     for (int l = 0; l < L; ++l) {
-        if (n_per_band[l] < 1) { delete p; return fail(-4, "every band needs at least one observation"); }
+        if (n_per_band[l] < 1) return fail(-4, "every band needs at least one observation");
         p->band_start[l + 1] = p->band_start[l] + n_per_band[l];
     }
     const int N = p->N = p->band_start[L];
@@ -535,10 +527,8 @@ int gpcc_problem_create(gpcc_ctx* ctx, int L, const int* n_per_band, const doubl
             double v = 0; for (int i = a; i < b; ++i) v += (y[i] - mean) * (y[i] - mean);
             p->Sigmab[l] = n > 1 ? 100.0 * v / (n - 1) : std::numeric_limits<double>::quiet_NaN();
         }
-        if (!(p->Sigmab[l] > 0) || !std::isfinite(p->mub[l])) {
-            delete p;
+        if (!(p->Sigmab[l] > 0) || !std::isfinite(p->mub[l]))
             return fail(-5, "prior of the shift b is degenerate (band with <2 points or zero variance)");
-        }
     }
     p->band.resize(N); p->resid.resize(N); p->s2.resize(N); p->sigb.resize(N);
     for (int l = 0; l < L; ++l)
@@ -547,49 +537,37 @@ int gpcc_problem_create(gpcc_ctx* ctx, int L, const int* n_per_band, const doubl
             p->resid[i] = y[i] - p->mub[l];              // Y - Q*mu_b (:98, :139)
             p->s2[i] = sigma[i] * sigma[i];              // Sobs (:89)
             p->sigb[i] = p->Sigmab[l];                   // B = Q Sigma_b Q' (:96)
-            if (!std::isfinite(t[i]) || !std::isfinite(y[i]) || !std::isfinite(sigma[i])) {
-                delete p;
+            if (!std::isfinite(t[i]) || !std::isfinite(y[i]) || !std::isfinite(sigma[i]))
                 return fail(-6, "non-finite input data");
-            }
         }
     p->small_path = small_path_supports(N);
-    p->pd.resize(ctx->ds.size());
-    struct Guard { gpcc_problem* p; ~Guard() { if (p) gpcc_problem_destroy(p); } } guard{p};   // a failed upload frees what exists
-    for (size_t di = 0; di < ctx->ds.size(); ++di) {
-        auto& d = p->pd[di];
-        d.dev = ctx->ds[di].dev;
+    p->pd = std::vector<gpcc_problem::PerDev>(ctx->ds.size());   // not movable, like DeviceState
+    for (size_t di = 0; di < ctx->ds.size(); ++di) p->pd[di].dev = ctx->ds[di].dev;   // before a failed upload destroys them
+    for (auto& d : p->pd) {
         CUDA_TRY(cudaSetDevice(d.dev));
-        CUDA_TRY(cudaMalloc(&d.t, N * sizeof(double)));
-        CUDA_TRY(cudaMalloc(&d.resid, N * sizeof(double)));
-        CUDA_TRY(cudaMalloc(&d.y, N * sizeof(double)));
-        CUDA_TRY(cudaMalloc(&d.s2, N * sizeof(double)));
-        CUDA_TRY(cudaMalloc(&d.sigb, N * sizeof(double)));
-        CUDA_TRY(cudaMalloc(&d.band, N * sizeof(int)));
-        CUDA_TRY(cudaMemcpy(d.t, p->t.data(), N * sizeof(double), cudaMemcpyHostToDevice));
-        CUDA_TRY(cudaMemcpy(d.resid, p->resid.data(), N * sizeof(double), cudaMemcpyHostToDevice));
-        CUDA_TRY(cudaMemcpy(d.y, p->y.data(), N * sizeof(double), cudaMemcpyHostToDevice));
-        CUDA_TRY(cudaMemcpy(d.s2, p->s2.data(), N * sizeof(double), cudaMemcpyHostToDevice));
-        CUDA_TRY(cudaMemcpy(d.sigb, p->sigb.data(), N * sizeof(double), cudaMemcpyHostToDevice));
-        CUDA_TRY(cudaMemcpy(d.band, p->band.data(), N * sizeof(int), cudaMemcpyHostToDevice));
+        CUDA_TRY(d.t.reserve(N));
+        CUDA_TRY(d.resid.reserve(N));
+        CUDA_TRY(d.y.reserve(N));
+        CUDA_TRY(d.s2.reserve(N));
+        CUDA_TRY(d.sigb.reserve(N));
+        CUDA_TRY(d.band.reserve(N));
+        CUDA_TRY(cudaMemcpy(d.t.d, p->t.data(), N * sizeof(double), cudaMemcpyHostToDevice));
+        CUDA_TRY(cudaMemcpy(d.resid.d, p->resid.data(), N * sizeof(double), cudaMemcpyHostToDevice));
+        CUDA_TRY(cudaMemcpy(d.y.d, p->y.data(), N * sizeof(double), cudaMemcpyHostToDevice));
+        CUDA_TRY(cudaMemcpy(d.s2.d, p->s2.data(), N * sizeof(double), cudaMemcpyHostToDevice));
+        CUDA_TRY(cudaMemcpy(d.sigb.d, p->sigb.data(), N * sizeof(double), cudaMemcpyHostToDevice));
+        CUDA_TRY(cudaMemcpy(d.band.d, p->band.data(), N * sizeof(int), cudaMemcpyHostToDevice));
         d.dp.N = N; d.dp.L = L; d.dp.kernel_id = kernel_id;
-        d.dp.t = d.t; d.dp.resid = d.resid; d.dp.y = d.y; d.dp.s2 = d.s2; d.dp.sigb = d.sigb; d.dp.band = d.band;
+        d.dp.t = d.t.d; d.dp.resid = d.resid.d; d.dp.y = d.y.d; d.dp.s2 = d.s2.d; d.dp.sigb = d.sigb.d; d.dp.band = d.band.d;
         for (int l = 0; l <= L; ++l) d.dp.band_start[l] = p->band_start[l];
     }
-    guard.p = nullptr;
-    *out = p;
+    *out = p.release();
     return 0;
 }
 
 int gpcc_problem_destroy(gpcc_problem* p) {
-    if (!p) return 0;
-    if (p->cached_state) { gpcc_fit_state_destroy(p->cached_state); p->cached_state = nullptr; }
-    // only the problem's own copies of the device ids are read here: the context may already be gone (finalizer order in
-    // Julia / Python is unspecified), see the lifetime rule in include/gpcc_b200.h
-    for (size_t di = 0; di < p->pd.size(); ++di) {
-        auto& d = p->pd[di];
-        cudaSetDevice(d.dev);
-        cudaFree(d.t); cudaFree(d.resid); cudaFree(d.y); cudaFree(d.s2); cudaFree(d.sigb); cudaFree(d.band);
-    }
+    // only the problem's own copies of the device ids are read here (PerDev::dev): the context may already be gone
+    // (finalizer order in Julia / Python is unspecified), see the lifetime rule in include/gpcc_b200.h
     delete p;
     return 0;
 }
@@ -783,20 +761,21 @@ int gpcc_getprobabilities(gpcc_ctx* ctx, int M, const double* loglik, const doub
     if (M < 1) return fail(-2, "M < 1");
     DeviceState& s = ctx->ds[0];
     CUDA_TRY(cudaSetDevice(s.dev));
+    cudaStream_t st = s.stream.get();
     // persistent buffers: cudaMalloc/cudaFree serialise against every other context on the box (and stall for hundreds
     // of milliseconds when several ranks with NCCL peer mappings hit them at once), so the hot path never calls them
     CUDA_TRY(s.post_ll.reserve(M));
     CUDA_TRY(s.post_out.reserve(M));
     if (logprior) CUDA_TRY(s.post_prior.reserve(M));
     std::memcpy(s.post_ll.h, loglik, (size_t)M * sizeof(double));
-    CUDA_TRY(cudaMemcpyAsync(s.post_ll.d, s.post_ll.h, (size_t)M * sizeof(double), cudaMemcpyHostToDevice, s.stream));
+    CUDA_TRY(cudaMemcpyAsync(s.post_ll.d, s.post_ll.h, (size_t)M * sizeof(double), cudaMemcpyHostToDevice, st));
     if (logprior) {
         std::memcpy(s.post_prior.h, logprior, (size_t)M * sizeof(double));
-        CUDA_TRY(cudaMemcpyAsync(s.post_prior.d, s.post_prior.h, (size_t)M * sizeof(double), cudaMemcpyHostToDevice, s.stream));
+        CUDA_TRY(cudaMemcpyAsync(s.post_prior.d, s.post_prior.h, (size_t)M * sizeof(double), cudaMemcpyHostToDevice, st));
     }
-    CUDA_TRY(posterior_launch(M, s.post_ll.d, logprior ? s.post_prior.d : nullptr, s.post_out.d, s.stream));
-    CUDA_TRY(cudaMemcpyAsync(s.post_out.h, s.post_out.d, (size_t)M * sizeof(double), cudaMemcpyDeviceToHost, s.stream));
-    CUDA_TRY(cudaStreamSynchronize(s.stream));
+    CUDA_TRY(posterior_launch(M, s.post_ll.d, logprior ? s.post_prior.d : nullptr, s.post_out.d, st));
+    CUDA_TRY(cudaMemcpyAsync(s.post_out.h, s.post_out.d, (size_t)M * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
     std::memcpy(out_post, s.post_out.h, (size_t)M * sizeof(double));
     return 0;
 }
@@ -850,19 +829,20 @@ int posterior_on_devices(gpcc_ctx* ctx, int L, int M, const GatherIO& io, const 
                 for (int q = 2; q < REC; ++q) r[q] = 0.0;
             }
         }
-        CUDA_TRY(cudaMemcpyAsync(s.gat_send.d, h, (size_t)per * REC * sizeof(double), cudaMemcpyHostToDevice, s.stream));
-        CUDA_TRY(posterior_partial_launch(per, REC, JCOL, s.gat_send.d, s.stream));
-        d_send[di] = s.gat_send.d; d_recv[di] = s.gat_recv.d; streams[di] = s.stream;
+        CUDA_TRY(cudaMemcpyAsync(s.gat_send.d, h, (size_t)per * REC * sizeof(double), cudaMemcpyHostToDevice, s.stream.get()));
+        CUDA_TRY(posterior_partial_launch(per, REC, JCOL, s.gat_send.d, s.stream.get()));
+        d_send[di] = s.gat_send.d; d_recv[di] = s.gat_recv.d; streams[di] = s.stream.get();
     }
     std::string err;
     if (nccl_bridge_allgather(ctx->nccl, d_send, d_recv, (int)blk, streams, err)) return fail(2001, "ncclAllGather: " + err);
     DeviceState& s0 = ctx->ds[0];
     CUDA_TRY(cudaSetDevice(s0.dev));
+    cudaStream_t st0 = s0.stream.get();
     CUDA_TRY(s0.gat_post.reserve((size_t)per * G));
-    CUDA_TRY(posterior_combine_launch(G, per, REC, JCOL, s0.gat_recv.d, s0.gat_post.d, s0.stream));
-    CUDA_TRY(cudaMemcpyAsync(s0.gat_post.h, s0.gat_post.d, (size_t)per * G * sizeof(double), cudaMemcpyDeviceToHost, s0.stream));
-    CUDA_TRY(cudaMemcpyAsync(s0.gat_recv.h, s0.gat_recv.d, blk * G * sizeof(double), cudaMemcpyDeviceToHost, s0.stream));
-    CUDA_TRY(cudaStreamSynchronize(s0.stream));
+    CUDA_TRY(posterior_combine_launch(G, per, REC, JCOL, s0.gat_recv.d, s0.gat_post.d, st0));
+    CUDA_TRY(cudaMemcpyAsync(s0.gat_post.h, s0.gat_post.d, (size_t)per * G * sizeof(double), cudaMemcpyDeviceToHost, st0));
+    CUDA_TRY(cudaMemcpyAsync(s0.gat_recv.h, s0.gat_recv.d, blk * G * sizeof(double), cudaMemcpyDeviceToHost, st0));
+    CUDA_TRY(cudaStreamSynchronize(st0));
     for (int g = 0; g < G; ++g)
         for (int k = 0; k < per; ++k) {
             const int m = g + k * G;

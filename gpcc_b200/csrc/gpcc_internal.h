@@ -1,12 +1,54 @@
 // Internal declarations shared by the CUDA translation units of libgpcc_b200.so.
 #pragma once
 #include <cuda_runtime.h>
+#include <algorithm>
+#include <memory>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 namespace gpcc {
 
 constexpr int MAX_BANDS = 8;   // == GPCC_MAX_BANDS
+
+// Device array that only ever grows, to exactly the size asked for (no cudaMalloc on repeated calls of the same size).
+// It owns its memory and frees it when destroyed; the owner makes its device current first.
+template <class T>
+struct DevArray {
+    T* d = nullptr;
+    size_t cap = 0;
+    DevArray() = default;
+    DevArray(const DevArray&) = delete;
+    DevArray& operator=(const DevArray&) = delete;
+    ~DevArray() { if (d) cudaFree(d); }
+    cudaError_t reserve(size_t n) {
+        if (n <= cap) return cudaSuccess;
+        if (d) cudaFree(d);
+        d = nullptr; cap = 0;
+        cudaError_t e = cudaMalloc(&d, std::max<size_t>(n, 1) * sizeof(T));
+        if (e == cudaSuccess) cap = n;
+        else d = nullptr;
+        return e;
+    }
+};
+
+// Owning stream and event handles (cudaStream_t and cudaEvent_t are pointer types).
+struct StreamDestroy { void operator()(cudaStream_t s) const { cudaStreamDestroy(s); } };
+struct EventDestroy { void operator()(cudaEvent_t e) const { cudaEventDestroy(e); } };
+using Stream = std::unique_ptr<std::remove_pointer_t<cudaStream_t>, StreamDestroy>;
+using Event = std::unique_ptr<std::remove_pointer_t<cudaEvent_t>, EventDestroy>;
+inline cudaError_t create_stream(Stream& s, int priority) {
+    cudaStream_t h = nullptr;
+    cudaError_t e = cudaStreamCreateWithPriority(&h, cudaStreamNonBlocking, priority);
+    if (e == cudaSuccess) s.reset(h);
+    return e;
+}
+inline cudaError_t create_event(Event& ev, unsigned flags = cudaEventDefault) {
+    cudaEvent_t h = nullptr;
+    cudaError_t e = cudaEventCreateWithFlags(&h, flags);
+    if (e == cudaSuccess) ev.reset(h);
+    return e;
+}
 
 // Problem data resident on one device (uploaded once by gpcc_problem_create).
 struct DevProblem {
@@ -75,9 +117,9 @@ struct FitBuffers {           // all on the device
 cudaError_t small_fit_launch(const DevProblem& p, const FitParams& fp, const FitBuffers& fb, cudaStream_t stream);
 
 // ---- large-N path: tiled matrix in HBM, blocked sweep with DMMA trailing updates (large_path.cu) --
-struct LargeWorkspace {
-    void* impl = nullptr;
-};
+struct LargeImpl;
+struct LargeImplDelete { void operator()(LargeImpl* w) const; };
+using LargeWorkspace = std::unique_ptr<LargeImpl, LargeImplDelete>;   // built on first use by large_eval
 struct LargeTimings {
     double ms_assembly = 0, ms_factor = 0, ms_gradreduce = 0;
     long long launches = 0;
@@ -87,7 +129,6 @@ struct LargeTimings {
 };
 cudaError_t large_eval(const DevProblem& p, const EvalBatch& b, LargeWorkspace& ws, cudaStream_t stream, bool profile,
                        LargeTimings* timings);
-void large_workspace_release(LargeWorkspace& ws);
 
 // ---- posterior over candidates (posterior.cu): src/getprobabilities.jl:10-20 --------------------
 cudaError_t posterior_launch(int M, const double* d_ll, const double* d_logprior, double* d_out, cudaStream_t stream,

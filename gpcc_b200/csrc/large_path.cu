@@ -32,6 +32,7 @@
 #include <cstdio>
 #include <cstring>
 #include <map>
+#include <memory>
 
 namespace gpcc {
 namespace {
@@ -920,107 +921,107 @@ __global__ void dump_chol_kernel(EvalBatch b, int e0, LargeArgs a) {
     }
 }
 
-struct LargeImpl {
-    int N = 0, T = 0, Np = 0, B = 0;
-    size_t mat_stride = 0;
-    double *mats = nullptr, *Pws = nullptr, *Xws = nullptr, *Linv = nullptr, *Dinv = nullptr, *rvec = nullptr, *zk = nullptr,
-           *scal = nullptr, *tsh = nullptr, *av = nullptr, *part = nullptr, *epart = nullptr;
-    int* info = nullptr;
-    int *eidx_d = nullptr, *slot_d = nullptr;    // [B] per-wave maps of the last-band cache
-    double *XC = nullptr, *AC = nullptr, *RC = nullptr;   // the cache itself: [slots][...]
-    int cache_slots = 0, cache_T = 0, cache_Tc = 0, cache_Tq = 0;
-    size_t xc_stride = 0, ac_stride = 0, rc_stride = 0;
-    cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
-    cudaStream_t bulk = nullptr;                 // second stream: the bulk of each trailing update (look-ahead)
-    cudaEvent_t ev_panel[2] = {nullptr, nullptr}, ev_bulk[2] = {nullptr, nullptr}, ev_join = nullptr;
-    bool attr_set = false;
-    void release_cache() {
-        for (double* q : {XC, AC, RC}) if (q) cudaFree(q);
-        XC = AC = RC = nullptr;
-        cache_slots = 0;
-    }
-    void release() {
-        for (double* p : {mats, Pws, Xws, Linv, Dinv, rvec, zk, scal, tsh, av, part, epart}) if (p) cudaFree(p);
-        if (info) cudaFree(info);
-        for (int* q : {eidx_d, slot_d}) if (q) cudaFree(q);
-        eidx_d = slot_d = nullptr;
-        release_cache();
-        for (auto& e : ev) if (e) { cudaEventDestroy(e); e = nullptr; }
-        for (auto& e : ev_panel) if (e) { cudaEventDestroy(e); e = nullptr; }
-        for (auto& e : ev_bulk) if (e) { cudaEventDestroy(e); e = nullptr; }
-        if (ev_join) { cudaEventDestroy(ev_join); ev_join = nullptr; }
-        if (bulk) { cudaStreamDestroy(bulk); bulk = nullptr; }
-        mats = Pws = Xws = Linv = Dinv = rvec = zk = scal = tsh = av = part = epart = nullptr;
-        info = nullptr;
-        B = 0;
-    }
+}  // namespace
+
+// Last-band cache: [slots][...] per array.
+struct TauCache {
+    DevArray<double> XC, AC, RC;
+    int slots = 0, Tc = 0, Tq = 0;
+    size_t xc_stride = 0, ac_stride = 0, rc_stride = 0;   // doubles per slot
 };
 
-cudaError_t ensure(LargeImpl& w, int N, int want_B) {
+// Workspace of one shape: N, and B matrices per wave.  ensure() builds a new one whenever N changes or B must grow.
+struct LargeImpl {
+    int dev = 0;
+    int N = 0, T = 0, Np = 0, B = 0;
+    size_t mat_stride = 0;
+    DevArray<double> mats, Pws, Xws, Linv, Dinv, rvec, zk, scal, tsh, av, part, epart;
+    DevArray<int> info;
+    DevArray<int> eidx_d, slot_d;                // [B] per-wave maps of the last-band cache
+    std::unique_ptr<TauCache> cache;
+    Event ev[4];
+    Stream bulk;                                 // second stream: the bulk of each trailing update (look-ahead)
+    Event ev_panel[2], ev_bulk[2];
+    bool attr_set = false;
+    ~LargeImpl() { cudaSetDevice(dev); }
+};
+
+void LargeImplDelete::operator()(LargeImpl* w) const { delete w; }
+
+namespace {
+
+// The old workspace is freed before the new one is allocated, so that peak memory is one workspace.  On failure `ws` is
+// empty and the next call allocates again.
+cudaError_t ensure(LargeWorkspace& ws, int N, int want_B) {
     const int T = (N + BT - 1) / BT;
-    if (w.N == N && w.B >= want_B) return cudaSuccess;
-    w.release();
-    w.N = N; w.T = T; w.Np = T * BT;
-    const size_t ntiles = (size_t)T * (T + 1) / 2;
-    w.mat_stride = ntiles * TILE_ELEMS;
-    size_t free_b = 0, total_b = 0;
-    cudaError_t e = cudaMemGetInfo(&free_b, &total_b);
+    if (ws && ws->N == N && ws->B >= want_B) return cudaSuccess;
+    ws.reset();
+    LargeWorkspace w(new LargeImpl());
+    cudaError_t e = cudaGetDevice(&w->dev);
     if (e != cudaSuccess) return e;
-    const size_t per = (w.mat_stride + 3 * (size_t)T * TILE_ELEMS + 2 * TILE_ELEMS + (size_t)T * T * BT + ntiles + 4 * (size_t)w.Np) * sizeof(double);
+    const int Np = T * BT;
+    const size_t ntiles = (size_t)T * (T + 1) / 2;
+    const size_t mat_stride = ntiles * TILE_ELEMS;
+    size_t free_b = 0, total_b = 0;
+    e = cudaMemGetInfo(&free_b, &total_b);
+    if (e != cudaSuccess) return e;
+    const size_t per = (mat_stride + 3 * (size_t)T * TILE_ELEMS + 2 * TILE_ELEMS + (size_t)T * T * BT + ntiles + 4 * (size_t)Np) * sizeof(double);
     int B = want_B;
     while (B > 1 && (size_t)B * per > free_b / 2) B /= 2;
     if ((size_t)B * per > free_b) return cudaErrorMemoryAllocation;
-    w.B = B;
-#define ALLOC(ptr, n) if ((e = cudaMalloc(&ptr, (size_t)(n) * sizeof(*ptr))) != cudaSuccess) return e;
-    ALLOC(w.mats, (size_t)B * w.mat_stride)
-    ALLOC(w.Pws, (size_t)B * T * TILE_ELEMS)
-    ALLOC(w.Xws, (size_t)2 * B * T * TILE_ELEMS)
-    ALLOC(w.Linv, (size_t)B * TILE_ELEMS)
-    ALLOC(w.Dinv, (size_t)B * TILE_ELEMS)
-    ALLOC(w.rvec, (size_t)B * w.Np)
-    ALLOC(w.zk, (size_t)B * BT)
-    ALLOC(w.scal, (size_t)B * 4)
-    ALLOC(w.tsh, (size_t)B * w.Np)
-    ALLOC(w.av, (size_t)B * w.Np)
-    ALLOC(w.part, (size_t)B * T * T * BT)
-    ALLOC(w.epart, (size_t)B * ntiles)
-    ALLOC(w.info, (size_t)B)
-    ALLOC(w.eidx_d, (size_t)B)
-    ALLOC(w.slot_d, (size_t)B)
+#define ALLOC(arr, n) if ((e = w->arr.reserve((size_t)(n))) != cudaSuccess) return e;
+    ALLOC(mats, (size_t)B * mat_stride)
+    ALLOC(Pws, (size_t)B * T * TILE_ELEMS)
+    ALLOC(Xws, (size_t)2 * B * T * TILE_ELEMS)
+    ALLOC(Linv, (size_t)B * TILE_ELEMS)
+    ALLOC(Dinv, (size_t)B * TILE_ELEMS)
+    ALLOC(rvec, (size_t)B * Np)
+    ALLOC(zk, (size_t)B * BT)
+    ALLOC(scal, (size_t)B * 4)
+    ALLOC(tsh, (size_t)B * Np)
+    ALLOC(av, (size_t)B * Np)
+    ALLOC(part, (size_t)B * T * T * BT)
+    ALLOC(epart, (size_t)B * ntiles)
+    ALLOC(info, (size_t)B)
+    ALLOC(eidx_d, (size_t)B)
+    ALLOC(slot_d, (size_t)B)
 #undef ALLOC
-    for (auto& ev : w.ev) if ((e = cudaEventCreate(&ev)) != cudaSuccess) return e;
-    for (auto& ev : w.ev_panel) if ((e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming)) != cudaSuccess) return e;
-    for (auto& ev : w.ev_bulk) if ((e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming)) != cudaSuccess) return e;
-    if ((e = cudaEventCreateWithFlags(&w.ev_join, cudaEventDisableTiming)) != cudaSuccess) return e;
+    for (auto& ev : w->ev) if ((e = create_event(ev)) != cudaSuccess) return e;
+    for (auto& ev : w->ev_panel) if ((e = create_event(ev, cudaEventDisableTiming)) != cudaSuccess) return e;
+    for (auto& ev : w->ev_bulk) if ((e = create_event(ev, cudaEventDisableTiming)) != cudaSuccess) return e;
     int prio_lo = 0, prio_hi = 0;
     if ((e = cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi)) != cudaSuccess) return e;
-    if ((e = cudaStreamCreateWithPriority(&w.bulk, cudaStreamNonBlocking, prio_lo)) != cudaSuccess) return e;
+    if ((e = create_stream(w->bulk, prio_lo)) != cudaSuccess) return e;
+    w->N = N; w->T = T; w->Np = Np; w->B = B; w->mat_stride = mat_stride;
+    ws = std::move(w);
     return cudaSuccess;
 }
 
-// Last-band cache: room for `slots` distinct values of the last delay.  Returns false (no error) when it does not fit.
+// Last-band cache: room for `slots` distinct values of the last delay.  Returns false (no error) when it does not fit; the
+// cache is then empty.
 bool ensure_cache(LargeImpl& w, int slots, int Tq, int Tc) {
+    const TauCache* old = w.cache.get();
+    if (old && old->slots >= slots && old->Tc == Tc && old->Tq == Tq) return true;
+    w.cache.reset();
+    auto c = std::make_unique<TauCache>();
     const int nC = w.T - Tc;
-    if (w.cache_slots >= slots && w.cache_T == w.T && w.cache_Tc == Tc && w.cache_Tq == Tq) return true;
-    w.release_cache();
     const int wanted = slots;
-    w.xc_stride = (size_t)Tq * nC * TILE_ELEMS;
-    w.ac_stride = (size_t)nC * (nC + 1) / 2 * TILE_ELEMS;
-    w.rc_stride = (size_t)nC * BT;
-    const size_t bytes = (size_t)slots * (w.xc_stride + w.ac_stride + w.rc_stride) * sizeof(double);
+    c->xc_stride = (size_t)Tq * nC * TILE_ELEMS;
+    c->ac_stride = (size_t)nC * (nC + 1) / 2 * TILE_ELEMS;
+    c->rc_stride = (size_t)nC * BT;
+    const size_t bytes = (size_t)slots * (c->xc_stride + c->ac_stride + c->rc_stride) * sizeof(double);
     size_t free_b = 0, total_b = 0;
     if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess || bytes > free_b / 2) return false;
     // head-room (a grid has ~10^2 distinct delays per band): a first call with a few candidates must not force a re-allocation,
     // and its allocator stall, into the next one
     while (slots < 128 && (size_t)(2 * slots) * (bytes / wanted) <= free_b / 8) slots *= 2;
-    if (cudaMalloc(&w.XC, (size_t)slots * w.xc_stride * sizeof(double)) != cudaSuccess ||
-        cudaMalloc(&w.AC, (size_t)slots * w.ac_stride * sizeof(double)) != cudaSuccess ||
-        cudaMalloc(&w.RC, (size_t)slots * w.rc_stride * sizeof(double)) != cudaSuccess) {
+    if (c->XC.reserve((size_t)slots * c->xc_stride) != cudaSuccess || c->AC.reserve((size_t)slots * c->ac_stride) != cudaSuccess ||
+        c->RC.reserve((size_t)slots * c->rc_stride) != cudaSuccess) {
         cudaGetLastError();
-        w.release_cache();
         return false;
     }
-    w.cache_slots = slots; w.cache_T = w.T; w.cache_Tc = Tc; w.cache_Tq = Tq;
+    c->slots = slots; c->Tc = Tc; c->Tq = Tq;
+    w.cache = std::move(c);
     return true;
 }
 
@@ -1029,22 +1030,24 @@ bool ensure_cache(LargeImpl& w, int slots, int Tq, int Tc) {
 template <int KID>
 cudaError_t run_wave(const DevProblem& p, const EvalBatch& b, int e0, int nb, int Tp, LargeImpl& w, cudaStream_t st, bool profile,
                      LargeTimings* tm, int cmode = 0, int Tq = 0, int Tc = 0, const int* h_eidx = nullptr, const int* h_slot = nullptr) {
-    LargeArgs a;
+    LargeArgs a{};
     a.N = p.N; a.L = p.L; a.T = w.T; a.Np = w.Np; a.kid = KID;
     a.sweep = b.want_grad ? 1 : 0;
     a.Tp = a.sweep ? 0 : Tp;
     a.mode_postb = b.mode_postb;
-    a.mats = w.mats; a.Pws = w.Pws; a.Xws = w.Xws; a.Linv = w.Linv; a.Dinv = w.Dinv; a.rvec = w.rvec; a.zk = w.zk;
-    a.scal = w.scal; a.info = w.info; a.tsh = w.tsh; a.av = w.av; a.part = w.part; a.epart = w.epart; a.mat_stride = w.mat_stride;
+    a.mats = w.mats.d; a.Pws = w.Pws.d; a.Xws = w.Xws.d; a.Linv = w.Linv.d; a.Dinv = w.Dinv.d; a.rvec = w.rvec.d; a.zk = w.zk.d;
+    a.scal = w.scal.d; a.info = w.info.d; a.tsh = w.tsh.d; a.av = w.av.d; a.part = w.part.d; a.epart = w.epart.d; a.mat_stride = w.mat_stride;
     a.x_parity_stride = (size_t)w.B * w.T * TILE_ELEMS;
     a.cmode = a.sweep ? 0 : cmode; a.Tq = Tq; a.Tc = Tc;
-    a.eidx = nullptr; a.slot = w.slot_d;
-    a.XC = w.XC; a.AC = w.AC; a.RC = w.RC; a.xc_stride = w.xc_stride; a.ac_stride = w.ac_stride; a.rc_stride = w.rc_stride;
+    a.eidx = nullptr; a.slot = w.slot_d.d;
+    if (const TauCache* c = w.cache.get()) {
+        a.XC = c->XC.d; a.AC = c->AC.d; a.RC = c->RC.d; a.xc_stride = c->xc_stride; a.ac_stride = c->ac_stride; a.rc_stride = c->rc_stride;
+    }
     if (a.cmode) {      // pageable source: the copy is staged before the call returns; ordered behind the previous wave on `st`
-        cudaMemcpyAsync(w.slot_d, h_slot, (size_t)nb * sizeof(int), cudaMemcpyHostToDevice, st);
+        cudaMemcpyAsync(w.slot_d.d, h_slot, (size_t)nb * sizeof(int), cudaMemcpyHostToDevice, st);
         if (a.cmode == 1) {
-            cudaMemcpyAsync(w.eidx_d, h_eidx, (size_t)nb * sizeof(int), cudaMemcpyHostToDevice, st);
-            a.eidx = w.eidx_d;
+            cudaMemcpyAsync(w.eidx_d.d, h_eidx, (size_t)nb * sizeof(int), cudaMemcpyHostToDevice, st);
+            a.eidx = w.eidx_d.d;
             a.Tp = Tq;      // the matrices of a FILL wave share band 1 (same hyper-parameters, same first delay)
         }
     }
@@ -1064,7 +1067,7 @@ cudaError_t run_wave(const DevProblem& p, const EvalBatch& b, int e0, int nb, in
         update_half_kernel<<<dim3(2 * ntile, nb), 128, half_smem, strm>>>(a, kk, phase);
     };
     long long launches = 0;
-    if (profile) cudaEventRecord(w.ev[0], st);
+    if (profile) cudaEventRecord(w.ev[0].get(), st);
     prep_kernel<<<dim3((w.Np + 255) / 256, nb), 256, 0, st>>>(p, b, e0, a);
     assemble_kernel<KID><<<dim3(ntiles, nb), 256, 0, st>>>(p, b, e0, a);
     launches += 2;
@@ -1078,7 +1081,7 @@ cudaError_t run_wave(const DevProblem& p, const EvalBatch& b, int e0, int nb, in
         tm->assembly_bytes += ((long long)nb * own + lead) * (long long)(TILE_ELEMS * sizeof(double));
         (void)nM;
     }
-    if (profile) cudaEventRecord(w.ev[1], st);
+    if (profile) cudaEventRecord(w.ev[1].get(), st);
     // Look-ahead schedule on two streams.  Critical stream `st`: pivot_k, gather_k, panel_k, then the part of update k
     // that touches block row/column k+1, so that pivot/gather/panel of step k+1 start while the bulk stream is still
     // busy with the rest of update k (the pivot kernel occupies one SM per matrix; without look-ahead the other SMs idle).
@@ -1099,27 +1102,27 @@ cudaError_t run_wave(const DevProblem& p, const EvalBatch& b, int e0, int nb, in
         const int n_rest_side = a.sweep ? T - 2 : T - 2 - k;
         const int n_rest = n_rest_side > 0 ? n_rest_side * (n_rest_side + 1) / 2 : 0;
         if (!lookahead || !has_next) {
-            if (bulk_pending[(k + 1) & 1]) { cudaStreamWaitEvent(st, w.ev_bulk[(k + 1) & 1], 0); bulk_pending[(k + 1) & 1] = false; }
+            if (bulk_pending[(k + 1) & 1]) { cudaStreamWaitEvent(st, w.ev_bulk[(k + 1) & 1].get(), 0); bulk_pending[(k + 1) & 1] = false; }
             launch_update(nI * (nI + 1) / 2, 0, k, st);
             ++launches;
             continue;
         }
-        cudaEventRecord(w.ev_panel[k & 1], st);
+        cudaEventRecord(w.ev_panel[k & 1].get(), st);
         // the critical tiles were last written by the bulk part of update k-1
-        if (bulk_pending[(k + 1) & 1]) { cudaStreamWaitEvent(st, w.ev_bulk[(k + 1) & 1], 0); bulk_pending[(k + 1) & 1] = false; }
+        if (bulk_pending[(k + 1) & 1]) { cudaStreamWaitEvent(st, w.ev_bulk[(k + 1) & 1].get(), 0); bulk_pending[(k + 1) & 1] = false; }
         launch_update(n_crit, 1, k, st);
         ++launches;
         if (n_rest > 0) {
-            cudaStreamWaitEvent(w.bulk, w.ev_panel[k & 1], 0);
-            launch_update(n_rest, 2, k, w.bulk);
-            cudaEventRecord(w.ev_bulk[k & 1], w.bulk);
+            cudaStreamWaitEvent(w.bulk.get(), w.ev_panel[k & 1].get(), 0);
+            launch_update(n_rest, 2, k, w.bulk.get());
+            cudaEventRecord(w.ev_bulk[k & 1].get(), w.bulk.get());
             bulk_pending[k & 1] = true;
             ++launches;
         }
     }
     for (int q = 0; q < 2; ++q)
-        if (bulk_pending[q]) cudaStreamWaitEvent(st, w.ev_bulk[q], 0);
-    if (profile) cudaEventRecord(w.ev[2], st);
+        if (bulk_pending[q]) cudaStreamWaitEvent(st, w.ev_bulk[q].get(), 0);
+    if (profile) cudaEventRecord(w.ev[2].get(), st);
     if (a.cmode == 1) {
         const int nC = T - Tc;
         export_state_kernel<<<dim3(nC * (nC + 1) / 2 + 1, nb), 256, 0, st>>>(a);
@@ -1134,16 +1137,16 @@ cudaError_t run_wave(const DevProblem& p, const EvalBatch& b, int e0, int nb, in
         dump_chol_kernel<<<dim3(592, nb), 256, 0, st>>>(b, e0, a);
         ++launches;
     }
-    if (profile) cudaEventRecord(w.ev[3], st);
+    if (profile) cudaEventRecord(w.ev[3].get(), st);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     if (profile) {
-        e = cudaEventSynchronize(w.ev[3]);
+        e = cudaEventSynchronize(w.ev[3].get());
         if (e != cudaSuccess) return e;
         float t01 = 0, t12 = 0, t23 = 0;
-        cudaEventElapsedTime(&t01, w.ev[0], w.ev[1]);
-        cudaEventElapsedTime(&t12, w.ev[1], w.ev[2]);
-        cudaEventElapsedTime(&t23, w.ev[2], w.ev[3]);
+        cudaEventElapsedTime(&t01, w.ev[0].get(), w.ev[1].get());
+        cudaEventElapsedTime(&t12, w.ev[1].get(), w.ev[2].get());
+        cudaEventElapsedTime(&t23, w.ev[2].get(), w.ev[3].get());
         tm->ms_assembly += t01; tm->ms_factor += t12; tm->ms_gradreduce += t23;
     }
     tm->launches += launches;
@@ -1154,15 +1157,14 @@ cudaError_t run_wave(const DevProblem& p, const EvalBatch& b, int e0, int nb, in
 
 cudaError_t large_eval(const DevProblem& p, const EvalBatch& b, LargeWorkspace& ws, cudaStream_t stream, bool profile,
                        LargeTimings* tm) {
-    if (!ws.impl) ws.impl = new LargeImpl();
-    LargeImpl& w = *static_cast<LargeImpl*>(ws.impl);
     // Matrices per wave.  The pivot kernel is one CTA per matrix and its 128-column chain is the critical path of a block step;
     // a wave must hold enough matrices for the DMMA trailing updates of the others to cover it (measured at N = 6144: 8 per
     // wave 21.6 TFLOP/s, pivot bound; 32 per wave update bound).  ensure() halves the wave if memory is short.
     static const int wave_env = getenv("GPCC_LARGE_WAVE") ? atoi(getenv("GPCC_LARGE_WAVE")) : 0;
     const int want_B = std::min(b.M, wave_env > 0 ? wave_env : (p.N >= 8192 ? 16 : (p.N >= 4096 ? 32 : (p.N >= 1024 ? 128 : 512))));
-    cudaError_t e = ensure(w, p.N, std::max(want_B, 1));
+    cudaError_t e = ensure(ws, p.N, std::max(want_B, 1));
     if (e != cudaSuccess) return e;
+    LargeImpl& w = *ws;
     // Structure reuse across the grid (SURVEY.md 8f item 2; src/delayedCovariance.jl:23-31: block (l, m) of the covariance depends
     // on tau_l - tau_m only).  Evaluations that share the hyper-parameters and the delays of all bands but the last have an
     // identical leading principal block; in forward (Cholesky) mode a wave made of such a run factorises that block ONCE.
@@ -1252,14 +1254,6 @@ cudaError_t large_eval(const DevProblem& p, const EvalBatch& b, LargeWorkspace& 
     }
     tm->shared_prefix_evals += shared_evals;
     return cudaSuccess;
-}
-
-void large_workspace_release(LargeWorkspace& ws) {
-    if (!ws.impl) return;
-    LargeImpl* w = static_cast<LargeImpl*>(ws.impl);
-    w->release();
-    delete w;
-    ws.impl = nullptr;
 }
 
 }  // namespace gpcc

@@ -23,6 +23,7 @@
 #include <cmath>
 #include <cstring>
 #include <limits>
+#include <memory>
 
 using namespace gpcc;
 
@@ -44,38 +45,23 @@ struct PostB {      // posterior of the shifts, device resident
     double S[GPCC_MAX_BANDS][GPCC_MAX_BANDS];
 };
 
-template <class T>
-struct GrowBuf {    // device buffer that only ever grows (no cudaMalloc on repeated calls of the same size)
-    T* d = nullptr;
-    size_t cap = 0;
-    cudaError_t reserve(size_t n) {
-        if (n <= cap) return cudaSuccess;
-        if (d) cudaFree(d);
-        d = nullptr; cap = 0;
-        cudaError_t e = cudaMalloc(&d, std::max<size_t>(n, 1) * sizeof(T));
-        if (e == cudaSuccess) cap = n;
-        return e;
-    }
-    void release() { if (d) cudaFree(d); d = nullptr; cap = 0; }
-};
-
 }  // namespace
 
 struct gpcc_fit_state {
-    gpcc_problem* p = nullptr;
+    gpcc_problem* p = nullptr;   // used by the calls, never by the destructor: the problem may be destroyed first
     int dev = 0;
     int N = 0, L = 0, kernel_id = 0;
     HyperDev h{};
-    double* Lc = nullptr;      // [N][N] column-major Cholesky factor of K + Sobs (lower)
-    double* VU = nullptr;      // [N][L+1] column-major: V = Lc^-1 Q, last column u = Lc^-1 Y
-    double* w = nullptr;       // [N]  Lc^-1 (Y - Q mu_postb)
-    PostB* postb_d = nullptr;  // device copy
+    DevArray<double> Lc;       // [N][N] column-major Cholesky factor of K + Sobs (lower)
+    DevArray<double> VU;       // [N][L+1] column-major: V = Lc^-1 Q, last column u = Lc^-1 Y
+    DevArray<double> w;        // [N]  Lc^-1 (Y - Q mu_postb)
+    DevArray<PostB> postb_d;   // device copy
     PostB postb_h{};           // host copy
-    int* band_start_d = nullptr;
     // scratch of the prediction calls, kept between calls
-    GrowBuf<double> Z, R, G, S, mu, sd, tt, extra, yv, zv, scal;
-    GrowBuf<int> bandt, info;
+    DevArray<double> Z, R, G, S, mu, sd, tt, extra, yv, zv, scal;
+    DevArray<int> bandt, info;
     long long n_factorisations = 0;   // diagnostics: how often the N^3 work ran for this state (must stay 1)
+    ~gpcc_fit_state() { cudaSetDevice(dev); }
 };
 
 namespace {
@@ -441,27 +427,18 @@ int check_hyper(const gpcc_problem* p, const double* delays, const double* alpha
     return 0;
 }
 
-void free_state(gpcc_fit_state* s) {
-    cudaSetDevice(s->dev);
-    for (void* q : {(void*)s->Lc, (void*)s->VU, (void*)s->w, (void*)s->postb_d, (void*)s->band_start_d}) if (q) cudaFree(q);
-    s->Z.release(); s->R.release(); s->G.release(); s->S.release(); s->mu.release(); s->sd.release(); s->tt.release();
-    s->extra.release(); s->yv.release(); s->zv.release(); s->scal.release(); s->bandt.release(); s->info.release();
-    delete s;
-}
-
 int create_state(gpcc_problem* p, const double* delays, const double* alpha, double rho, gpcc_fit_state** out) {
     const int L = p->L, N = p->N;
     DeviceState& ds = p->ctx->ds[0];
     CUDA_TRY(cudaSetDevice(ds.dev));
-    gpcc_fit_state* s = new gpcc_fit_state();
+    std::unique_ptr<gpcc_fit_state> s(new gpcc_fit_state());
     s->p = p; s->dev = ds.dev; s->N = N; s->L = L; s->kernel_id = p->kernel_id;
     s->h.L = L; s->h.rho = rho;
     for (int l = 0; l < L; ++l) { s->h.delays[l] = delays[l]; s->h.alpha[l] = alpha[l]; }
-    struct Guard { gpcc_fit_state* s; ~Guard() { if (s) free_state(s); } } guard{s};
-    CUDA_TRY(cudaMalloc(&s->Lc, (size_t)N * N * sizeof(double)));
-    CUDA_TRY(cudaMalloc(&s->VU, (size_t)N * (L + 1) * sizeof(double)));
-    CUDA_TRY(cudaMalloc(&s->w, (size_t)N * sizeof(double)));
-    CUDA_TRY(cudaMalloc(&s->postb_d, sizeof(PostB)));
+    CUDA_TRY(s->Lc.reserve((size_t)N * N));
+    CUDA_TRY(s->VU.reserve((size_t)N * (L + 1)));
+    CUDA_TRY(s->w.reserve(N));
+    CUDA_TRY(s->postb_d.reserve(1));
     // ---- A = K + Sobs (no B) = Lc Lc': blocked right-looking Cholesky with DMMA trailing updates (large_path.cu) ----
     int rc = reserve_eval(p, 0, 1);
     if (rc) return rc;
@@ -469,32 +446,31 @@ int create_state(gpcc_problem* p, const double* delays, const double* alpha, dou
     std::memcpy(q.delays.h, delays, L * sizeof(double));
     std::memcpy(q.alpha.h, alpha, L * sizeof(double));
     q.rho.h[0] = rho;
-    cudaStream_t st = ds.stream;
+    cudaStream_t st = ds.stream.get();
     CUDA_TRY(cudaMemcpyAsync(q.delays.d, q.delays.h, L * sizeof(double), cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(q.alpha.d, q.alpha.h, L * sizeof(double), cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(q.rho.d, q.rho.h, sizeof(double), cudaMemcpyHostToDevice, st));
     EvalBatch b;
     b.M = 1; b.delays = q.delays.d; b.alpha = q.alpha.d; b.rho = q.rho.d; b.want_grad = 0;
-    b.ll = q.ll.d; b.grad = q.grad.d; b.info = q.info.d; b.mode_postb = 1; b.dump_chol = s->Lc;
+    b.ll = q.ll.d; b.grad = q.grad.d; b.info = q.info.d; b.mode_postb = 1; b.dump_chol = s->Lc.d;
     LargeTimings lt;
     CUDA_TRY(large_eval(p->pd[0].dp, b, ds.large, st, false, &lt));
     s->n_factorisations += 1;
     CUDA_TRY(cudaMemcpyAsync(q.info.h, q.info.d, sizeof(int), cudaMemcpyDeviceToHost, st));
     // ---- V = Lc^-1 Q, u = Lc^-1 Y, postb, w ----------------------------------------------------------------------
     const auto& dp = p->pd[0].dp;
-    rhs_qy_kernel<<<(N * (L + 1) + 255) / 256, 256, 0, st>>>(N, L, dp.band, dp.y, s->VU);
-    trsm_lower_kernel<<<(L + 1 + TC - 1) / TC, 256, 0, st>>>(N, L + 1, s->Lc, s->VU);
+    rhs_qy_kernel<<<(N * (L + 1) + 255) / 256, 256, 0, st>>>(N, L, dp.band, dp.y, s->VU.d);
+    trsm_lower_kernel<<<(L + 1 + TC - 1) / TC, 256, 0, st>>>(N, L + 1, s->Lc.d, s->VU.d);
     CUDA_TRY(s->scal.reserve(2 * GPCC_MAX_BANDS + 2));
     CUDA_TRY(cudaMemcpyAsync(s->scal.d, p->Sigmab.data(), L * sizeof(double), cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(s->scal.d + GPCC_MAX_BANDS, p->mub.data(), L * sizeof(double), cudaMemcpyHostToDevice, st));
-    state_finish_kernel<<<1, 256, 0, st>>>(N, L, s->VU, s->scal.d, s->scal.d + GPCC_MAX_BANDS, s->postb_d, s->w);
+    state_finish_kernel<<<1, 256, 0, st>>>(N, L, s->VU.d, s->scal.d, s->scal.d + GPCC_MAX_BANDS, s->postb_d.d, s->w.d);
     CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaMemcpyAsync(&s->postb_h, s->postb_d, sizeof(PostB), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(&s->postb_h, s->postb_d.d, sizeof(PostB), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     if (q.info.h[0] != 0) return fail(-6, "K + Sobs is not positive definite for these hyper-parameters");
     ds.launches += lt.launches + 3;
-    guard.s = nullptr;
-    *out = s;
+    *out = s.release();
     return 0;
 }
 
@@ -503,13 +479,13 @@ int predict_impl(gpcc_fit_state* s, int NT, bool want_sd, bool want_cov, const d
     const int N = s->N, L = s->L;
     const auto& dp = s->p->pd[0].dp;
     cross_cov_kernel<KID><<<dim3((N + 255) / 256, std::min(NT, 32768)), 256, 0, st>>>(N, NT, dp.t, dp.band, s->tt.d, s->bandt.d, s->h, s->Z.d);
-    trsm_lower_kernel<<<std::min((NT + TC - 1) / TC, 65535), 256, 0, st>>>(N, NT, s->Lc, s->Z.d);                 // Z = Lc^-1 k*
-    col_stats_kernel<<<(NT + 7) / 8, 256, 0, st>>>(N, NT, L, s->Z.d, s->VU, s->w, s->bandt.d, s->h, s->postb_d, s->mu.d, s->R.d,
+    trsm_lower_kernel<<<std::min((NT + TC - 1) / TC, 65535), 256, 0, st>>>(N, NT, s->Lc.d, s->Z.d);               // Z = Lc^-1 k*
+    col_stats_kernel<<<(NT + 7) / 8, 256, 0, st>>>(N, NT, L, s->Z.d, s->VU.d, s->w.d, s->bandt.d, s->h, s->postb_d.d, s->mu.d, s->R.d,
                                                   want_sd ? s->sd.d : nullptr);
     if (want_cov) {
         gemm_tn_kernel<<<dim3((NT + 63) / 64, (NT + 63) / 64), 256, 0, st>>>(NT, NT, N, s->Z.d, s->Z.d, s->G.d);   // Z'Z
         pred_cov_kernel<KID><<<dim3((NT + 255) / 256, std::min(NT, 32768)), 256, 0, st>>>(NT, L, s->G.d, s->R.d, s->tt.d, s->bandt.d, s->h,
-                                                                                         s->postb_d, d_extra, s->S.d);
+                                                                                         s->postb_d.d, d_extra, s->S.d);
     }
     CUDA_TRY(cudaGetLastError());
     return 0;
@@ -530,7 +506,7 @@ int predict_common(gpcc_fit_state* s, const int* ntest_per_band, const double* t
     for (int l = 0, k = 0; l < L; ++l) for (int i = 0; i < ntest_per_band[l]; ++i) bandt[k++] = l;
     DeviceState& ds = s->p->ctx->ds[0];
     CUDA_TRY(cudaSetDevice(s->dev));
-    cudaStream_t st = ds.stream;
+    cudaStream_t st = ds.stream.get();
     const bool want_ll = out_ll != nullptr;
     const bool want_cov = out_Sigma || want_ll;
     CUDA_TRY(s->Z.reserve((size_t)N * NT));
@@ -583,13 +559,13 @@ int predict_common(gpcc_fit_state* s, const int* ntest_per_band, const double* t
 int cached_state(gpcc_problem* p, const double* delays, const double* alpha, double rho, gpcc_fit_state** out) {
     int rc = check_hyper(p, delays, alpha, rho);
     if (rc) return rc;
-    gpcc_fit_state* c = p->cached_state;
+    gpcc_fit_state* c = p->cached_state.get();
     if (c && c->h.rho == rho && std::memcmp(c->h.delays, delays, p->L * sizeof(double)) == 0 &&
         std::memcmp(c->h.alpha, alpha, p->L * sizeof(double)) == 0) { *out = c; return 0; }
-    if (c) { free_state(c); p->cached_state = nullptr; }
+    p->cached_state.reset();
     rc = create_state(p, delays, alpha, rho, &c);
     if (rc) return rc;
-    p->cached_state = c;
+    p->cached_state.reset(c);
     *out = c;
     return 0;
 }
@@ -607,9 +583,7 @@ int gpcc_fit_state_create(gpcc_problem* p, const double* delays, const double* a
 }
 
 int gpcc_fit_state_destroy(gpcc_fit_state* s) {
-    if (!s) return 0;
-    if (s->p && s->p->cached_state == s) s->p->cached_state = nullptr;
-    free_state(s);
+    delete s;
     return 0;
 }
 
@@ -642,11 +616,11 @@ int gpcc_fit_state_sample(gpcc_fit_state* s, unsigned long long seed, int nsampl
     const size_t n = (size_t)N * nsamples;
     DeviceState& ds = s->p->ctx->ds[0];
     CUDA_TRY(cudaSetDevice(s->dev));
-    cudaStream_t st = ds.stream;
+    cudaStream_t st = ds.stream.get();
     CUDA_TRY(s->Z.reserve(n));          // deviates
     CUDA_TRY(s->G.reserve(n));          // draws
     normal_kernel<<<(int)std::min<size_t>(1184, (n / 2 + 255) / 256 + 1), 256, 0, st>>>(n, seed, s->Z.d);
-    trmv_lower_kernel<<<dim3((N + 255) / 256, std::min((nsamples + 3) / 4, 1024)), 256, 0, st>>>(N, nsamples, s->Lc, s->Z.d, s->G.d);
+    trmv_lower_kernel<<<dim3((N + 255) / 256, std::min((nsamples + 3) / 4, 1024)), 256, 0, st>>>(N, nsamples, s->Lc.d, s->Z.d, s->G.d);
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaMemcpyAsync(out_f, s->G.d, n * sizeof(double), cudaMemcpyDeviceToHost, st));
     if (out_z) CUDA_TRY(cudaMemcpyAsync(out_z, s->Z.d, n * sizeof(double), cudaMemcpyDeviceToHost, st));

@@ -21,26 +21,20 @@ const std::string& last_error();
     } while (0)
 
 template <class T>
-struct DevBuf {   // growable device buffer + pinned host mirror
-    T* d = nullptr;
+struct DevBuf : DevArray<T> {   // growable device buffer (1.5x head-room) + pinned host mirror of the same size
     T* h = nullptr;
-    size_t cap = 0;
+    ~DevBuf() { if (h) cudaFreeHost(h); }
     cudaError_t reserve(size_t n) {
-        if (n <= cap) return cudaSuccess;
-        release();
+        if (n <= this->cap) return cudaSuccess;
+        if (h) cudaFreeHost(h);
+        h = nullptr;
         size_t c = std::max<size_t>(n, 1024);
         c = c + c / 2;
-        cudaError_t e = cudaMalloc(&d, c * sizeof(T));
+        cudaError_t e = DevArray<T>::reserve(c);
         if (e != cudaSuccess) return e;
         e = cudaMallocHost(&h, c * sizeof(T));
-        if (e != cudaSuccess) return e;
-        cap = c;
-        return cudaSuccess;
-    }
-    void release() {
-        if (d) cudaFree(d);
-        if (h) cudaFreeHost(h);
-        d = nullptr; h = nullptr; cap = 0;
+        if (e != cudaSuccess) { h = nullptr; this->cap = 0; }   // no mirror: the next reserve allocates both again
+        return e;
     }
 };
 
@@ -50,9 +44,10 @@ struct EvalSlot {
     DevBuf<int> info;
 };
 
+// Everything the context holds on one device.  Members are destroyed after the destructor's body, with `dev` current.
 struct DeviceState {
     int dev = 0;
-    cudaStream_t stream = nullptr;
+    Stream stream;
     EvalSlot slot;
     DevBuf<double> post_ll, post_prior, post_out;   // persistent staging of the posterior kernel (no cudaMalloc/cudaFree per call)
     // staging of the device-resident fit (small_fit.cu)
@@ -60,12 +55,15 @@ struct DeviceState {
     DevBuf<int> fit_iters, fit_nfev, fit_status, fit_order;
     DevBuf<unsigned long long> fit_counters;
     DevBuf<double> gat_send, gat_recv, gat_post;     // all-gather of the grid results (persistent: no cudaMalloc per call)
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;        // around the small-N kernel launch of the call (profiling)
+    Event ev0, ev1;                                  // around the small-N kernel launch of the call (profiling)
     LargeWorkspace large;     // tiled large-N path (large_path.cu)
     // per-call statistics (profiling)
     double ms_eval = 0, ms_assembly = 0, ms_factor = 0, ms_gradreduce = 0;
     long long launches = 0, evals = 0, evals_grad = 0, shared_prefix_evals = 0, tau_cache_evals = 0, assembly_bytes = 0;
+    ~DeviceState() { cudaSetDevice(dev); }
 };
+
+struct FitStateDelete { void operator()(gpcc_fit_state* s) const { gpcc_fit_state_destroy(s); } };
 
 }  // namespace gpcc
 
@@ -77,8 +75,6 @@ struct gpcc_ctx {
     int world = 1, rank = 0;      // > 1 ranks: one process per device, joined by gpcc_ctx_comm_init_rank
 };
 
-struct gpcc_fit_state;
-
 struct gpcc_problem {
     gpcc_ctx* ctx = nullptr;
     int L = 0, N = 0, kernel_id = 0;
@@ -86,13 +82,15 @@ struct gpcc_problem {
     std::vector<double> t, y, sigma, mub, Sigmab, resid, s2, sigb;
     struct PerDev {
         int dev = 0;              // CUDA device id, copied from the context at creation: destroying a problem never reads the context
-        double *t = nullptr, *resid = nullptr, *y = nullptr, *s2 = nullptr, *sigb = nullptr;
-        int* band = nullptr;
+        gpcc::DevArray<double> t, resid, y, s2, sigb;
+        gpcc::DevArray<int> band;
         gpcc::DevProblem dp;
+        ~PerDev() { cudaSetDevice(dev); }
     };
     std::vector<PerDev> pd;
     bool small_path = true;
-    gpcc_fit_state* cached_state = nullptr;   // fitted state of the last gpcc_postb / gpcc_predict* call (predict.cu)
+    // fitted state of the last gpcc_postb / gpcc_predict* call (predict.cu); never handed to a caller
+    std::unique_ptr<gpcc_fit_state, gpcc::FitStateDelete> cached_state;
 };
 
 namespace gpcc {

@@ -7,6 +7,7 @@ the shared leading block and the last-band cache (large_path.cu); the fitted sta
 and one-CTA Cholesky (predict.cu).  A bug in one of them shows only in the calls that select it, so each is selected here
 on purpose.  Tolerances are those of test_gpu_parity.py; "bitwise" means np.array_equal.
 """
+import itertools
 import os
 import subprocess
 import sys
@@ -371,6 +372,50 @@ def test_no_state_leaks_between_problems(ctx):
     a2, _ = pa.loglik_batch(*_sweep_inputs())
     assert np.array_equal(a1, a2)
     st.close()
+
+
+DESTROY_ORDERS = list(itertools.permutations(("ctx", "problem", "state")))
+
+
+@pytest.mark.parametrize("order", DESTROY_ORDERS, ids=["-".join(o) for o in DESTROY_ORDERS])
+def test_objects_may_be_destroyed_in_any_order(order):
+    """A context, a problem and a caller's fit state may be destroyed in any order (garbage-collected hosts run finalizers
+    in unspecified order, include/gpcc_b200.h), each while it holds device resources: the context a tiled-path workspace
+    with a filled last-band cache, the problem the cached fitted state of postb.  Afterwards a fresh context reproduces the
+    first sweep bitwise.  gpcc_fit_state_destroy used to read the problem the state was made from: in the orders that
+    destroy the problem before the state, that read freed host memory, which is not guaranteed to fail, so on that code these cases
+    were not guaranteed to fail either."""
+    data = gpcc_b200.synthetic_bands([256, 256, 200], seed=21)[:3]          # N = 712: the tiled path
+    sweep = _sweep_inputs()
+    ctx = gpcc_b200.Context(1)
+    p = Problem(*data, "matern52", ctx)
+    ref, info = p.loglik_batch(*sweep)
+    assert np.all(info == 0) and ctx.stats()["path"] == 1 and ctx.stats()["n_tau_cache"] > 0
+    p.postb([0.0, 1.5, 3.0], [1.1, 1.8, 2.3], 2.9)
+    objs = {"ctx": ctx, "problem": p, "state": p.fit_state([0.0, 0.5, 4.0], [0.9, 1.7, 2.2], 3.1)}
+    for name in order:
+        objs[name].close()
+    ctx2 = gpcc_b200.Context(1)
+    again, _ = Problem(*data, "matern52", ctx2).loglik_batch(*sweep)
+    assert np.array_equal(again, ref)
+    ctx2.close()
+
+
+def test_rejected_device_id_leaves_no_cuda_error_behind():
+    """A context asked for a device id outside 0 .. count-1 fails before any CUDA call uses that id.  A call with the bad
+    id would leave cudaErrorInvalidDevice as the thread's last error, and the next launch check (the fused evaluator, the
+    fitted state's kernels) would report it as its own failure."""
+    import torch
+    t, y, s, d = gpcc_b200.synthetic_bands([20, 15], seed=3, span=10.0)
+    for bad in (-1, torch.cuda.device_count()):
+        with pytest.raises(gpcc_b200.GpccError):
+            gpcc_b200.Context(devices=[bad])
+        ctx = gpcc_b200.Context(1)
+        p = Problem(t, y, s, "OU", ctx)
+        ll, info = p.loglik_batch([d], [[1.0, 1.2]], [2.0])
+        assert info[0] == 0 and np.isfinite(ll[0]), bad
+        p.postb(d, [1.0, 1.2], 2.0)
+        p.close(); ctx.close()
 
 
 # ---- D. fitted state (predict.cu) ---------------------------------------------------------------------------------------------

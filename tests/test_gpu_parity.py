@@ -660,10 +660,6 @@ def test_fit_state_factorises_once_and_handles_many_test_points(ctx):
     with pytest.raises(gpcc_b200.GpccError):
         p.fit_state(d, [1.0, -1.0], rho)                     # all(scale .> 0) (delayedCovariance.jl:3)
     st.close()
-    ctx2 = gpcc_b200.Context(1)                              # destroy order: context first, then state and problem (finalizers)
-    p2 = Problem(t, y, s, "OU", ctx2)
-    st2 = p2.fit_state(d, alpha, rho)
-    ctx2.close(); st2.close(); p2.close()
 
 
 # ---- edge cases of the batched entry points ---------------------------------------------------------------------
