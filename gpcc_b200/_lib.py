@@ -13,7 +13,7 @@ EXPORTS = [
     "gpcc_grid_posterior", "gpcc_getprobabilities", "gpcc_postb", "gpcc_predict", "gpcc_predict_loglik",
     "gpcc_fit_options_default", "gpcc_fit_state_create", "gpcc_fit_state_destroy", "gpcc_fit_state_postb",
     "gpcc_fit_state_predict", "gpcc_fit_state_predict_loglik", "gpcc_fit_state_factorisations",
-    "gpcc_comm_unique_id", "gpcc_ctx_comm_init_rank", "gpcc_fit_state_sample",
+    "gpcc_comm_unique_id", "gpcc_ctx_comm_init_rank", "gpcc_fit_state_sample", "gpcc_problem_set_method",
 ]
 
 
@@ -58,6 +58,7 @@ def load():
     lib.gpcc_problem_create.argtypes = [vp, C.c_int, ip, dp, dp, dp, C.c_int, dp, dp, C.POINTER(vp)]
     lib.gpcc_problem_destroy.argtypes = [vp]
     lib.gpcc_problem_get_prior.argtypes = [vp, dp, dp]
+    lib.gpcc_problem_set_method.argtypes = [vp, C.c_int]
     lib.gpcc_loglik_batch.argtypes = [vp, C.c_int, dp, dp, dp, C.c_int, dp, dp, ip]
     lib.gpcc_loglik_theta_batch.argtypes = [vp, C.c_int, dp, dp, C.POINTER(FitOptions), C.c_int, dp, dp, ip]
     lib.gpcc_fit_batch.argtypes = [vp, C.c_int, dp, C.c_int, dp, C.POINTER(FitOptions), dp, dp, dp, dp, ip, ip, ip]

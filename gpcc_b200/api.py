@@ -169,10 +169,17 @@ def _options(iterations, rhomin, rhomax, per_candidate=False, gtol=None, ftol=No
     return o
 
 
-class Problem:
-    """Device-resident data of one `gpcc` call (gpccfixdelay_marginaliseb.jl:85-98)."""
+_METHODS = {"dense": 0, "statespace": 1}
 
-    def __init__(self, tarray, yarray, stdarray, kernel, ctx=None):
+
+class Problem:
+    """Device-resident data of one `gpcc` call (gpccfixdelay_marginaliseb.jl:85-98).
+
+    `method` selects how the likelihood is evaluated: "dense" (default) factorises K + Sobs + B; "statespace" (OU,
+    matern32, matern52) runs an exact Kalman filter in O(N) per evaluation (gpcc_problem_set_method), for light curves
+    far beyond what a dense factorisation can hold.  Fit states and predictions stay dense under either method."""
+
+    def __init__(self, tarray, yarray, stdarray, kernel, ctx=None, method="dense"):
         self.ctx = ctx or default_context()
         self.L = len(tarray)
         if not (self.L == len(yarray) == len(stdarray)):
@@ -193,6 +200,16 @@ class Problem:
                                               None, None, C.byref(self._h)))
         self.mub, self.Sigmab = np.empty(self.L), np.empty(self.L)
         check(_lib.load().gpcc_problem_get_prior(self._h, _d(self.mub), _d(self.Sigmab)))
+        self.method = "dense"
+        if method != "dense":
+            self.set_method(method)
+
+    def set_method(self, method):
+        """Switch between "dense" and "statespace" (see the class docstring)."""
+        if method not in _METHODS:
+            raise GpccError("method must be 'dense' or 'statespace'")
+        check(_lib.load().gpcc_problem_set_method(self._h, _METHODS[method]))
+        self.method = method
 
     def close(self):
         if getattr(self, "_h", None) and self._h.value:
@@ -409,10 +426,49 @@ def _informuser(out, seed, iterations, numberofrestarts, initialrandom, rhomin, 
     out.write("\t Σb                     = " + "".join("%.3f " % v for v in Sigmab) + "\n")
 
 
+def _pred_call(state, L, ttest, ytest=None, stest=None):                                                # :259-343
+    if ytest is not None:
+        ll, info = state.predict_loglik(ttest, ytest, stest)
+        if info != 0:
+            # PosDefException branch of the reference (:323-341): nearestposdef(Sigma; minimumeigenvalue=1e-6), i.e.
+            # eigenvalues clamped from below (src/UNUSED/gpcc.jl:294-300 spells it out), then logpdf.  The reference does
+            # this repair in host code (MiscUtil) on an exceptional path; mu and Sigma still come from the device.
+            mu_, _, S_, _ = state.predict(ttest, full_cov=True)
+            S_ = S_ + np.diag(np.concatenate([_f64(a) for a in stest]) ** 2)
+            return repaired_logpdf(mu_, S_, np.concatenate([_f64(a) for a in ytest]))
+        return ll
+    if len(ttest) > 0 and np.ndim(ttest[0]) > 0:                    # Vector{Vector}: (mu, Sigma) (:259-289)
+        mu_, _, S_, _ = state.predict(ttest, full_cov=True)
+        return mu_, S_
+    tt = np.asarray(ttest, dtype=np.float64)                       # Vector: per band (mu, sigma) (:293-307)
+    mu_, sd_, _, _ = state.predict([tt] * L)
+    nt = len(tt)
+    return [mu_[i * nt:(i + 1) * nt] for i in range(L)], [sd_[i * nt:(i + 1) * nt] for i in range(L)]
+
+
+class _LazyPred:
+    """`pred` of a state-space fit: the dense fit state (one N^3 factorisation) is only built on the first call or on the
+    first access of `state`, so that a fit at large N that never predicts never factorises."""
+
+    def __init__(self, problem, delays, alpha, rho, info):
+        self._args, self._p, self._state, self.info = (delays, alpha, rho), problem, None, info
+
+    @property
+    def state(self):
+        if self._state is None:
+            self._state = self._p.fit_state(*self._args)
+        return self._state
+
+    def __call__(self, ttest, ytest=None, stest=None):
+        return _pred_call(self.state, self._p.L, ttest, ytest, stest)
+
+
 def gpcc(tarray, yarray, stdarray, *, kernel, delays, iterations, seed=1, numberofrestarts=1, initialrandom=5,
-         rhomin=0.1, rhomax, theta0=None, ctx=None, verbose=True, problem=None, optimizer="lbfgs"):
-    """Drop-in for `gpcc` (gpccfixdelay_marginaliseb.jl:46-53): returns (loglikel, pred, (alpha, postb, rho))."""
-    p = problem or Problem(tarray, yarray, stdarray, kernel, ctx)
+         rhomin=0.1, rhomax, theta0=None, ctx=None, verbose=True, problem=None, optimizer="lbfgs", method="dense"):
+    """Drop-in for `gpcc` (gpccfixdelay_marginaliseb.jl:46-53): returns (loglikel, pred, (alpha, postb, rho)).
+    method="statespace" fits with the Kalman filter (see Problem), takes postb from it, and builds the dense fit state
+    behind `pred` only when `pred` is first used."""
+    p = problem or Problem(tarray, yarray, stdarray, kernel, ctx, method)
     delays = _f64(delays)
     if delays.shape != (p.L,):
         raise GpccError("L == length(delays) violated")                                   # :78
@@ -434,40 +490,28 @@ def gpcc(tarray, yarray, stdarray, *, kernel, delays, iterations, seed=1, number
     if verbose:
         out.write("\n\tOverall minimum is %f\n" % (-loglikel))                                          # :228
         out.write("(α, ρ) = unpack(paramopt) = (%s, %s)\n" % (alpha.tolist(), rho))                      # :235
+    info = dict(nfev=int(res["nfev"][best]), iters=int(res["iters"][best]), status=int(res["info"][best]),
+                theta=res["theta"][best].copy())
+    if p.method == "statespace":
+        mu, S = p.postb(delays, alpha, rho)                                                              # :248-252, by the filter
+        return loglikel, _LazyPred(p, delays, alpha, rho, info), (alpha, MvNormal(mu, S), rho)
     state = p.fit_state(delays, alpha, rho)                      # K = delayedCovariance(...); KSobsB (:237-241), factorised once
     mu, S = state.postb()                                                                                # :248-252
     postb = MvNormal(mu, S)
 
     def pred(ttest, ytest=None, stest=None):                                                             # :259-343
-        if ytest is not None:
-            ll, info = state.predict_loglik(ttest, ytest, stest)
-            if info != 0:
-                # PosDefException branch of the reference (:323-341): nearestposdef(Sigma; minimumeigenvalue=1e-6), i.e.
-                # eigenvalues clamped from below (src/UNUSED/gpcc.jl:294-300 spells it out), then logpdf.  The reference does
-                # this repair in host code (MiscUtil) on an exceptional path; mu and Sigma still come from the device.
-                mu_, _, S_, _ = state.predict(ttest, full_cov=True)
-                S_ = S_ + np.diag(np.concatenate([_f64(a) for a in stest]) ** 2)
-                return repaired_logpdf(mu_, S_, np.concatenate([_f64(a) for a in ytest]))
-            return ll
-        if len(ttest) > 0 and np.ndim(ttest[0]) > 0:                    # Vector{Vector}: (mu, Sigma) (:259-289)
-            mu_, _, S_, _ = state.predict(ttest, full_cov=True)
-            return mu_, S_
-        tt = np.asarray(ttest, dtype=np.float64)                       # Vector: per band (mu, sigma) (:293-307)
-        mu_, sd_, _, _ = state.predict([tt] * p.L)
-        nt = len(tt)
-        return [mu_[i * nt:(i + 1) * nt] for i in range(p.L)], [sd_[i * nt:(i + 1) * nt] for i in range(p.L)]
+        return _pred_call(state, p.L, ttest, ytest, stest)
 
     pred.state = state
-    pred.info = dict(nfev=int(res["nfev"][best]), iters=int(res["iters"][best]), status=int(res["info"][best]),
-                     theta=res["theta"][best].copy())
+    pred.info = info
     return loglikel, pred, (alpha, postb, rho)
 
 
 def gpccgrid(tarray, yarray, stdarray, candidatedelays, *, kernel, iterations, seed=1, initialrandom=5, rhomin=0.1,
-             rhomax, logprior=None, theta0=None, ctx=None, problem=None):
+             rhomax, logprior=None, theta0=None, ctx=None, problem=None, method="dense"):
     """Additive batched entry replacing the README's `map`/`pmap` idiom (README.md:170-210, 285):
     candidatedelays is [M][L]; returns a dict with loglikel[M], posterior[M] (getprobabilities), alpha, rho."""
-    p = problem or Problem(tarray, yarray, stdarray, kernel, ctx)
+    p = problem or Problem(tarray, yarray, stdarray, kernel, ctx, method)
     if theta0 is None:
         theta0 = initial_solutions(yarray, seed, 1, initialrandom, rhomin, rhomax)[0][0]
     return p.grid_posterior(candidatedelays, theta0, iterations=iterations, rhomin=rhomin, rhomax=rhomax,
@@ -521,7 +565,7 @@ def cv_folds(nper, numberoffolds=5, seedcv=1):
 
 
 def performcv(tobs, yobs, sobs, *, delays, kernel, iterations=1, seedcv=1, numberofrestarts=1, initialrandom=1,
-              numberoffolds=5, rhomin=0.1, rhomax=20.0, folds=None, theta0=None, ctx=None, out=None):
+              numberoffolds=5, rhomin=0.1, rhomax=20.0, folds=None, theta0=None, ctx=None, out=None, method="dense"):
     """K-fold cross-validation of the GPCC model at fixed delays, the retired consumer of `gpcc` + `pred(t, y, sigma)` in
     src/UNUSED/performcv.jl:41-139 (SURVEY.md 8f): per fold, fit on the training part and evaluate the test log-likelihood
     of the held-out part, both on the device.  Returns the vector of fold scores (to be fed to `getprobabilities`).
@@ -540,7 +584,7 @@ def performcv(tobs, yobs, sobs, *, delays, kernel, iterations=1, seedcv=1, numbe
         out.write("\n--- fold %d train size is %d, test size is %d ---\n" % (k + 1, sum(int(m.sum()) for m in tr), sum(int(m.sum()) for m in te)))
         pred = gpcc(part(tobs, tr), part(yobs, tr), part(sobs, tr), kernel=kernel, delays=delays, iterations=iterations,
                     seed=seedcv, numberofrestarts=numberofrestarts, initialrandom=initialrandom, rhomin=rhomin, rhomax=rhomax,
-                    theta0=None if theta0 is None else theta0[k], ctx=ctx, verbose=False)[1]                      # @suppress gpcc(...)[2] (:101)
+                    theta0=None if theta0 is None else theta0[k], ctx=ctx, verbose=False, method=method)[1]                      # @suppress gpcc(...)[2] (:101)
         fitness[k] = pred(part(tobs, te), part(yobs, te), part(sobs, te))                                         # :104
         out.write("\t perf for fold %d is %f\n" % (k + 1, fitness[k]))
     return fitness

@@ -68,9 +68,11 @@ int gpcc::evaluate_on_device(gpcc_problem* p, int di, int M, int want_grad) {
     b.ll = q.ll.d; b.grad = q.grad.d; b.info = q.info.d;
     b.h_delays = q.delays.h; b.h_alpha = q.alpha.h; b.h_rho = q.rho.h;
     const bool prof = p->ctx->profiling;
-    if (p->small_path) {
+    const bool one_kernel = p->method == GPCC_METHOD_STATESPACE || p->small_path;
+    if (one_kernel) {
         if (prof) CUDA_TRY(cudaEventRecord(s.ev0.get(), stream));
-        CUDA_TRY(small_sweep_launch(p->pd[di].dp, b, stream));
+        if (p->method == GPCC_METHOD_STATESPACE) CUDA_TRY(statespace_launch(p->kernel_id, p->pd[di].ssp, b, nullptr, stream));
+        else CUDA_TRY(small_sweep_launch(p->pd[di].dp, b, stream));
         if (prof) CUDA_TRY(cudaEventRecord(s.ev1.get(), stream));
         s.launches += 1;
     } else {
@@ -88,7 +90,7 @@ int gpcc::evaluate_on_device(gpcc_problem* p, int di, int M, int want_grad) {
         CUDA_TRY(cudaMemcpyAsync(q.grad.h, q.grad.d, (size_t)M * (L + 1) * sizeof(double), cudaMemcpyDeviceToHost, stream));
     CUDA_TRY(cudaMemcpyAsync(q.info.h, q.info.d, (size_t)M * sizeof(int), cudaMemcpyDeviceToHost, stream));
     CUDA_TRY(cudaStreamSynchronize(stream));
-    if (prof && p->small_path) {
+    if (prof && one_kernel) {
         float ms = 0;
         CUDA_TRY(cudaEventElapsedTime(&ms, s.ev0.get(), s.ev1.get()));
         s.ms_eval += ms;
@@ -139,7 +141,7 @@ void collect_stats(gpcc_ctx* ctx, const gpcc_problem* p, double ms_total) {
         st.n_tau_cache += s.tau_cache_evals;
         st.assembly_bytes = std::max(st.assembly_bytes, s.assembly_bytes);   // like ms_assembly: the busiest device
     }
-    st.path = (p && !p->small_path) ? 1 : 0;
+    st.path = !p ? 0 : p->method == GPCC_METHOD_STATESPACE ? 2 : p->small_path ? 0 : 1;
     st.n_devices = (int)ctx->ds.size();
     ctx->stats = st;
 }
@@ -282,9 +284,12 @@ int fit_shard(gpcc_problem* p, int di, const std::vector<int>& idx, const double
     const int m = (int)idx.size();
     if (m == 0) return 0;
     static const bool host_loop = getenv("GPCC_FIT_HOST") != nullptr;
-    if (p->small_path && (!host_loop || o.optimizer == GPCC_OPT_NELDERMEAD)) return fit_shard_device(p, di, idx, delays, P, theta0, o, out);
+    const bool dense = p->method == GPCC_METHOD_DENSE;
+    if (dense && p->small_path && (!host_loop || o.optimizer == GPCC_OPT_NELDERMEAD))
+        return fit_shard_device(p, di, idx, delays, P, theta0, o, out);
     if (o.optimizer == GPCC_OPT_NELDERMEAD)
-        return fail(-7, "the Nelder-Mead option runs on the fused small-N path only (N <= 199); use the default L-BFGS");
+        return fail(-7, dense ? "the Nelder-Mead option runs on the fused small-N path only (N <= 199); use the default L-BFGS"
+                              : "the Nelder-Mead option runs on the fused small-N dense path only; use the default L-BFGS");
     EvalSlot& q = p->ctx->ds[di].slot;
     LbfgsOptions lo;
     lo.max_iter = o.max_iter; lo.gtol = o.gtol; lo.ftol = o.ftol; lo.history = o.history; lo.n_scale = L;
@@ -299,7 +304,7 @@ int fit_shard(gpcc_problem* p, int di, const std::vector<int>& idx, const double
     if (rc) return rc;
     std::vector<int> seq(m);
     for (int c = 0; c < m; ++c) seq[c] = c;
-    if (!p->small_path && o.max_iter <= 0 && !o.theta0_per_candidate && L >= 2) {
+    if (dense && !p->small_path && o.max_iter <= 0 && !o.theta0_per_candidate && L >= 2) {
         // fixed-theta sweep on the tiled path (forward-only evaluations): candidates that share the delays of all bands but
         // the last become neighbours, so that a wave factorises their common leading block once (large_path.cu)
         std::stable_sort(seq.begin(), seq.end(), [&](int x, int y) {
@@ -418,7 +423,7 @@ int fit_all(gpcc_problem* p, int M, const double* delays, int P, const double* t
 // =====================================================================================================
 extern "C" {
 
-int gpcc_version(void) { return 101; }   // 101: gpcc_stats grew by n_tau_cache and assembly_bytes (appended)
+int gpcc_version(void) { return 102; }   // 102: gpcc_problem_set_method; 101: gpcc_stats grew by n_tau_cache and assembly_bytes
 const char* gpcc_last_error(void) { return gpcc::last_error().c_str(); }
 
 int gpcc_fit_options_default(gpcc_fit_options* o) {
@@ -579,6 +584,41 @@ int gpcc_problem_get_prior(const gpcc_problem* p, double* mub, double* Sigmab) {
     return 0;
 }
 
+int gpcc_problem_set_method(gpcc_problem* p, int method) {
+    if (!p) return fail(-1, "problem is NULL");
+    if (method != GPCC_METHOD_DENSE && method != GPCC_METHOD_STATESPACE) return fail(-2, "unknown method");
+    if (method == GPCC_METHOD_STATESPACE && p->kernel_id == GPCC_KERNEL_RBF)
+        return fail(-3, "the state-space method needs a Markovian kernel (OU, matern32 or matern52): rbf has no finite state-space form");
+    if (method == GPCC_METHOD_STATESPACE) {
+        // per band, a stable argsort of t: the merge of the filter (statespace.cu) keeps this order within a band
+        const int N = p->N, L = p->L;
+        std::vector<int> ord(N);
+        for (int i = 0; i < N; ++i) ord[i] = i;
+        for (int l = 0; l < L; ++l)
+            std::stable_sort(ord.begin() + p->band_start[l], ord.begin() + p->band_start[l + 1],
+                             [&](int a, int b) { return p->t[a] < p->t[b]; });
+        std::vector<double> t(N), r(N), s2(N);
+        for (int i = 0; i < N; ++i) { t[i] = p->t[ord[i]]; r[i] = p->resid[ord[i]]; s2[i] = p->s2[ord[i]]; }
+        for (auto& d : p->pd) {
+            CUDA_TRY(cudaSetDevice(d.dev));
+            CUDA_TRY(d.ss_t.reserve(N));
+            CUDA_TRY(d.ss_r.reserve(N));
+            CUDA_TRY(d.ss_s2.reserve(N));
+            CUDA_TRY(d.ss_postb.reserve((size_t)L + (size_t)L * L));
+            CUDA_TRY(cudaMemcpy(d.ss_t.d, t.data(), N * sizeof(double), cudaMemcpyHostToDevice));
+            CUDA_TRY(cudaMemcpy(d.ss_r.d, r.data(), N * sizeof(double), cudaMemcpyHostToDevice));
+            CUDA_TRY(cudaMemcpy(d.ss_s2.d, s2.data(), N * sizeof(double), cudaMemcpyHostToDevice));
+            SSProblem& q = d.ssp;
+            q.N = N; q.L = L;
+            for (int l = 0; l <= L; ++l) q.band_start[l] = p->band_start[l];
+            for (int l = 0; l < L; ++l) { q.mub[l] = p->mub[l]; q.Sigmab[l] = p->Sigmab[l]; }
+            q.t = d.ss_t.d; q.r = d.ss_r.d; q.s2 = d.ss_s2.d;
+        }
+    }
+    p->method = method;
+    return 0;
+}
+
 static int loglik_batch_impl(gpcc_problem* p, int M, const double* delays, const double* alpha, const double* rho,
                              const double* theta, const gpcc_fit_options* o, int want_grad, double* out_ll,
                              double* out_grad, int* out_info) {
@@ -601,7 +641,7 @@ static int loglik_batch_impl(gpcc_problem* p, int M, const double* delays, const
         EvalSlot& s = ctx->ds[di].slot;
         std::vector<int> mine;
         for (int m = di; m < M; m += nd) mine.push_back(m);
-        if (!p->small_path && !want_grad && !theta && L >= 2) {
+        if (p->method == GPCC_METHOD_DENSE && !p->small_path && !want_grad && !theta && L >= 2) {
             // logL-only sweep on the tiled path: bring evaluations with the same hyper-parameters and the same delays of all
             // bands but the last next to each other (structure reuse in large_path.cu); results are scattered back by index
             std::stable_sort(mine.begin(), mine.end(), [&](int x, int y) {
@@ -857,6 +897,41 @@ int posterior_on_devices(gpcc_ctx* ctx, int L, int M, const GatherIO& io, const 
             }
         }
     for (auto& s : ctx->ds) s.launches += 2;
+    return 0;
+}
+
+}  // namespace gpcc
+
+namespace gpcc {
+
+int statespace_postb(gpcc_problem* p, const double* delays, const double* alpha, double rho, double* out_mu, double* out_Sigma) {
+    const int L = p->L;
+    DeviceState& s = p->ctx->ds[0];
+    gpcc_problem::PerDev& d = p->pd[0];
+    CUDA_TRY(cudaSetDevice(s.dev));
+    int rc = reserve_eval(p, 0, 1);
+    if (rc) return rc;
+    EvalSlot& q = s.slot;
+    cudaStream_t st = s.stream.get();
+    CUDA_TRY(cudaStreamSynchronize(st));          // the pinned staging may still be read by an earlier call
+    std::memcpy(q.delays.h, delays, L * sizeof(double));
+    std::memcpy(q.alpha.h, alpha, L * sizeof(double));
+    q.rho.h[0] = rho;
+    CUDA_TRY(cudaMemcpyAsync(q.delays.d, q.delays.h, L * sizeof(double), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(q.alpha.d, q.alpha.h, L * sizeof(double), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(q.rho.d, q.rho.h, sizeof(double), cudaMemcpyHostToDevice, st));
+    EvalBatch b;
+    b.M = 1; b.delays = q.delays.d; b.alpha = q.alpha.d; b.rho = q.rho.d; b.want_grad = 0;
+    b.ll = q.ll.d; b.grad = q.grad.d; b.info = q.info.d;
+    CUDA_TRY(statespace_launch(p->kernel_id, d.ssp, b, d.ss_postb.d, st));
+    const size_t n = (size_t)L + (size_t)L * L;
+    CUDA_TRY(cudaMemcpyAsync(d.ss_postb.h, d.ss_postb.d, n * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(q.info.h, q.info.d, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    s.launches += 1;
+    if (q.info.h[0] != 0) return fail(-6, "the filter met a non-positive innovation variance for these hyper-parameters");
+    std::memcpy(out_mu, d.ss_postb.h, L * sizeof(double));
+    std::memcpy(out_Sigma, d.ss_postb.h + L, (size_t)L * L * sizeof(double));    // symmetric: the layout does not matter
     return 0;
 }
 

@@ -130,6 +130,18 @@ struct LargeTimings {
 cudaError_t large_eval(const DevProblem& p, const EvalBatch& b, LargeWorkspace& ws, cudaStream_t stream, bool profile,
                        LargeTimings* timings);
 
+// ---- state-space method for OU / matern32 / matern52 (statespace.cu): Kalman filter over the merged shifted times ----
+struct SSProblem {
+    int N = 0, L = 0;
+    int band_start[MAX_BANDS + 1] = {0};
+    double mub[MAX_BANDS] = {0}, Sigmab[MAX_BANDS] = {0};
+    const double* t = nullptr;    // [N] each band sorted by t (stable argsort), bands concatenated
+    const double* r = nullptr;    // [N] resid = y - mu_b in the same order
+    const double* s2 = nullptr;   // [N] sigma^2 in the same order
+};
+// postb (may be NULL): with M = 1, receives the filter's final b-block, [L] mean + mu_b, then [L][L] covariance
+cudaError_t statespace_launch(int kernel_id, const SSProblem& p, const EvalBatch& b, double* postb, cudaStream_t stream);
+
 // ---- posterior over candidates (posterior.cu): src/getprobabilities.jl:10-20 --------------------
 cudaError_t posterior_launch(int M, const double* d_ll, const double* d_logprior, double* d_out, cudaStream_t stream,
                              bool joint_already = false);

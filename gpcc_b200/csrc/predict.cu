@@ -630,6 +630,12 @@ int gpcc_fit_state_sample(gpcc_fit_state* s, unsigned long long seed, int nsampl
 }
 
 int gpcc_postb(gpcc_problem* p, const double* delays, const double* alpha, double rho, double* out_mu, double* out_Sigma) {
+    if (p && p->method == GPCC_METHOD_STATESPACE) {      // one filter, no factorisation
+        int rc = check_hyper(p, delays, alpha, rho);
+        if (rc) return rc;
+        if (!out_mu || !out_Sigma) return fail(-1, "NULL argument");
+        return statespace_postb(p, delays, alpha, rho, out_mu, out_Sigma);
+    }
     gpcc_fit_state* s = nullptr;
     int rc = cached_state(p, delays, alpha, rho, &s);
     if (rc) return rc;

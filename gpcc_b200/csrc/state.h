@@ -85,10 +85,14 @@ struct gpcc_problem {
         gpcc::DevArray<double> t, resid, y, s2, sigb;
         gpcc::DevArray<int> band;
         gpcc::DevProblem dp;
+        gpcc::DevArray<double> ss_t, ss_r, ss_s2;   // state-space method: each band sorted by t (gpcc_problem_set_method)
+        gpcc::DevBuf<double> ss_postb;              // [L + L*L] postb of the filter
+        gpcc::SSProblem ssp;
         ~PerDev() { cudaSetDevice(dev); }
     };
     std::vector<PerDev> pd;
     bool small_path = true;
+    int method = GPCC_METHOD_DENSE;
     // fitted state of the last gpcc_postb / gpcc_predict* call (predict.cu); never handed to a caller
     std::unique_ptr<gpcc_fit_state, gpcc::FitStateDelete> cached_state;
 };
@@ -98,4 +102,6 @@ namespace gpcc {
 // results land in ds[di].slot.ll.h / grad.h / info.h.
 int evaluate_on_device(gpcc_problem* p, int di, int M, int want_grad);
 int reserve_eval(gpcc_problem* p, int di, size_t M);
+// postb of a GPCC_METHOD_STATESPACE problem: one filter on the first device
+int statespace_postb(gpcc_problem* p, const double* delays, const double* alpha, double rho, double* out_mu, double* out_Sigma);
 }  // namespace gpcc

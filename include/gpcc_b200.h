@@ -35,6 +35,9 @@ enum { GPCC_KERNEL_OU = 0, GPCC_KERNEL_RBF = 1, GPCC_KERNEL_MATERN32 = 2, GPCC_K
  * transformbetween, un-vendored): id 0 = softplus + 1e-8 floor, rhomin+(rhomax-rhomin)*logistic.   */
 enum { GPCC_TRANSFORM_SOFTPLUS_LOGISTIC = 0 };
 enum { GPCC_OPT_LBFGS = 0, GPCC_OPT_NELDERMEAD = 1 };
+/* How a problem evaluates its likelihood: the dense factorisation of K + Sobs + B (default), or an exact Kalman filter
+ * over the merged, delay-shifted times (OU, matern32, matern52 only; see gpcc_problem_set_method).                  */
+enum { GPCC_METHOD_DENSE = 0, GPCC_METHOD_STATESPACE = 1 };
 
 typedef struct gpcc_ctx gpcc_ctx;
 typedef struct gpcc_problem gpcc_problem;
@@ -69,7 +72,8 @@ typedef struct gpcc_stats {
     long long n_eval_launches;  /* kernels launched by this library in the call                     */
     long long n_evals;          /* (candidate, theta) evaluations                                   */
     long long n_evals_grad;     /* ... of which with gradient                                       */
-    int    path;                /* 0 = fused register-resident small-N kernel, 1 = tiled large-N    */
+    int    path;                /* 0 = fused register-resident small-N kernel, 1 = tiled large-N,
+                                   2 = state-space method (Kalman filter, gpcc_problem_set_method)   */
     int    n_devices;
     long long n_shared_prefix;  /* tiled path, logL only: evaluations whose leading block (all bands but the
                                    last) was factorised by another evaluation of their wave (structure reuse) */
@@ -79,7 +83,8 @@ typedef struct gpcc_stats {
                                    tiles imported from the last-band cache count read + written); pairs with ms_assembly      */
 } gpcc_stats;
 
-int         gpcc_version(void);   /* 101.  100 -> 101: gpcc_stats grew by n_tau_cache and assembly_bytes (appended at the end);
+int         gpcc_version(void);   /* 102.  101 -> 102: gpcc_problem_set_method (additive).
+                                      100 -> 101: gpcc_stats grew by n_tau_cache and assembly_bytes (appended at the end);
                                       a caller built against 100 must be rebuilt before it calls gpcc_ctx_get_stats                */
 const char* gpcc_last_error(void);
 
@@ -107,6 +112,22 @@ int gpcc_problem_create(gpcc_ctx* ctx, int L, const int* n_per_band, const doubl
                         gpcc_problem** out);
 int gpcc_problem_destroy(gpcc_problem* p);
 int gpcc_problem_get_prior(const gpcc_problem* p, double* mub, double* Sigmab);
+
+/* Select how the problem evaluates its likelihood; a problem starts in GPCC_METHOD_DENSE and may switch back and forth.
+ * GPCC_METHOD_STATESPACE (OU, matern32, matern52; rbf has no finite state-space form and is rejected) computes the same
+ * logL, gradient and postb exactly, by a Kalman filter over the N merged, delay-shifted times: O(N (d+L)^2) per
+ * evaluation (d = 1, 2, 3) instead of the N^3/3 of the dense factorisation, and O(N) memory.  Switching it on sorts
+ * every band by time once and uploads that copy to every device.  Under it:
+ *   - gpcc_loglik_batch / gpcc_loglik_theta_batch run the filter; info > 0 is the 1-based position, in the merged
+ *     order of the shifted times (ties to the lower band), of the first observation whose innovation variance is not
+ *     positive and finite (loglik = -Inf).  It is a position in that order, not a leading-minor index;
+ *   - gpcc_fit_batch / gpcc_grid_posterior always use the host-driven batched L-BFGS (screening, then one batched
+ *     evaluation per round), whatever N is; GPCC_OPT_NELDERMEAD is rejected with -7;
+ *   - gpcc_postb runs one filter and returns its final b-block;
+ *   - gpcc_fit_state_*, gpcc_predict, gpcc_predict_loglik and gpcc_fit_state_sample stay dense: a fit state is a
+ *     Cholesky factor of K + Sobs.
+ * Returns < 0 for a NULL problem, an unknown method, or rbf with GPCC_METHOD_STATESPACE.                              */
+int gpcc_problem_set_method(gpcc_problem* p, int method);
 
 /* objective(alpha, rho) of src/gpccfixdelay_marginaliseb.jl:133-141 for M (delay, hyper-parameter)
  * pairs in constrained space: K~ = delayedCovariance (src/delayedCovariance.jl:1-38) + Sobs + B,

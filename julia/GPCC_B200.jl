@@ -67,6 +67,12 @@ mutable struct Problem
     end
 end
 
+# :dense factorises K + Sobs + B; :statespace (OU, matern32, matern52) runs the exact O(N) Kalman filter
+# (gpcc_problem_set_method in include/gpcc_b200.h).  Fit states behind `pred` are dense under either method.
+const METHODS = Dict(:dense => Cint(0), :statespace => Cint(1))
+setmethod!(p::Problem, method::Symbol) =
+    check(ccall((:gpcc_problem_set_method, LIB), Cint, (Ptr{Cvoid}, Cint), p.h, METHODS[method]))
+
 function __init__()
     # the library hard-codes softplus / scaled logistic for MiscUtil.makepositive / transformbetween (transform_id 0)
     for x in (-3.0, 0.0, 2.5)
@@ -111,13 +117,15 @@ function fitbatch(p::Problem, delays::Matrix{Float64}, θ0, opt::FitOptions)    
 end
 
 """
-    loglikel, pred, (α, postb, ρ) = gpcc(tarray, yarray, stdarray; kernel, delays, iterations, seed = 1, numberofrestarts = 1, initialrandom = 5, rhomin = 0.1, rhomax)
+    loglikel, pred, (α, postb, ρ) = gpcc(tarray, yarray, stdarray; kernel, delays, iterations, seed = 1, numberofrestarts = 1, initialrandom = 5, rhomin = 0.1, rhomax, method = :dense)
 
-Same contract as GPCC.gpcc (gpccfixdelay_marginaliseb.jl:46-53, 351).
+Same contract as GPCC.gpcc (gpccfixdelay_marginaliseb.jl:46-53, 351).  `method = :statespace` (OU, matern32, matern52) fits with
+the exact O(N) Kalman filter, takes postb from it, and factorises K + Sobs only when `pred` is first called.
 """
 function gpcc(tarray, yarray, stdarray; kernel = kernel, delays = delays, iterations = iterations, seed = 1,
-              numberofrestarts = 1, initialrandom = 5, rhomin = 0.1, rhomax = rhomax, neldermead = false)
+              numberofrestarts = 1, initialrandom = 5, rhomin = 0.1, rhomax = rhomax, neldermead = false, method = :dense)
     p = Problem(defaultctx(), tarray, yarray, stdarray, kernel); L = p.L
+    method == :dense || setmethod!(p, method)
     @assert L == length(delays)
     Σb = 100 .* map(var, yarray)
     @printf("Running with random seed %d\n", seed)                                   # util.jl:1-11
@@ -131,28 +139,33 @@ function gpcc(tarray, yarray, stdarray; kernel = kernel, delays = delays, iterat
     b = argmax(ll); α = αs[:, b]; ρ = ρs[b]
     @printf("\n\tOverall minimum is %f\n", -ll[b]); @show α, ρ                        # :228, :235
     d = Float64.(delays); μ = zeros(L); Σ = zeros(L, L)
-    st = FitState(p, d, α, ρ)                                                        # K, KSobsB (:237-241): factorised once
-    GC.@preserve μ Σ check(ccall((:gpcc_fit_state_postb, LIB), Cint, (Ptr{Cvoid}, Ptr{Cdouble}, Ptr{Cdouble}), st.h, μ, Σ))
+    stref = Ref{Union{Nothing, FitState}}(nothing)
+    state() = (stref[] === nothing && (stref[] = FitState(p, d, α, ρ)); stref[])   # K, KSobsB (:237-241): factorised once
+    if method == :statespace          # postb from the filter; the factorisation waits for the first prediction
+        GC.@preserve d α μ Σ check(ccall((:gpcc_postb, LIB), Cint, (Ptr{Cvoid}, Ptr{Cdouble}, Ptr{Cdouble}, Cdouble, Ptr{Cdouble}, Ptr{Cdouble}), p.h, d, α, ρ, μ, Σ))
+    else
+        GC.@preserve μ Σ check(ccall((:gpcc_fit_state_postb, LIB), Cint, (Ptr{Cvoid}, Ptr{Cdouble}, Ptr{Cdouble}), state().h, μ, Σ))
+    end
     postb = MvNormal(μ, Symmetric(Σ))                                                # :252
 
     function predictTest(ttest::Union{Array{Array{Float64, 1}, 1}, Array{T} where T <: AbstractRange{S} where S <: Real})   # :259-289
         nt = Cint.(length.(ttest)); tt = Float64.(reduce(vcat, collect.(ttest))); NT = length(tt)
         μp = zeros(NT); Σp = zeros(NT, NT)
         GC.@preserve nt tt μp Σp check(ccall((:gpcc_fit_state_predict, LIB), Cint,
-            (Ptr{Cvoid}, Ptr{Cint}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}), st.h, nt, tt, μp, C_NULL, Σp))
+            (Ptr{Cvoid}, Ptr{Cint}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}), state().h, nt, tt, μp, C_NULL, Σp))
         μp, Σp
     end
     function predictTest(ttest::Union{AbstractRange{Float64}, Array{Float64, 1}})                                          # :293-307
         Nt = length(ttest); nt = fill(Cint(Nt), L); tt = repeat(Float64.(collect(ttest)), L); μp = zeros(L * Nt); σp = zeros(L * Nt)
         GC.@preserve nt tt μp σp check(ccall((:gpcc_fit_state_predict, LIB), Cint,
-            (Ptr{Cvoid}, Ptr{Cint}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}), st.h, nt, tt, μp, σp, C_NULL))
+            (Ptr{Cvoid}, Ptr{Cint}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}), state().h, nt, tt, μp, σp, C_NULL))
         [μp[idx] for idx in Iterators.partition(1:L*Nt, Nt)], [σp[idx] for idx in Iterators.partition(1:L*Nt, Nt)]
     end
     function predictTest(ttest::Array{Array{Float64, 1}, 1}, ytest::Array{Array{Float64, 1}, 1}, σtest::Array{Array{Float64, 1}, 1})   # :311-343
         nt = Cint.(length.(ttest)); tt = reduce(vcat, ttest); yt = reduce(vcat, ytest); σt = reduce(vcat, σtest)
         ll_ = Ref{Cdouble}(0.0); info = Ref{Cint}(0)
         GC.@preserve nt tt yt σt check(ccall((:gpcc_fit_state_predict_loglik, LIB), Cint,
-            (Ptr{Cvoid}, Ptr{Cint}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ref{Cdouble}, Ref{Cint}), st.h, nt, tt, yt, σt, ll_, info))
+            (Ptr{Cvoid}, Ptr{Cint}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ref{Cdouble}, Ref{Cint}), state().h, nt, tt, yt, σt, ll_, info))
         if info[] != 0      # PosDefException branch (:327-333): repair on the host exactly as the reference does
             μp, Σp = predictTest(ttest); Σp = Σp + Diagonal(σt .^ 2)
             return logpdf(MvNormal(μp, MiscUtil.nearestposdef(MiscUtil.makematrixsymmetric(Σp); minimumeigenvalue = 1e-6)), yt)
@@ -169,8 +182,9 @@ Batched replacement of the README's `map`/`pmap` idiom (README.md:170-210, 285):
 L-vectors; the grid is sharded over the context's GPUs, log-likelihoods are all-gathered with NCCL and normalised.
 """
 function gpccgrid(tarray, yarray, stdarray, candidatedelays; kernel = kernel, iterations = iterations, seed = 1, initialrandom = 5,
-                  rhomin = 0.1, rhomax = rhomax, logprior = nothing)
+                  rhomin = 0.1, rhomax = rhomax, logprior = nothing, method = :dense)
     p = Problem(defaultctx(), tarray, yarray, stdarray, kernel); L = p.L; M = length(candidatedelays)
+    method == :dense || setmethod!(p, method)
     τ = Float64.(reduce(hcat, candidatedelays)); θ0, _ = startpoints(yarray, seed, 1, initialrandom, rhomin, rhomax)
     ll = zeros(M); post = zeros(M); α = zeros(L, M); ρ = zeros(M); lp = logprior === nothing ? C_NULL : Float64.(vec(logprior))
     GC.@preserve τ θ0 ll post α ρ lp check(ccall((:gpcc_grid_posterior, LIB), Cint,
