@@ -8,5 +8,5 @@ marshals arrays.  Julia callers bind the same C ABI through julia/GPCC_B200.jl (
 """
 from .api import (Context, Problem, gpcc, gpccgrid, getprobabilities, uniformpriordelay, Uniform, MvNormal,  # noqa: F401
                   OU, rbf, matern32, matern52, initial_solutions, default_context, GpccError, performcv, cv_folds,
-                  FitState, comm_unique_id, simulatedata_device)
+                  FitState, StateSpaceFitState, comm_unique_id, simulatedata_device)
 from .synthetic import simulatetwolightcurves, simulatethreelightcurves, simulatedata, synthetic_bands  # noqa: F401,E402

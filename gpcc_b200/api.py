@@ -177,7 +177,8 @@ class Problem:
 
     `method` selects how the likelihood is evaluated: "dense" (default) factorises K + Sobs + B; "statespace" (OU,
     matern32, matern52) runs an exact Kalman filter in O(N) per evaluation (gpcc_problem_set_method), for light curves
-    far beyond what a dense factorisation can hold.  Fit states and predictions stay dense under either method."""
+    far beyond what a dense factorisation can hold.  `fit_state` and the prediction methods stay dense under either
+    method; `statespace_fit_state` is the O(N) fit state of the state-space method."""
 
     def __init__(self, tarray, yarray, stdarray, kernel, ctx=None, method="dense"):
         self.ctx = ctx or default_context()
@@ -283,6 +284,11 @@ class Problem:
         """The state the reference's `pred` closures capture (:235-252): one factorisation, cached on the device."""
         return FitState(self, delays, alpha, rho)
 
+    def statespace_fit_state(self, delays, alpha, rho):
+        """O(N) fit state of the state-space method (gpcc_ss_state_*): per-point predictions and the test log-likelihood
+        without a dense factorisation.  Needs method="statespace"."""
+        return StateSpaceFitState(self, delays, alpha, rho)
+
     def postb(self, delays, alpha, rho):
         delays, alpha = _f64(delays, (self.L,)), _f64(alpha, (self.L,))
         mu, S = np.empty(self.L), np.empty((self.L, self.L))
@@ -368,6 +374,56 @@ class FitState:
     def close(self):
         if getattr(self, "_h", None) and self._h.value:
             _lib.load().gpcc_fit_state_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class StateSpaceFitState:
+    """Fit state of the state-space method on the device (gpcc_ss_state_*): the filtered moments and the backward-pass adjoint
+    of the N merged training points at (delays, alpha, rho), O(N) memory.  Answers the per-point form of `pred` (means and
+    standard deviations) and the test log-likelihood; the full predictive covariance needs the dense `fit_state`.  The
+    state owns its data: it stays usable after its problem is closed."""
+
+    def __init__(self, problem, delays, alpha, rho):
+        self.problem = problem              # keeps the context alive
+        self.L = problem.L
+        self.delays, self.alpha, self.rho = _f64(delays, (self.L,)).copy(), _f64(alpha, (self.L,)).copy(), float(rho)
+        self._h = C.c_void_p()
+        check(_lib.load().gpcc_ss_state_create(problem._h, _d(self.delays), _d(self.alpha), self.rho, C.byref(self._h)))
+
+    def predict(self, ttest_per_band, full_cov=False):
+        if full_cov:
+            raise GpccError("the state-space fit state gives per-point means and standard deviations only: the full "
+                            "predictive covariance needs the dense fit_state")
+        nt, tt = self.problem._pack_test(ttest_per_band)
+        NT = int(nt.sum())
+        mu, sd = np.empty(NT), np.empty(NT)
+        check(_lib.load().gpcc_ss_state_predict(self._h, _i(nt), _d(tt), _d(mu), _d(sd)))
+        return mu, sd, None, nt
+
+    def predict_loglik(self, ttest, ytest, stest):
+        nt, tt = self.problem._pack_test(ttest)
+        yt = _f64(np.concatenate([np.asarray(a, dtype=np.float64) for a in ytest]))
+        st = _f64(np.concatenate([np.asarray(a, dtype=np.float64) for a in stest]))
+        if not (len(tt) == len(yt) == len(st)):
+            raise GpccError("test arrays differ in length")
+        ll, info = C.c_double(), C.c_int()
+        check(_lib.load().gpcc_ss_state_predict_loglik(self._h, _i(nt), _d(tt), _d(yt), _d(st), C.byref(ll), C.byref(info)))
+        return ll.value, info.value
+
+    def pred(self, ttest, ytest=None, stest=None):
+        """The reference's `pred` forms (:259-343) except the full covariance (Vector{Vector} form, and the nearestposdef
+        repair of a failed test likelihood), which raise GpccError."""
+        return _pred_call(self, self.L, ttest, ytest, stest)
+
+    def close(self):
+        if getattr(self, "_h", None) and self._h.value:
+            _lib.load().gpcc_ss_state_destroy(self._h)
             self._h = C.c_void_p()
 
     def __del__(self):

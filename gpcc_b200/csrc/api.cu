@@ -423,7 +423,7 @@ int fit_all(gpcc_problem* p, int M, const double* delays, int P, const double* t
 // =====================================================================================================
 extern "C" {
 
-int gpcc_version(void) { return 102; }   // 102: gpcc_problem_set_method; 101: gpcc_stats grew by n_tau_cache and assembly_bytes
+int gpcc_version(void) { return 103; }   // 103: gpcc_ss_state_*; 102: gpcc_problem_set_method; 101: gpcc_stats grew by n_tau_cache and assembly_bytes
 const char* gpcc_last_error(void) { return gpcc::last_error().c_str(); }
 
 int gpcc_fit_options_default(gpcc_fit_options* o) {
@@ -584,21 +584,31 @@ int gpcc_problem_get_prior(const gpcc_problem* p, double* mub, double* Sigmab) {
     return 0;
 }
 
+}  // extern "C"
+
+// Per band, a stable argsort of t: the merge of the filter (statespace.cu) keeps this order within a band.
+static void sort_bands(const gpcc_problem* p, std::vector<double>& t, std::vector<double>& r, std::vector<double>& s2) {
+    const int N = p->N;
+    std::vector<int> ord(N);
+    for (int i = 0; i < N; ++i) ord[i] = i;
+    for (int l = 0; l < p->L; ++l)
+        std::stable_sort(ord.begin() + p->band_start[l], ord.begin() + p->band_start[l + 1],
+                         [&](int a, int b) { return p->t[a] < p->t[b]; });
+    t.resize(N); r.resize(N); s2.resize(N);
+    for (int i = 0; i < N; ++i) { t[i] = p->t[ord[i]]; r[i] = p->resid[ord[i]]; s2[i] = p->s2[ord[i]]; }
+}
+
+extern "C" {
+
 int gpcc_problem_set_method(gpcc_problem* p, int method) {
     if (!p) return fail(-1, "problem is NULL");
     if (method != GPCC_METHOD_DENSE && method != GPCC_METHOD_STATESPACE) return fail(-2, "unknown method");
     if (method == GPCC_METHOD_STATESPACE && p->kernel_id == GPCC_KERNEL_RBF)
         return fail(-3, "the state-space method needs a Markovian kernel (OU, matern32 or matern52): rbf has no finite state-space form");
     if (method == GPCC_METHOD_STATESPACE) {
-        // per band, a stable argsort of t: the merge of the filter (statespace.cu) keeps this order within a band
         const int N = p->N, L = p->L;
-        std::vector<int> ord(N);
-        for (int i = 0; i < N; ++i) ord[i] = i;
-        for (int l = 0; l < L; ++l)
-            std::stable_sort(ord.begin() + p->band_start[l], ord.begin() + p->band_start[l + 1],
-                             [&](int a, int b) { return p->t[a] < p->t[b]; });
-        std::vector<double> t(N), r(N), s2(N);
-        for (int i = 0; i < N; ++i) { t[i] = p->t[ord[i]]; r[i] = p->resid[ord[i]]; s2[i] = p->s2[ord[i]]; }
+        std::vector<double> t, r, s2;
+        sort_bands(p, t, r, s2);
         for (auto& d : p->pd) {
             CUDA_TRY(cudaSetDevice(d.dev));
             CUDA_TRY(d.ss_t.reserve(N));
@@ -936,3 +946,193 @@ int statespace_postb(gpcc_problem* p, const double* delays, const double* alpha,
 }
 
 }  // namespace gpcc
+
+// ---- fit state of the state-space method (gpcc_ss_state_*): O(N) memory, predictions in O(D^3) per test point ----
+struct gpcc_ss_state {
+    int dev = 0, kernel_id = 0, N = 0, L = 0, D = 0;
+    SSProblem prior;                    // N, L, band_start, mu_b, Sigma_b of the training problem (no data pointers)
+    std::vector<double> tr_t, tr_r, tr_s2;   // training data, each band sorted by t: merged with the test points of a call
+    double ll_train = 0.0;
+    Stream stream;
+    DevArray<double> hyp;               // delays [L], alpha [L], rho
+    DevArray<double> st_t, st_m, st_P, st_lam, st_Lam;
+    DevArray<int> st_band;
+    SSStore st;
+    // scratch of the calls, kept between calls
+    DevArray<double> tt, mu, sd, mt, mr, ms2, ll;
+    DevArray<int> bt, info;
+    ~gpcc_ss_state() { cudaSetDevice(dev); }
+};
+
+namespace {
+
+int ss_state_create(gpcc_problem* p, const double* delays, const double* alpha, double rho, gpcc_ss_state** out) {
+    const int N = p->N, L = p->L, d = p->kernel_id == GPCC_KERNEL_OU ? 1 : p->kernel_id == GPCC_KERNEL_MATERN32 ? 2 : 3;
+    const size_t D = (size_t)(d + L), NP = D * (D + 1) / 2;
+    const gpcc_problem::PerDev& pd = p->pd[0];
+    CUDA_TRY(cudaSetDevice(pd.dev));
+    std::unique_ptr<gpcc_ss_state> s(new gpcc_ss_state());
+    s->dev = pd.dev; s->kernel_id = p->kernel_id; s->N = N; s->L = L; s->D = (int)D;
+    s->prior = pd.ssp;
+    s->prior.t = s->prior.r = s->prior.s2 = nullptr;
+    sort_bands(p, s->tr_t, s->tr_r, s->tr_s2);
+    CUDA_TRY(create_stream(s->stream, 0));
+    cudaStream_t st = s->stream.get();
+    std::vector<double> h(2 * L + 1);
+    std::memcpy(h.data(), delays, L * sizeof(double));
+    std::memcpy(h.data() + L, alpha, L * sizeof(double));
+    h[2 * L] = rho;
+    CUDA_TRY(s->hyp.reserve(h.size()));
+    CUDA_TRY(s->st_t.reserve(N));
+    CUDA_TRY(s->st_band.reserve(N));
+    CUDA_TRY(s->st_m.reserve((size_t)N * D));
+    CUDA_TRY(s->st_P.reserve((size_t)N * NP));
+    CUDA_TRY(s->st_lam.reserve((size_t)N * D));
+    CUDA_TRY(s->st_Lam.reserve((size_t)N * NP));
+    CUDA_TRY(s->ll.reserve(1));
+    CUDA_TRY(s->info.reserve(1));
+    s->st = SSStore{s->st_t.d, s->st_band.d, s->st_m.d, s->st_P.d, s->st_lam.d, s->st_Lam.d};
+    CUDA_TRY(cudaMemcpyAsync(s->hyp.d, h.data(), h.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+    // the problem's sorted device copies are read only here: the state keeps what its calls need
+    CUDA_TRY(statespace_store_launch(s->kernel_id, pd.ssp, s->hyp.d, s->ll.d, s->info.d, s->st, st));
+    int info = 0;
+    CUDA_TRY(cudaMemcpyAsync(&s->ll_train, s->ll.d, sizeof(double), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(&info, s->info.d, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    if (info != 0) return fail(-6, "the filter met a non-positive innovation variance for these hyper-parameters");
+    *out = s.release();
+    return 0;
+}
+
+// Test points of one call: counts, band of every point in input order, and the checks shared by both calls.
+int ss_test_points(const gpcc_ss_state* s, const int* ntest_per_band, const double* ttest, std::vector<int>& bt) {
+    if (!s || !ntest_per_band) return fail(-1, "NULL argument");
+    long long NT = 0;
+    for (int l = 0; l < s->L; ++l) {
+        if (ntest_per_band[l] < 0) return fail(-5, "negative test count");
+        NT += ntest_per_band[l];
+    }
+    if (NT > (1LL << 30)) return fail(-7, "too many test points for one call");
+    if (NT > 0 && !ttest) return fail(-1, "NULL argument");
+    bt.resize((size_t)NT);
+    for (int l = 0, k = 0; l < s->L; ++l)
+        for (int i = 0; i < ntest_per_band[l]; ++i, ++k) {
+            if (!std::isfinite(ttest[k])) return fail(-3, "non-finite test time");
+            bt[k] = l;
+        }
+    return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int gpcc_ss_state_create(gpcc_problem* p, const double* delays, const double* alpha, double rho, gpcc_ss_state** out) {
+    if (!out) return fail(-1, "out is NULL");
+    *out = nullptr;
+    if (!p || !delays || !alpha) return fail(-1, "NULL argument");
+    if (p->method != GPCC_METHOD_STATESPACE) return fail(-5, "the problem is not in GPCC_METHOD_STATESPACE (gpcc_problem_set_method)");
+    for (int l = 0; l < p->L; ++l) {
+        if (!(alpha[l] > 0) || !std::isfinite(alpha[l])) return fail(-2, "all(scale .> 0) violated (delayedCovariance.jl:3)");
+        if (!std::isfinite(delays[l])) return fail(-3, "non-finite delay");
+    }
+    if (!(rho > 0) || !std::isfinite(rho)) return fail(-4, "rho is <= 0 (delayedCovariance.jl:5-7)");
+    return ss_state_create(p, delays, alpha, rho, out);
+}
+
+int gpcc_ss_state_destroy(gpcc_ss_state* s) {
+    delete s;
+    return 0;
+}
+
+int gpcc_ss_state_predict(gpcc_ss_state* s, const int* ntest_per_band, const double* ttest, double* out_mu, double* out_sd) {
+    std::vector<int> bt;
+    int rc = ss_test_points(s, ntest_per_band, ttest, bt);
+    if (rc) return rc;
+    const size_t NT = bt.size();
+    if (NT == 0) return 0;
+    if (!out_mu) return fail(-1, "NULL argument");
+    CUDA_TRY(cudaSetDevice(s->dev));
+    cudaStream_t st = s->stream.get();
+    CUDA_TRY(s->tt.reserve(NT));
+    CUDA_TRY(s->bt.reserve(NT));
+    CUDA_TRY(s->mu.reserve(NT));
+    if (out_sd) CUDA_TRY(s->sd.reserve(NT));
+    CUDA_TRY(cudaMemcpyAsync(s->tt.d, ttest, NT * sizeof(double), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(s->bt.d, bt.data(), NT * sizeof(int), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(statespace_predict_launch(s->kernel_id, s->prior, s->hyp.d, s->st, (int)NT, s->tt.d, s->bt.d, s->mu.d,
+                                       out_sd ? s->sd.d : nullptr, st));
+    CUDA_TRY(cudaMemcpyAsync(out_mu, s->mu.d, NT * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (out_sd) CUDA_TRY(cudaMemcpyAsync(out_sd, s->sd.d, NT * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    return 0;
+}
+
+// log p(ytest | training data) = ll(train + test) - ll(train): one filter over the training points merged with the test points
+// (per band, both sorted by t, training first on ties), each test point with noise sigmatest^2 + 1e-8 (the jitter of the
+// predictive covariance).  info > 0: 1-based merged position of the first non-positive innovation variance, ll = -Inf.
+int gpcc_ss_state_predict_loglik(gpcc_ss_state* s, const int* ntest_per_band, const double* ttest, const double* ytest,
+                                 const double* sigmatest, double* out_ll, int* out_info) {
+    std::vector<int> bt;
+    int rc = ss_test_points(s, ntest_per_band, ttest, bt);
+    if (rc) return rc;
+    if (!out_ll) return fail(-1, "NULL argument");
+    const size_t NT = bt.size();
+    if (NT == 0) { *out_ll = 0.0; if (out_info) *out_info = 0; return 0; }
+    if (!ytest || !sigmatest) return fail(-1, "NULL argument");
+    for (size_t k = 0; k < NT; ++k) {
+        if (!std::isfinite(ytest[k]) || !std::isfinite(sigmatest[k])) return fail(-3, "non-finite test value");
+        if (sigmatest[k] < 0) return fail(-4, "sigmatest < 0");
+    }
+    const int L = s->L;
+    const size_t NM = (size_t)s->N + NT;
+    if (NM > (size_t)std::numeric_limits<int>::max()) return fail(-7, "too many test points for one call");
+    std::vector<double> mt(NM), mr(NM), ms2(NM);
+    SSProblem q = s->prior;
+    q.N = (int)NM;
+    std::vector<size_t> ord;
+    size_t k = 0, first = 0;
+    for (int l = 0; l < L; ++l) {
+        const size_t nt = (size_t)ntest_per_band[l];
+        ord.resize(nt);
+        for (size_t i = 0; i < nt; ++i) ord[i] = first + i;
+        std::stable_sort(ord.begin(), ord.end(), [&](size_t a, size_t b) { return ttest[a] < ttest[b]; });
+        q.band_start[l] = (int)k;
+        size_t a = s->prior.band_start[l], b = 0;
+        const size_t ae = s->prior.band_start[l + 1];
+        while (a < ae || b < nt) {
+            if (b == nt || (a < ae && s->tr_t[a] <= ttest[ord[b]])) {
+                mt[k] = s->tr_t[a]; mr[k] = s->tr_r[a]; ms2[k] = s->tr_s2[a]; ++a;
+            } else {
+                const size_t j = ord[b++];
+                mt[k] = ttest[j]; mr[k] = ytest[j] - s->prior.mub[l]; ms2[k] = sigmatest[j] * sigmatest[j] + 1e-8;
+            }
+            ++k;
+        }
+        first += nt;
+    }
+    q.band_start[L] = (int)k;
+    CUDA_TRY(cudaSetDevice(s->dev));
+    cudaStream_t st = s->stream.get();
+    CUDA_TRY(s->mt.reserve(NM));
+    CUDA_TRY(s->mr.reserve(NM));
+    CUDA_TRY(s->ms2.reserve(NM));
+    CUDA_TRY(cudaMemcpyAsync(s->mt.d, mt.data(), NM * sizeof(double), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(s->mr.d, mr.data(), NM * sizeof(double), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(s->ms2.d, ms2.data(), NM * sizeof(double), cudaMemcpyHostToDevice, st));
+    q.t = s->mt.d; q.r = s->mr.d; q.s2 = s->ms2.d;
+    EvalBatch b;
+    b.M = 1; b.delays = s->hyp.d; b.alpha = s->hyp.d + L; b.rho = s->hyp.d + 2 * L; b.want_grad = 0;
+    b.ll = s->ll.d; b.info = s->info.d;
+    CUDA_TRY(statespace_launch(s->kernel_id, q, b, nullptr, st));
+    double ll = 0.0;
+    int info = 0;
+    CUDA_TRY(cudaMemcpyAsync(&ll, s->ll.d, sizeof(double), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(&info, s->info.d, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    *out_ll = info ? -std::numeric_limits<double>::infinity() : ll - s->ll_train;
+    if (out_info) *out_info = info;
+    return 0;
+}
+
+}  // extern "C"

@@ -141,6 +141,25 @@ struct SSProblem {
 };
 // postb (may be NULL): with M = 1, receives the filter's final b-block, [L] mean + mu_b, then [L][L] covariance
 cudaError_t statespace_launch(int kernel_id, const SSProblem& p, const EvalBatch& b, double* postb, cudaStream_t stream);
+// Per merged training step k (N steps, D = d + L, NP = D (D+1) / 2), the moments behind the O(N) predictions of the state-space
+// fit state: shifted time, band, filtered mean and packed covariance after the update, and the Bryson-Frazier adjoint of the
+// step before its update (lam, Lam: smoothed mean m- - P- lam, smoothed covariance P- - P- Lam P-).
+struct SSStore {
+    double* t = nullptr;       // [N]
+    int* band = nullptr;       // [N]
+    double* m = nullptr;       // [N][D]
+    double* P = nullptr;       // [N][NP]
+    double* lam = nullptr;     // [N][D]
+    double* Lam = nullptr;     // [N][NP]
+};
+// One forward filter that fills st (ll[0], info[0] as statespace_launch with M = 1), then the sequential backward pass (skipped
+// when info[0] != 0).  hyp = [delays (L), alpha (L), rho] on the device.
+cudaError_t statespace_store_launch(int kernel_id, const SSProblem& p, const double* hyp, double* ll, int* info,
+                                    const SSStore& st, cudaStream_t stream);
+// Smoothed predictive mean (+ mu_b) and standard deviation sqrt(max(var + 1e-8, 1e-6)) of NT test points (tt, band bt, any
+// order) from st; p supplies N, L and the prior.  sd may be NULL.
+cudaError_t statespace_predict_launch(int kernel_id, const SSProblem& p, const double* hyp, const SSStore& st, int NT,
+                                      const double* tt, const int* bt, double* mu, double* sd, cudaStream_t stream);
 
 // ---- posterior over candidates (posterior.cu): src/getprobabilities.jl:10-20 --------------------
 cudaError_t posterior_launch(int M, const double* d_ll, const double* d_logprior, double* d_out, cudaStream_t stream,

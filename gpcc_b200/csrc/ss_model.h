@@ -19,8 +19,10 @@
 
 #if defined(__CUDACC__)
 #define GPCC_HD __host__ __device__
+#define GPCC_HDFI __host__ __device__ __forceinline__
 #else
 #define GPCC_HD
+#define GPCC_HDFI inline
 #endif
 
 namespace gpcc {
@@ -180,6 +182,101 @@ GPCC_HD inline void step(const Coef<Dim<KID>::d>& c, double D, double (&A)[Dim<K
                 if (want_d) dQ[i][j] = dQ[j][i] = c.dPinf[i][j] - ds;
             }
     }
+}
+
+template <int D>
+GPCC_HD constexpr int sym(int i, int j) {      // packed upper triangle, row-major
+    return i <= j ? i * D - i * (i - 1) / 2 + (j - i) : j * D - j * (j - 1) / 2 + (i - j);
+}
+
+// Moments of x = [f-state (d); b (D - d)] carried over a gap with the f-block transition A and process noise Q (the b-block
+// is static): m_f = A m_f, P_fb = A P_fb, P_ff = A P_ff A' + Q.  The primal lines of the gap predict of ss_filter_kernel
+// (statespace.cu), which keeps its own inline copy: called from there, a shared function changes the register allocation
+// and the spills of eight gradient instantiations of that kernel.
+template <int d, int D>
+GPCC_HDFI void predict_moments(const double (&A)[d][d], const double (&Q)[d][d], double (&m)[D], double (&P)[D * (D + 1) / 2]) {
+#pragma unroll
+    for (int k = d; k < D; ++k) {               // P_fb = A P_fb, one column at a time
+        double col[d];
+#pragma unroll
+        for (int i = 0; i < d; ++i) {
+            double s = 0.0;
+#pragma unroll
+            for (int q = 0; q < d; ++q) s = fma(A[i][q], P[sym<D>(q, k)], s);
+            col[i] = s;
+        }
+#pragma unroll
+        for (int i = 0; i < d; ++i) P[sym<D>(i, k)] = col[i];
+    }
+    double AP[d][d];                            // A P_ff
+#pragma unroll
+    for (int i = 0; i < d; ++i)
+#pragma unroll
+        for (int k = 0; k < d; ++k) {
+            double s = 0.0;
+#pragma unroll
+            for (int q = 0; q < d; ++q) s = fma(A[i][q], P[sym<D>(q, k)], s);
+            AP[i][k] = s;
+        }
+#pragma unroll
+    for (int i = 0; i < d; ++i)
+#pragma unroll
+        for (int k = i; k < d; ++k) {           // P_ff = A P_ff A' + Q
+            double s = Q[i][k];
+#pragma unroll
+            for (int q = 0; q < d; ++q) s = fma(AP[i][q], A[k][q], s);
+            P[sym<D>(i, k)] = s;
+        }
+    double mf[d];
+#pragma unroll
+    for (int i = 0; i < d; ++i) {
+        double s = 0.0;
+#pragma unroll
+        for (int q = 0; q < d; ++q) s = fma(A[i][q], m[q], s);
+        mf[i] = s;
+    }
+#pragma unroll
+    for (int i = 0; i < d; ++i) m[i] = mf[i];
+}
+
+// Smoothed mean and variance of h'x, h = a e_0 + e_(d+l), at a test time t between two training steps (statespace.cu, the
+// fit state).  On entry m, P are the filtered moments of the last training step i at or before t (the prior if t precedes
+// every training point); dt1 = t - s_i.  lam, Lam (packed) are the Bryson-Frazier adjoint of step i+1 before its update,
+// so that the smoothed moments there are m- - P- lam and P- - P- Lam P-; NULL when t follows the last training step.
+// dt2 = s_(i+1) - t > 0.  At t the adjoint is A2' lam and A2' Lam A2 (A2 over dt2, identity on the b-block), hence with
+// u = P h and w = A2 u:  mean = h'm - w'lam,  var = h'P h - w' Lam w.  No matrix is inverted.
+template <int KID, int L>
+GPCC_HD inline void point_moments(const Coef<Dim<KID>::d>& c, int l, double a, double (&m)[Dim<KID>::d + L],
+                                  double (&P)[(Dim<KID>::d + L) * (Dim<KID>::d + L + 1) / 2], double dt1,
+                                  const double* lam, const double* Lam, double dt2, double& mean, double& var) {
+    constexpr int d = Dim<KID>::d, D = d + L;
+    double A[d][d], Q[d][d], dA[d][d], dQ[d][d];
+    if (dt1 > 0.0) {
+        step<KID, false>(c, dt1, A, Q, dA, dQ);
+        predict_moments<d, D>(A, Q, m, P);
+    }
+    double u[D];
+    for (int i = 0; i < D; ++i) u[i] = fma(a, P[sym<D>(i, 0)], P[sym<D>(i, d + l)]);
+    mean = fma(a, m[0], m[d + l]);
+    var = fma(a, u[0], u[d + l]);
+    if (!lam) return;
+    step<KID, false>(c, dt2, A, Q, dA, dQ);
+    double w[D];
+    for (int i = 0; i < D; ++i) {
+        double s = i < d ? 0.0 : u[i];
+        if (i < d)
+            for (int q = 0; q < d; ++q) s = fma(A[i][q], u[q], s);
+        w[i] = s;
+    }
+    double wl = 0.0, wLw = 0.0;
+    for (int i = 0; i < D; ++i) {
+        wl = fma(w[i], lam[i], wl);
+        double s = 0.0;
+        for (int q = 0; q < D; ++q) s = fma(Lam[sym<D>(i, q)], w[q], s);
+        wLw = fma(w[i], s, wLw);
+    }
+    mean -= wl;
+    var -= wLw;
 }
 
 }  // namespace ss

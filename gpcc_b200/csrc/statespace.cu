@@ -26,10 +26,7 @@ namespace {
 
 constexpr double LOG2PI = 1.8378770664093454836;
 
-template <int D>
-__host__ __device__ constexpr int sym(int i, int j) {      // packed upper triangle, row-major
-    return i <= j ? i * D - i * (i - 1) / 2 + (j - i) : j * D - j * (j - 1) / 2 + (i - j);
-}
+using ss::sym;
 
 struct Head { double t, r, s2; };
 
@@ -40,10 +37,13 @@ __device__ __forceinline__ Head load_point(const SSProblem& p, int i, int end, d
     return h;
 }
 
-template <int KID, int L, bool GRAD>
+// STORE (with GRAD = false and M = 1; the fit state of gpcc_ss_state_create): also writes, per merged step, the shifted time,
+// the band and the filtered moments after the update to `st`.
+template <int KID, int L, bool GRAD, bool STORE = false>
 __global__ void __launch_bounds__(128) ss_filter_kernel(SSProblem p, int M, const double* __restrict__ delays,
                                                         const double* __restrict__ alpha, const double* __restrict__ rho,
-                                                        double* ll_out, double* grad_out, int* info_out, double* postb) {
+                                                        double* ll_out, double* grad_out, int* info_out, double* postb,
+                                                        SSStore st) {
     constexpr int d = ss::Dim<KID>::d, D = d + L, NP = D * (D + 1) / 2;
     constexpr int G = GRAD ? L + 1 : 1, GPW = 32 / G;
     const int lane = threadIdx.x & 31;
@@ -212,6 +212,15 @@ __global__ void __launch_bounds__(128) ss_filter_kernel(SSProblem p, int M, cons
         for (int i = 0; i < D; ++i)
 #pragma unroll
             for (int q = i; q < D; ++q) P[sym<D>(i, q)] = fma(-Ph[i], k[q], P[sym<D>(i, q)]);
+        if (STORE) {
+            const size_t o = (size_t)(step - 1);
+            st.t[o] = ts;
+            st.band[o] = l;
+#pragma unroll
+            for (int i = 0; i < D; ++i) st.m[o * D + i] = m[i];
+#pragma unroll
+            for (int i = 0; i < NP; ++i) st.P[o * NP + i] = P[i];
+        }
     }
 
     if (j == 0) {
@@ -234,7 +243,7 @@ cudaError_t launch_one(const SSProblem& p, const EvalBatch& b, double* postb, cu
     constexpr int G = GRAD ? L + 1 : 1, GPW = 32 / G, THREADS = 128;
     const int warps = (b.M + GPW - 1) / GPW;
     const int blocks = (warps + THREADS / 32 - 1) / (THREADS / 32);
-    ss_filter_kernel<KID, L, GRAD><<<blocks, THREADS, 0, stream>>>(p, b.M, b.delays, b.alpha, b.rho, b.ll, b.grad, b.info, postb);
+    ss_filter_kernel<KID, L, GRAD><<<blocks, THREADS, 0, stream>>>(p, b.M, b.delays, b.alpha, b.rho, b.ll, b.grad, b.info, postb, SSStore{});
     return cudaGetLastError();
 }
 
@@ -242,6 +251,215 @@ template <int KID, int L>
 cudaError_t launch_l(const SSProblem& p, const EvalBatch& b, double* postb, cudaStream_t stream) {
     if (p.L == L) return b.want_grad ? launch_one<KID, L, true>(p, b, postb, stream) : launch_one<KID, L, false>(p, b, postb, stream);
     if constexpr (L < MAX_BANDS) return launch_l<KID, L + 1>(p, b, postb, stream);
+    return cudaErrorInvalidValue;
+}
+
+// ---- fit state of the state-space method (gpcc_ss_state_*): stored forward pass, backward pass, per-point predictions ----
+constexpr double JITTER = 1e-8;       // added to every predictive variance, as the dense fit state does (predict.cu)
+constexpr double SIGMA_FLOOR = 1e-6;  // sd = sqrt(max(var + JITTER, SIGMA_FLOOR)), as the dense fit state does
+
+template <int KID, int L>
+__device__ __forceinline__ void prior_moments(const ss::Coef<ss::Dim<KID>::d>& c, const SSProblem& p,
+                                              double (&m)[ss::Dim<KID>::d + L],
+                                              double (&P)[(ss::Dim<KID>::d + L) * (ss::Dim<KID>::d + L + 1) / 2]) {
+    constexpr int d = ss::Dim<KID>::d, D = d + L;
+#pragma unroll
+    for (int i = 0; i < D; ++i) {
+        m[i] = 0.0;
+#pragma unroll
+        for (int k = i; k < D; ++k) P[sym<D>(i, k)] = k < d ? c.Pinf[i][k] : i == k ? p.Sigmab[i - d] : 0.0;
+    }
+}
+
+// Bryson-Frazier backward pass over the stored forward pass: one thread, the steps are one sequential chain.  The predicted
+// moments of step k are recomputed from the stored filtered moments of step k-1 with the filter's own predict, so gain and
+// innovation are those of the forward pass.  With lam^, Lam^ the adjoint after the update of step k (zero after the last),
+// k = P- h / S and w = Lam^ k, the adjoint before the update is
+//   lam~ = (I - k h')' lam^ - h v / S             = lam^ - h (k'lam^ + v / S)
+//   Lam~ = (I - k h')' Lam^ (I - k h') + h h' / S = Lam^ - h w' - w h' + (k'w + 1 / S) h h'
+// and the adjoint after the update of step k-1 is A' lam~, A' Lam~ A (A over s_k - s_(k-1), identity on the b-block).
+// Only scalar divisions (by S); no matrix is inverted.
+template <int KID, int L>
+__global__ void __launch_bounds__(32) ss_adjoint_kernel(SSProblem p, const double* __restrict__ hyp, const int* __restrict__ info,
+                                                        SSStore st) {
+    constexpr int d = ss::Dim<KID>::d, D = d + L, NP = D * (D + 1) / 2;
+    if (threadIdx.x != 0 || *info != 0) return;
+    double al[L];
+    int cnt[L];
+#pragma unroll
+    for (int l = 0; l < L; ++l) { al[l] = hyp[L + l]; cnt[l] = p.band_start[l + 1]; }
+    ss::Coef<d> c;
+    ss::setup<KID>(hyp[2 * L], c);
+    double lam[D], Lam[NP];
+#pragma unroll
+    for (int i = 0; i < D; ++i) lam[i] = 0.0;
+#pragma unroll
+    for (int i = 0; i < NP; ++i) Lam[i] = 0.0;
+    for (int k = p.N - 1; k >= 0; --k) {
+        const int l = st.band[k];
+        int idx = 0;
+        double a = 0.0;
+#pragma unroll
+        for (int lb = 0; lb < L; ++lb)
+            if (lb == l) { idx = --cnt[lb]; a = al[lb]; }       // the k-th step of band l is its next sorted point, backwards
+        const double r = p.r[idx], s2 = p.s2[idx];
+        double m[D], P[NP];
+        double A[d][d], Q[d][d], dA[d][d], dQ[d][d];
+        const double Dt = k > 0 ? st.t[k] - st.t[k - 1] : 0.0;
+        if (k > 0) {
+#pragma unroll
+            for (int i = 0; i < D; ++i) m[i] = st.m[(size_t)(k - 1) * D + i];
+#pragma unroll
+            for (int i = 0; i < NP; ++i) P[i] = st.P[(size_t)(k - 1) * NP + i];
+        } else {
+            prior_moments<KID, L>(c, p, m, P);
+        }
+        if (Dt > 0.0) {
+            ss::step<KID, false>(c, Dt, A, Q, dA, dQ);
+            ss::predict_moments<d, D>(A, Q, m, P);
+        }
+        double h[D], Ph[D];
+#pragma unroll
+        for (int i = 0; i < D; ++i) {
+            h[i] = i == 0 ? a : (i >= d && i - d == l) ? 1.0 : 0.0;
+            double s = 0.0;
+#pragma unroll
+            for (int lb = 0; lb < L; ++lb)
+                if (lb == l) s = P[sym<D>(i, d + lb)];
+            Ph[i] = fma(a, P[sym<D>(i, 0)], s);
+        }
+        double Phb = 0.0, mb = 0.0;
+#pragma unroll
+        for (int lb = 0; lb < L; ++lb)
+            if (lb == l) { Phb = Ph[d + lb]; mb = m[d + lb]; }
+        const double S = fma(a, Ph[0], Phb) + s2;            // the filter's innovation variance and residual
+        const double v = r - fma(a, m[0], mb);
+        const double iS = 1.0 / S;
+        double kg[D], w[D], kl = 0.0, kw = 0.0;
+#pragma unroll
+        for (int i = 0; i < D; ++i) kg[i] = Ph[i] * iS;
+#pragma unroll
+        for (int i = 0; i < D; ++i) {
+            double s = 0.0;
+#pragma unroll
+            for (int q = 0; q < D; ++q) s = fma(Lam[sym<D>(i, q)], kg[q], s);
+            w[i] = s;
+            kl = fma(kg[i], lam[i], kl);
+        }
+#pragma unroll
+        for (int i = 0; i < D; ++i) kw = fma(kg[i], w[i], kw);
+        const double cl = fma(v, iS, kl), cL = kw + iS;
+#pragma unroll
+        for (int i = 0; i < D; ++i) lam[i] = fma(-h[i], cl, lam[i]);
+#pragma unroll
+        for (int i = 0; i < D; ++i)
+#pragma unroll
+            for (int q = i; q < D; ++q)
+                Lam[sym<D>(i, q)] = fma(cL * h[i], h[q], Lam[sym<D>(i, q)] - fma(h[i], w[q], w[i] * h[q]));
+#pragma unroll
+        for (int i = 0; i < D; ++i) st.lam[(size_t)k * D + i] = lam[i];
+#pragma unroll
+        for (int i = 0; i < NP; ++i) st.Lam[(size_t)k * NP + i] = Lam[i];
+        if (k > 0 && Dt > 0.0) {
+            double lf[d], B[d][d];
+#pragma unroll
+            for (int i = 0; i < d; ++i) {
+                double s = 0.0;
+#pragma unroll
+                for (int q = 0; q < d; ++q) s = fma(A[q][i], lam[q], s);
+                lf[i] = s;
+            }
+#pragma unroll
+            for (int i = 0; i < d; ++i) lam[i] = lf[i];
+#pragma unroll
+            for (int kc = d; kc < D; ++kc) {            // Lam_fb = A' Lam_fb
+#pragma unroll
+                for (int i = 0; i < d; ++i) {
+                    double s = 0.0;
+#pragma unroll
+                    for (int q = 0; q < d; ++q) s = fma(A[q][i], Lam[sym<D>(q, kc)], s);
+                    lf[i] = s;
+                }
+#pragma unroll
+                for (int i = 0; i < d; ++i) Lam[sym<D>(i, kc)] = lf[i];
+            }
+#pragma unroll
+            for (int i = 0; i < d; ++i)                 // B = Lam_ff A, then Lam_ff = A' B
+#pragma unroll
+                for (int j = 0; j < d; ++j) {
+                    double s = 0.0;
+#pragma unroll
+                    for (int q = 0; q < d; ++q) s = fma(Lam[sym<D>(i, q)], A[q][j], s);
+                    B[i][j] = s;
+                }
+#pragma unroll
+            for (int i = 0; i < d; ++i)
+#pragma unroll
+                for (int j = i; j < d; ++j) {
+                    double s = 0.0;
+#pragma unroll
+                    for (int q = 0; q < d; ++q) s = fma(A[q][i], B[q][j], s);
+                    Lam[sym<D>(i, j)] = s;
+                }
+        }
+    }
+}
+
+// One thread per test point, in input order: the last stored step at or before its shifted time (binary search; a test
+// time equal to a training time sits after it), then ss::point_moments.
+template <int KID, int L>
+__global__ void __launch_bounds__(128) ss_point_kernel(SSProblem p, const double* __restrict__ hyp, SSStore st, int NT,
+                                                       const double* __restrict__ tt, const int* __restrict__ bt,
+                                                       double* __restrict__ mu, double* __restrict__ sd) {
+    constexpr int d = ss::Dim<KID>::d, D = d + L, NP = D * (D + 1) / 2;
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= NT) return;
+    const int l = bt[j];
+    const double ts = tt[j] - hyp[l], a = hyp[L + l];
+    ss::Coef<d> c;
+    ss::setup<KID>(hyp[2 * L], c);
+    int lo = 0, hi = p.N;                          // first step with s > ts
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (st.t[mid] <= ts) lo = mid + 1; else hi = mid;
+    }
+    const int i = lo - 1;
+    double m[D], P[NP];
+    if (i >= 0) {
+#pragma unroll
+        for (int q = 0; q < D; ++q) m[q] = st.m[(size_t)i * D + q];
+#pragma unroll
+        for (int q = 0; q < NP; ++q) P[q] = st.P[(size_t)i * NP + q];
+    } else {
+        prior_moments<KID, L>(c, p, m, P);          // stationary: no propagation to ts
+    }
+    const bool later = i + 1 < p.N;
+    double mean, var;
+    ss::point_moments<KID, L>(c, l, a, m, P, i >= 0 ? ts - st.t[i] : 0.0, later ? st.lam + (size_t)(i + 1) * D : nullptr,
+                              later ? st.Lam + (size_t)(i + 1) * NP : nullptr, later ? st.t[i + 1] - ts : 0.0, mean, var);
+    mu[j] = mean + p.mub[l];
+    if (sd) sd[j] = sqrt(fmax(var + JITTER, SIGMA_FLOOR));
+}
+
+template <int KID, int L>
+cudaError_t store_l(const SSProblem& p, const double* hyp, double* ll, int* info, const SSStore& st, cudaStream_t stream) {
+    if (p.L == L) {
+        ss_filter_kernel<KID, L, false, true><<<1, 32, 0, stream>>>(p, 1, hyp, hyp + L, hyp + 2 * L, ll, nullptr, info, nullptr, st);
+        ss_adjoint_kernel<KID, L><<<1, 32, 0, stream>>>(p, hyp, info, st);
+        return cudaGetLastError();
+    }
+    if constexpr (L < MAX_BANDS) return store_l<KID, L + 1>(p, hyp, ll, info, st, stream);
+    return cudaErrorInvalidValue;
+}
+
+template <int KID, int L>
+cudaError_t point_l(const SSProblem& p, const double* hyp, const SSStore& st, int NT, const double* tt, const int* bt,
+                    double* mu, double* sd, cudaStream_t stream) {
+    if (p.L == L) {
+        ss_point_kernel<KID, L><<<(NT + 127) / 128, 128, 0, stream>>>(p, hyp, st, NT, tt, bt, mu, sd);
+        return cudaGetLastError();
+    }
+    if constexpr (L < MAX_BANDS) return point_l<KID, L + 1>(p, hyp, st, NT, tt, bt, mu, sd, stream);
     return cudaErrorInvalidValue;
 }
 
@@ -254,6 +472,31 @@ cudaError_t statespace_launch(int kernel_id, const SSProblem& p, const EvalBatch
         case K_M32: return launch_l<K_M32, 1>(p, b, postb, stream);
         case K_M52: return launch_l<K_M52, 1>(p, b, postb, stream);
         default:       return cudaErrorInvalidValue;     // rbf: rejected by gpcc_problem_set_method
+    }
+}
+
+}  // namespace gpcc
+
+namespace gpcc {
+
+cudaError_t statespace_store_launch(int kernel_id, const SSProblem& p, const double* hyp, double* ll, int* info,
+                                    const SSStore& st, cudaStream_t stream) {
+    switch (kernel_id) {
+        case K_OU:  return store_l<K_OU, 1>(p, hyp, ll, info, st, stream);
+        case K_M32: return store_l<K_M32, 1>(p, hyp, ll, info, st, stream);
+        case K_M52: return store_l<K_M52, 1>(p, hyp, ll, info, st, stream);
+        default:    return cudaErrorInvalidValue;
+    }
+}
+
+cudaError_t statespace_predict_launch(int kernel_id, const SSProblem& p, const double* hyp, const SSStore& st, int NT,
+                                      const double* tt, const int* bt, double* mu, double* sd, cudaStream_t stream) {
+    if (NT <= 0) return cudaSuccess;
+    switch (kernel_id) {
+        case K_OU:  return point_l<K_OU, 1>(p, hyp, st, NT, tt, bt, mu, sd, stream);
+        case K_M32: return point_l<K_M32, 1>(p, hyp, st, NT, tt, bt, mu, sd, stream);
+        case K_M52: return point_l<K_M52, 1>(p, hyp, st, NT, tt, bt, mu, sd, stream);
+        default:    return cudaErrorInvalidValue;
     }
 }
 

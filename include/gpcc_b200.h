@@ -42,6 +42,7 @@ enum { GPCC_METHOD_DENSE = 0, GPCC_METHOD_STATESPACE = 1 };
 typedef struct gpcc_ctx gpcc_ctx;
 typedef struct gpcc_problem gpcc_problem;
 typedef struct gpcc_fit_state gpcc_fit_state;
+typedef struct gpcc_ss_state gpcc_ss_state;
 
 /* Keyword arguments / constants of gpcc (src/gpccfixdelay_marginaliseb.jl:46, :69, :112, :205). */
 typedef struct gpcc_fit_options {
@@ -83,7 +84,7 @@ typedef struct gpcc_stats {
                                    tiles imported from the last-band cache count read + written); pairs with ms_assembly      */
 } gpcc_stats;
 
-int         gpcc_version(void);   /* 102.  101 -> 102: gpcc_problem_set_method (additive).
+int         gpcc_version(void);   /* 103.  102 -> 103: gpcc_ss_state_* (additive).  101 -> 102: gpcc_problem_set_method (additive).
                                       100 -> 101: gpcc_stats grew by n_tau_cache and assembly_bytes (appended at the end);
                                       a caller built against 100 must be rebuilt before it calls gpcc_ctx_get_stats                */
 const char* gpcc_last_error(void);
@@ -125,7 +126,9 @@ int gpcc_problem_get_prior(const gpcc_problem* p, double* mub, double* Sigmab);
  *     evaluation per round), whatever N is; GPCC_OPT_NELDERMEAD is rejected with -7;
  *   - gpcc_postb runs one filter and returns its final b-block;
  *   - gpcc_fit_state_*, gpcc_predict, gpcc_predict_loglik and gpcc_fit_state_sample stay dense: a fit state is a
- *     Cholesky factor of K + Sobs.
+ *     Cholesky factor of K + Sobs;
+ *   - gpcc_ss_state_create builds the O(N) fit state of this method (see below): predictive means, standard deviations
+ *     and the test log-likelihood without a factorisation.
  * Returns < 0 for a NULL problem, an unknown method, or rbf with GPCC_METHOD_STATESPACE.                              */
 int gpcc_problem_set_method(gpcc_problem* p, int method);
 
@@ -207,6 +210,26 @@ int gpcc_predict(gpcc_problem* p, const double* delays, const double* alpha, dou
 int gpcc_predict_loglik(gpcc_problem* p, const double* delays, const double* alpha, double rho,
                         const int* ntest_per_band, const double* ttest, const double* ytest,
                         const double* sigmatest, double* out_ll, int* out_info);
+
+/* Fit state of the state-space method (a problem in GPCC_METHOD_STATESPACE; OU, matern32, matern52) at (delays, alpha, rho):
+ * one forward Kalman filter that stores its filtered moments and one backward (Bryson-Frazier) pass over the N merged
+ * training points, on the problem's first device.  O(N (d+L)^2) memory and time, no N x N matrix.  The state owns all it
+ * reads (its own copy of the sorted training data, mu_b, Sigma_b and ll(train)): it may be used after its problem is
+ * destroyed or switched back to GPCC_METHOD_DENSE.  Returns < 0 for a NULL argument, a problem not in
+ * GPCC_METHOD_STATESPACE, alpha <= 0, rho <= 0 or non-finite values; -6 when the filter meets an innovation variance
+ * that is not positive and finite.                                                                                      */
+int gpcc_ss_state_create(gpcc_problem* p, const double* delays, const double* alpha, double rho, gpcc_ss_state** out);
+int gpcc_ss_state_destroy(gpcc_ss_state* s);
+/* Per-point predictTest (:293-307): out_mu[NT] and out_sd[NT] (may be NULL) as gpcc_fit_state_predict returns them (sd =
+ * sqrt(max(var + 1e-8, 1e-6))), in O((d+L)^3) per test point; test times in any order.  The full predictive covariance
+ * needs the dense fit state.  Returns < 0 for negative counts or non-finite times; NT = 0 does nothing.             */
+int gpcc_ss_state_predict(gpcc_ss_state* s, const int* ntest_per_band, const double* ttest, double* out_mu, double* out_sd);
+/* Test log-likelihood (:311-343), logpdf(N(mu_pred, Sigma_pred + diag(sigmatest^2)), ytest) with the 1e-8 jitter in
+ * Sigma_pred, as ll(train + test) - ll(train): one filter over the N + NT merged points.  out_info (may be NULL) = 0, or the
+ * 1-based merged position of the first innovation variance that is not positive and finite (out_ll = -Inf).  Returns < 0
+ * for negative counts, non-finite times or values, or sigmatest < 0; NT = 0 gives out_ll = 0.                         */
+int gpcc_ss_state_predict_loglik(gpcc_ss_state* s, const int* ntest_per_band, const double* ttest, const double* ytest,
+                                 const double* sigmatest, double* out_ll, int* out_info);
 
 /* Fill `opt` with the reference defaults (seed-independent part of :46, :112, :205).               */
 int gpcc_fit_options_default(gpcc_fit_options* opt);

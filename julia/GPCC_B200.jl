@@ -10,7 +10,7 @@ module GPCC_B200
 using Distributions, LinearAlgebra, Random, Printf
 import MiscUtil    # only to assert at load time that the library's transform formulas match MiscUtil's
 
-export gpcc, gpccgrid, getprobabilities, uniformpriordelay, OU, rbf, matern32, matern52
+export gpcc, gpccgrid, getprobabilities, uniformpriordelay, OU, rbf, matern32, matern52, statespace_fit_state
 
 const LIB = get(ENV, "GPCC_B200_LIB", joinpath(@__DIR__, "..", "gpcc_b200", "libgpcc_b200.so"))
 
@@ -68,7 +68,8 @@ mutable struct Problem
 end
 
 # :dense factorises K + Sobs + B; :statespace (OU, matern32, matern52) runs the exact O(N) Kalman filter
-# (gpcc_problem_set_method in include/gpcc_b200.h).  Fit states behind `pred` are dense under either method.
+# (gpcc_problem_set_method in include/gpcc_b200.h).  Fit states behind `pred` of `gpcc` are dense under either method;
+# `statespace_fit_state` is the O(N) fit state of :statespace.
 const METHODS = Dict(:dense => Cint(0), :statespace => Cint(1))
 setmethod!(p::Problem, method::Symbol) =
     check(ccall((:gpcc_problem_set_method, LIB), Cint, (Ptr{Cvoid}, Cint), p.h, METHODS[method]))
@@ -173,6 +174,46 @@ function gpcc(tarray, yarray, stdarray; kernel = kernel, delays = delays, iterat
         ll_[]
     end
     ll[b], predictTest, (α, postb, ρ)
+end
+
+# The O(N) fit state of the state-space method (gpcc_ss_state_*): filtered moments and backward-pass adjoint, no N x N matrix.
+mutable struct SSFitState
+    h::Ptr{Cvoid}; p::Problem
+    function SSFitState(p::Problem, d::Vector{Float64}, α::Vector{Float64}, ρ::Float64)
+        r = Ref{Ptr{Cvoid}}(C_NULL)
+        GC.@preserve d α check(ccall((:gpcc_ss_state_create, LIB), Cint, (Ptr{Cvoid}, Ptr{Cdouble}, Ptr{Cdouble}, Cdouble, Ref{Ptr{Cvoid}}), p.h, d, α, ρ, r))
+        s = new(r[], p); finalizer(s -> ccall((:gpcc_ss_state_destroy, LIB), Cint, (Ptr{Cvoid},), s.h), s); s   # the state owns its data
+    end
+end
+
+"""
+    pred = statespace_fit_state(tarray, yarray, stdarray; kernel, delays, α, ρ)
+
+`pred` at fixed (delays, α, ρ) from the O(N) fit state of the state-space method (OU, matern32, matern52): `pred(ttest)`
+gives per band (μ, σ) (:293-307) and `pred(ttest, ytest, σtest)` the test log-likelihood (:311-343), for light curves far
+beyond a dense factorisation.  The full predictive covariance (`pred(::Vector{Vector})`) needs the dense state of `gpcc`.
+"""
+function statespace_fit_state(tarray, yarray, stdarray; kernel = kernel, delays = delays, α = α, ρ = ρ)
+    p = Problem(defaultctx(), tarray, yarray, stdarray, kernel); L = p.L
+    setmethod!(p, :statespace)
+    st = SSFitState(p, Float64.(delays), Float64.(α), Float64(ρ))
+    function predictTest(ttest::Union{AbstractRange{Float64}, Array{Float64, 1}})                                          # :293-307
+        Nt = length(ttest); nt = fill(Cint(Nt), L); tt = repeat(Float64.(collect(ttest)), L); μp = zeros(L * Nt); σp = zeros(L * Nt)
+        GC.@preserve nt tt μp σp check(ccall((:gpcc_ss_state_predict, LIB), Cint,
+            (Ptr{Cvoid}, Ptr{Cint}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}), st.h, nt, tt, μp, σp))
+        [μp[idx] for idx in Iterators.partition(1:L*Nt, Nt)], [σp[idx] for idx in Iterators.partition(1:L*Nt, Nt)]
+    end
+    predictTest(ttest::Array{Array{Float64, 1}, 1}) =
+        error("the state-space fit state gives per-point means and standard deviations: the full predictive covariance needs the dense state of gpcc")
+    function predictTest(ttest::Array{Array{Float64, 1}, 1}, ytest::Array{Array{Float64, 1}, 1}, σtest::Array{Array{Float64, 1}, 1})   # :311-343
+        nt = Cint.(length.(ttest)); tt = reduce(vcat, ttest); yt = reduce(vcat, ytest); σt = reduce(vcat, σtest)
+        ll_ = Ref{Cdouble}(0.0); info = Ref{Cint}(0)
+        GC.@preserve nt tt yt σt check(ccall((:gpcc_ss_state_predict_loglik, LIB), Cint,
+            (Ptr{Cvoid}, Ptr{Cint}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ref{Cdouble}, Ref{Cint}), st.h, nt, tt, yt, σt, ll_, info))
+        info[] == 0 || error("non-positive innovation variance at merged position $(info[]): the nearestposdef repair needs the dense state of gpcc")
+        ll_[]
+    end
+    predictTest
 end
 
 """
