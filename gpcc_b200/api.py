@@ -178,7 +178,8 @@ class Problem:
     `method` selects how the likelihood is evaluated: "dense" (default) factorises K + Sobs + B; "statespace" (OU,
     matern32, matern52) runs an exact Kalman filter in O(N) per evaluation (gpcc_problem_set_method), for light curves
     far beyond what a dense factorisation can hold.  `fit_state` and the prediction methods stay dense under either
-    method; `statespace_fit_state` is the O(N) fit state of the state-space method."""
+    method; `statespace_fit_state` is the O(N) fit state of the state-space method and `statespace_sample` its O(N)
+    draw."""
 
     def __init__(self, tarray, yarray, stdarray, kernel, ctx=None, method="dense"):
         self.ctx = ctx or default_context()
@@ -288,6 +289,24 @@ class Problem:
         """O(N) fit state of the state-space method (gpcc_ss_state_*): per-point predictions and the test log-likelihood
         without a dense factorisation.  Needs method="statespace"."""
         return StateSpaceFitState(self, delays, alpha, rho)
+
+    def statespace_sample(self, delays, alpha, rho, seed, nsamples=1, z=None, return_z=False):
+        """Exact draws f ~ N(0, K + Sobs) in O(N) (gpcc_ss_sample), shape (nsamples, N) in input order.  Needs
+        method="statespace".  z (nsamples, N, d+1), d = 1, 2, 3 for OU, matern32, matern52: the d process deviates and
+        the noise deviate of every point, used instead of the generator (seed is then ignored).  return_z=True also
+        returns the deviates used."""
+        delays, alpha = _f64(delays, (self.L,)), _f64(alpha, (self.L,))
+        d = {OU.kid: 1, matern32.kid: 2, matern52.kid: 3}.get(self.kernel_id, 1)
+        ns = int(nsamples)
+        if z is not None:
+            z = _f64(z)
+            if z.shape != (ns, self.N, d + 1):
+                raise GpccError(f"z must have shape (nsamples, N, d+1) = {(ns, self.N, d + 1)}")
+        f = np.empty((max(ns, 0), self.N))
+        zo = np.empty((max(ns, 0), self.N, d + 1)) if return_z else None
+        check(_lib.load().gpcc_ss_sample(self._h, _d(delays), _d(alpha), float(rho), int(seed) & (2 ** 64 - 1), ns, _d(z),
+                                         _d(f), _d(zo)))
+        return (f, zo) if return_z else f
 
     def postb(self, delays, alpha, rho):
         delays, alpha = _f64(delays, (self.L,)), _f64(alpha, (self.L,))
@@ -574,19 +593,26 @@ def gpccgrid(tarray, yarray, stdarray, candidatedelays, *, kernel, iterations, s
                             logprior=logprior)
 
 
-def simulatedata_device(tarray, *, delays, alpha, b, rho=3.5, sigma=0.75, kernel=OU, seed=1, ctx=None):
+def simulatedata_device(tarray, *, delays, alpha, b, rho=3.5, sigma=0.75, kernel=OU, seed=1, ctx=None, method="dense"):
     """The reference's simulator (src/simulatedata.jl:96-162) with the O(N^3) part on the device: the latent process is drawn
     from N(0, C + 1e-6 I), C = delayedCovariance(kernel, alpha, delays, rho, tarray) (:128; the 1e-6 stands in for the
-    eigenvalue clamp of :132-138), through the tiled Cholesky and the device generator of gpcc_fit_state_sample; scaling,
-    offsets and observation noise (:151-159, alpha applied a second time as the reference does) are host arithmetic.
-    Returns (tarray, yarray, stdarray).  Meant for large synthetic benchmarks (N in the thousands)."""
+    eigenvalue clamp of :132-138); scaling, offsets and observation noise (:151-159, alpha applied a second time as the
+    reference does) are host arithmetic.  Returns (tarray, yarray, stdarray).
+    method="dense" (default) draws through the tiled Cholesky and the generator of gpcc_fit_state_sample, for N in the
+    thousands; method="statespace" draws exactly in O(N) through gpcc_ss_sample, for any N (OU, matern32, matern52)."""
     tarray = [_f64(a) for a in tarray]
     L = len(tarray)
+    if method not in _METHODS:
+        raise GpccError("method must be 'dense' or 'statespace'")
     dummy = [np.arange(len(a), dtype=np.float64) for a in tarray]              # the prior of b needs a variance; unused by the draw
-    p = Problem(tarray, dummy, [np.full(len(a), 1e-3) for a in tarray], kernel, ctx)
-    st = p.fit_state(delays, alpha, rho)
-    f = st.sample(seed, 1)[0]
-    st.close(); p.close()
+    p = Problem(tarray, dummy, [np.full(len(a), 1e-3) for a in tarray], kernel, ctx, method)
+    if method == "statespace":
+        f = p.statespace_sample(delays, alpha, rho, seed)[0]
+    else:
+        st = p.fit_state(delays, alpha, rho)
+        f = st.sample(seed, 1)[0]
+        st.close()
+    p.close()
     rg = np.random.default_rng(seed)
     y, mark = [], 0
     for l in range(L):

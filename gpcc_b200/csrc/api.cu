@@ -423,7 +423,7 @@ int fit_all(gpcc_problem* p, int M, const double* delays, int P, const double* t
 // =====================================================================================================
 extern "C" {
 
-int gpcc_version(void) { return 103; }   // 103: gpcc_ss_state_*; 102: gpcc_problem_set_method; 101: gpcc_stats grew by n_tau_cache and assembly_bytes
+int gpcc_version(void) { return 103; }   // 103: gpcc_ss_state_*, then gpcc_ss_sample (additive, same number); 102: gpcc_problem_set_method; 101: gpcc_stats grew by n_tau_cache and assembly_bytes
 const char* gpcc_last_error(void) { return gpcc::last_error().c_str(); }
 
 int gpcc_fit_options_default(gpcc_fit_options* o) {
@@ -586,8 +586,10 @@ int gpcc_problem_get_prior(const gpcc_problem* p, double* mub, double* Sigmab) {
 
 }  // extern "C"
 
-// Per band, a stable argsort of t: the merge of the filter (statespace.cu) keeps this order within a band.
-static void sort_bands(const gpcc_problem* p, std::vector<double>& t, std::vector<double>& r, std::vector<double>& s2) {
+// Per band, a stable argsort of t: the merge of the filter (statespace.cu) keeps this order within a band.  ord (may be
+// NULL) receives the input index of every sorted point.
+static void sort_bands(const gpcc_problem* p, std::vector<double>& t, std::vector<double>& r, std::vector<double>& s2,
+                       std::vector<int>* ord_out = nullptr) {
     const int N = p->N;
     std::vector<int> ord(N);
     for (int i = 0; i < N; ++i) ord[i] = i;
@@ -596,6 +598,7 @@ static void sort_bands(const gpcc_problem* p, std::vector<double>& t, std::vecto
                          [&](int a, int b) { return p->t[a] < p->t[b]; });
     t.resize(N); r.resize(N); s2.resize(N);
     for (int i = 0; i < N; ++i) { t[i] = p->t[ord[i]]; r[i] = p->resid[ord[i]]; s2[i] = p->s2[ord[i]]; }
+    if (ord_out) ord_out->swap(ord);
 }
 
 extern "C" {
@@ -608,16 +611,19 @@ int gpcc_problem_set_method(gpcc_problem* p, int method) {
     if (method == GPCC_METHOD_STATESPACE) {
         const int N = p->N, L = p->L;
         std::vector<double> t, r, s2;
-        sort_bands(p, t, r, s2);
+        std::vector<int> ord;
+        sort_bands(p, t, r, s2, &ord);
         for (auto& d : p->pd) {
             CUDA_TRY(cudaSetDevice(d.dev));
             CUDA_TRY(d.ss_t.reserve(N));
             CUDA_TRY(d.ss_r.reserve(N));
             CUDA_TRY(d.ss_s2.reserve(N));
+            CUDA_TRY(d.ss_perm.reserve(N));
             CUDA_TRY(d.ss_postb.reserve((size_t)L + (size_t)L * L));
             CUDA_TRY(cudaMemcpy(d.ss_t.d, t.data(), N * sizeof(double), cudaMemcpyHostToDevice));
             CUDA_TRY(cudaMemcpy(d.ss_r.d, r.data(), N * sizeof(double), cudaMemcpyHostToDevice));
             CUDA_TRY(cudaMemcpy(d.ss_s2.d, s2.data(), N * sizeof(double), cudaMemcpyHostToDevice));
+            CUDA_TRY(cudaMemcpy(d.ss_perm.d, ord.data(), N * sizeof(int), cudaMemcpyHostToDevice));
             SSProblem& q = d.ssp;
             q.N = N; q.L = L;
             for (int l = 0; l <= L; ++l) q.band_start[l] = p->band_start[l];
@@ -1004,6 +1010,52 @@ int ss_state_create(gpcc_problem* p, const double* delays, const double* alpha, 
     return 0;
 }
 
+// The argument checks of the calls that take a state-space problem and its hyper-parameters.
+int ss_check_hyper(const gpcc_problem* p, const double* delays, const double* alpha, double rho) {
+    if (!p || !delays || !alpha) return fail(-1, "NULL argument");
+    if (p->method != GPCC_METHOD_STATESPACE) return fail(-5, "the problem is not in GPCC_METHOD_STATESPACE (gpcc_problem_set_method)");
+    for (int l = 0; l < p->L; ++l) {
+        if (!(alpha[l] > 0) || !std::isfinite(alpha[l])) return fail(-2, "all(scale .> 0) violated (delayedCovariance.jl:3)");
+        if (!std::isfinite(delays[l])) return fail(-3, "non-finite delay");
+    }
+    if (!(rho > 0) || !std::isfinite(rho)) return fail(-4, "rho is <= 0 (delayedCovariance.jl:5-7)");
+    return 0;
+}
+
+// gpcc_ss_sample after its checks: the five kernels of ss_sample.cu on the first device and stream.
+int ss_sample(gpcc_problem* p, const double* delays, const double* alpha, double rho, unsigned long long seed, int nsamples,
+              const double* z_in, double* out_f, double* out_z) {
+    const int N = p->N, L = p->L, d = p->kernel_id == GPCC_KERNEL_OU ? 1 : p->kernel_id == GPCC_KERNEL_MATERN32 ? 2 : 3;
+    const size_t nf = (size_t)nsamples * N, nz = nf * (d + 1);
+    gpcc_problem::PerDev& pd = p->pd[0];
+    DeviceState& ds = p->ctx->ds[0];
+    CUDA_TRY(cudaSetDevice(pd.dev));
+    cudaStream_t st = ds.stream.get();
+    SSSampleBuffers& b = pd.ss_smp;
+    size_t n_step, n_aggA, n_aggc;
+    statespace_sample_scratch(p->kernel_id, N, nsamples, n_step, n_aggA, n_aggc);
+    CUDA_TRY(b.ints.reserve(2 * (size_t)N));
+    CUDA_TRY(b.step.reserve(n_step));
+    CUDA_TRY(b.aggA.reserve(n_aggA));
+    CUDA_TRY(b.aggc.reserve(n_aggc));
+    CUDA_TRY(b.f.reserve(nf));
+    if (z_in || out_z) CUDA_TRY(b.z.reserve(nz));
+    if (z_in) CUDA_TRY(cudaMemcpyAsync(b.z.d, z_in, nz * sizeof(double), cudaMemcpyHostToDevice, st));
+    SSSampleArgs a;
+    for (int l = 0; l < L; ++l) { a.tau[l] = delays[l]; a.alpha[l] = alpha[l]; }
+    a.rho = rho; a.seed = seed; a.nsamples = nsamples; a.perm = pd.ss_perm.d;
+    a.zin = z_in ? b.z.d : nullptr;
+    a.zout = out_z && !z_in ? b.z.d : nullptr;
+    a.f = b.f.d;
+    SSSampleScratch sc{b.ints.d, b.ints.d + N, b.step.d, b.aggA.d, b.aggc.d};
+    CUDA_TRY(statespace_sample_launch(p->kernel_id, pd.ssp, a, sc, st));
+    CUDA_TRY(cudaMemcpyAsync(out_f, b.f.d, nf * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (out_z) CUDA_TRY(cudaMemcpyAsync(out_z, b.z.d, nz * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    ds.launches += 5;
+    return 0;
+}
+
 // Test points of one call: counts, band of every point in input order, and the checks shared by both calls.
 int ss_test_points(const gpcc_ss_state* s, const int* ntest_per_band, const double* ttest, std::vector<int>& bt) {
     if (!s || !ntest_per_band) return fail(-1, "NULL argument");
@@ -1030,13 +1082,8 @@ extern "C" {
 int gpcc_ss_state_create(gpcc_problem* p, const double* delays, const double* alpha, double rho, gpcc_ss_state** out) {
     if (!out) return fail(-1, "out is NULL");
     *out = nullptr;
-    if (!p || !delays || !alpha) return fail(-1, "NULL argument");
-    if (p->method != GPCC_METHOD_STATESPACE) return fail(-5, "the problem is not in GPCC_METHOD_STATESPACE (gpcc_problem_set_method)");
-    for (int l = 0; l < p->L; ++l) {
-        if (!(alpha[l] > 0) || !std::isfinite(alpha[l])) return fail(-2, "all(scale .> 0) violated (delayedCovariance.jl:3)");
-        if (!std::isfinite(delays[l])) return fail(-3, "non-finite delay");
-    }
-    if (!(rho > 0) || !std::isfinite(rho)) return fail(-4, "rho is <= 0 (delayedCovariance.jl:5-7)");
+    int rc = ss_check_hyper(p, delays, alpha, rho);
+    if (rc) return rc;
     return ss_state_create(p, delays, alpha, rho, out);
 }
 
@@ -1133,6 +1180,21 @@ int gpcc_ss_state_predict_loglik(gpcc_ss_state* s, const int* ntest_per_band, co
     *out_ll = info ? -std::numeric_limits<double>::infinity() : ll - s->ll_train;
     if (out_info) *out_info = info;
     return 0;
+}
+
+int gpcc_ss_sample(gpcc_problem* p, const double* delays, const double* alpha, double rho, unsigned long long seed, int nsamples,
+                   const double* z_in, double* out_f, double* out_z) {
+    if (!out_f) return fail(-1, "NULL argument");
+    int rc = ss_check_hyper(p, delays, alpha, rho);
+    if (rc) return rc;
+    if (nsamples < 1) return fail(-7, "nsamples < 1");
+    if (z_in) {
+        const size_t d = p->kernel_id == GPCC_KERNEL_OU ? 1 : p->kernel_id == GPCC_KERNEL_MATERN32 ? 2 : 3;
+        const size_t nz = (size_t)nsamples * p->N * (d + 1);
+        for (size_t k = 0; k < nz; ++k)
+            if (!std::isfinite(z_in[k])) return fail(-8, "non-finite deviate in z_in");
+    }
+    return ss_sample(p, delays, alpha, rho, seed, nsamples, z_in, out_f, out_z);
 }
 
 }  // extern "C"

@@ -161,6 +161,29 @@ cudaError_t statespace_store_launch(int kernel_id, const SSProblem& p, const dou
 cudaError_t statespace_predict_launch(int kernel_id, const SSProblem& p, const double* hyp, const SSStore& st, int NT,
                                       const double* tt, const int* bt, double* mu, double* sd, cudaStream_t stream);
 
+// ---- exact O(N) draws of the state-space model (ss_sample.cu): the SDE recurrence over the merged times, as a scan ----
+struct SSSampleArgs {
+    double tau[MAX_BANDS] = {0}, alpha[MAX_BANDS] = {0}, rho = 0;
+    unsigned long long seed = 0;
+    int nsamples = 0;
+    const int* perm = nullptr;    // [N] input index of the point at each position of p's sorted per-band copy
+    const double* zin = nullptr;  // [nsamples][N][d+1] deviates in input order, or NULL: Philox from (seed, sample, point)
+    double* zout = nullptr;       // [nsamples][N][d+1] or NULL: the deviates used
+    double* f = nullptr;          // [nsamples][N] draws in input order
+};
+struct SSSampleScratch {          // sizes from statespace_sample_scratch
+    int* order = nullptr;         // [N] merged step -> sorted position
+    int* idx = nullptr;           // [N] merged step -> input index
+    double* step = nullptr;       // [N][d*d + d(d+1)/2 + 2] A, packed lower C, alpha, sigma of every merged step
+    double* aggA = nullptr;       // [tiles][d*d]
+    double* aggc = nullptr;       // [nsamples][tiles][d]
+};
+// doubles of SSSampleScratch::step, aggA and aggc (ints: 2 N)
+void statespace_sample_scratch(int kernel_id, int N, int nsamples, size_t& n_step, size_t& n_aggA, size_t& n_aggc);
+// Five launches on `stream`: merged ranks, per-step factors, tile aggregates, scan of the aggregates, tile re-run.
+cudaError_t statespace_sample_launch(int kernel_id, const SSProblem& p, const SSSampleArgs& a, const SSSampleScratch& s,
+                                     cudaStream_t stream);
+
 // ---- posterior over candidates (posterior.cu): src/getprobabilities.jl:10-20 --------------------
 cudaError_t posterior_launch(int M, const double* d_ll, const double* d_logprior, double* d_out, cudaStream_t stream,
                              bool joint_already = false);

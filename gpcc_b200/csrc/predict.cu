@@ -20,6 +20,7 @@
 // a quantity of size Sigma_b and is held to 1e-8 against 50-digit arithmetic (tests/golden/pred_exact.npz).
 #include "state.h"
 #include "kernfun.cuh"
+#include "philox.cuh"
 #include <cmath>
 #include <cstring>
 #include <limits>
@@ -369,21 +370,9 @@ __global__ void __launch_bounds__(1024) chol_logpdf_kernel(int n, double* __rest
 
 // ---------------------------------------------------------------------------------------------------------------------
 // Sampling from the fitted process (the draw of src/simulatedata.jl:128-145, Y ~ MvNormal(0, C), on the device).
-// Counter-based generator: Philox-4x32-10 (Salmon et al. 2011), counter = (index, 0, sample stream, 0), key = seed; two
+// Counter-based generator: Philox-4x32-10 (philox.cuh), counter = (index, 0, sample stream, 0), key = seed; two
 // 53-bit uniforms per call -> Box-Muller pair.  Reproducible for a given seed whatever the launch geometry.
 // ---------------------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
-#pragma unroll
-    for (int r = 0; r < 10; ++r) {
-        const unsigned hi0 = __umulhi(0xD2511F53u, c.x), lo0 = 0xD2511F53u * c.x;
-        const unsigned hi1 = __umulhi(0xCD9E8D57u, c.z), lo1 = 0xCD9E8D57u * c.z;
-        c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
-        k.x += 0x9E3779B9u;
-        k.y += 0xBB67AE85u;
-    }
-    return c;
-}
-
 __global__ void normal_kernel(size_t n, unsigned long long seed, double* __restrict__ z) {
     const uint2 key = make_uint2((unsigned)seed, (unsigned)(seed >> 32));
     for (size_t pair = (size_t)blockIdx.x * blockDim.x + threadIdx.x; 2 * pair < n; pair += (size_t)gridDim.x * blockDim.x) {

@@ -184,6 +184,35 @@ GPCC_HD inline void step(const Coef<Dim<KID>::d>& c, double D, double (&A)[Dim<K
     }
 }
 
+// Lower Cholesky factor C (C C' = Q, upper part zero) of a process noise or stationary covariance (the sampler of
+// ss_sample.cu).  Q's entries span many orders of magnitude at small lambda D (Q_ij ~ D^(2d-1-i-j)), so Q is factored in
+// diagonally scaled form, Q = S R S with S = diag(sqrt(Q_ii)) and R the correlation matrix, C = S chol(R): its rounding
+// error is relative to sqrt(Q_ii Q_jj) entry by entry.  A zero diagonal entry or a non-positive pivot (rounding) gives a
+// zero column, so D = 0 (Q = 0 exactly) gives C = 0 exactly.
+template <int d>
+GPCC_HD inline void noise_factor(const double (&Q)[d][d], double (&C)[d][d]) {
+    double s[d];
+    for (int i = 0; i < d; ++i) s[i] = Q[i][i] > 0.0 ? sqrt(Q[i][i]) : 0.0;
+    for (int i = 0; i < d; ++i)
+        for (int j = 0; j < d; ++j) C[i][j] = 0.0;
+    for (int j = 0; j < d; ++j) {                 // column j of chol(R), then scaled by S
+        if (!(s[j] > 0.0)) continue;
+        double p = 1.0;
+        for (int k = 0; k < j; ++k) p -= C[j][k] * C[j][k];
+        if (!(p > 0.0)) continue;
+        const double cjj = sqrt(p);
+        C[j][j] = cjj;
+        for (int i = j + 1; i < d; ++i) {
+            if (!(s[i] > 0.0)) continue;
+            double r = Q[i][j] / (s[i] * s[j]);
+            for (int k = 0; k < j; ++k) r -= C[i][k] * C[j][k];
+            C[i][j] = r / cjj;
+        }
+    }
+    for (int i = 0; i < d; ++i)
+        for (int j = 0; j <= i; ++j) C[i][j] *= s[i];
+}
+
 template <int D>
 GPCC_HD constexpr int sym(int i, int j) {      // packed upper triangle, row-major
     return i <= j ? i * D - i * (i - 1) / 2 + (j - i) : j * D - j * (j - 1) / 2 + (i - j);

@@ -63,6 +63,11 @@ struct DeviceState {
     ~DeviceState() { cudaSetDevice(dev); }
 };
 
+struct SSSampleBuffers {
+    DevArray<int> ints;                          // order, idx: [2 N]
+    DevArray<double> step, aggA, aggc, f, z;     // SSSampleScratch; f [nsamples][N]; z [nsamples][N][d+1] (z_in, or the deviates)
+};
+
 struct FitStateDelete { void operator()(gpcc_fit_state* s) const { gpcc_fit_state_destroy(s); } };
 
 }  // namespace gpcc
@@ -86,6 +91,8 @@ struct gpcc_problem {
         gpcc::DevArray<int> band;
         gpcc::DevProblem dp;
         gpcc::DevArray<double> ss_t, ss_r, ss_s2;   // state-space method: each band sorted by t (gpcc_problem_set_method)
+        gpcc::DevArray<int> ss_perm;                // ... and the input index of each of those points
+        gpcc::SSSampleBuffers ss_smp;               // scratch and outputs of gpcc_ss_sample (first device), kept between calls
         gpcc::DevBuf<double> ss_postb;              // [L + L*L] postb of the filter
         gpcc::SSProblem ssp;
         ~PerDev() { cudaSetDevice(dev); }

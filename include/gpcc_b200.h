@@ -84,7 +84,8 @@ typedef struct gpcc_stats {
                                    tiles imported from the last-band cache count read + written); pairs with ms_assembly      */
 } gpcc_stats;
 
-int         gpcc_version(void);   /* 103.  102 -> 103: gpcc_ss_state_* (additive).  101 -> 102: gpcc_problem_set_method (additive).
+int         gpcc_version(void);   /* 103.  102 -> 103: gpcc_ss_state_* (additive); gpcc_ss_sample was added later under the same
+                                      number (additive: a caller that needs it looks the symbol up).  101 -> 102: gpcc_problem_set_method (additive).
                                       100 -> 101: gpcc_stats grew by n_tau_cache and assembly_bytes (appended at the end);
                                       a caller built against 100 must be rebuilt before it calls gpcc_ctx_get_stats                */
 const char* gpcc_last_error(void);
@@ -128,7 +129,9 @@ int gpcc_problem_get_prior(const gpcc_problem* p, double* mub, double* Sigmab);
  *   - gpcc_fit_state_*, gpcc_predict, gpcc_predict_loglik and gpcc_fit_state_sample stay dense: a fit state is a
  *     Cholesky factor of K + Sobs;
  *   - gpcc_ss_state_create builds the O(N) fit state of this method (see below): predictive means, standard deviations
- *     and the test log-likelihood without a factorisation.
+ *     and the test log-likelihood without a factorisation;
+ *   - gpcc_ss_sample draws from N(0, K + Sobs) in O(N), the O(N) form of gpcc_fit_state_sample.
+ * The full predictive covariance has no O(N) form and stays dense.
  * Returns < 0 for a NULL problem, an unknown method, or rbf with GPCC_METHOD_STATESPACE.                              */
 int gpcc_problem_set_method(gpcc_problem* p, int method);
 
@@ -230,6 +233,19 @@ int gpcc_ss_state_predict(gpcc_ss_state* s, const int* ntest_per_band, const dou
  * for negative counts, non-finite times or values, or sigmatest < 0; NT = 0 gives out_ll = 0.                         */
 int gpcc_ss_state_predict_loglik(gpcc_ss_state* s, const int* ntest_per_band, const double* ttest, const double* ytest,
                                  const double* sigmatest, double* out_ll, int* out_info);
+
+/* Exact draws f ~ N(0, K + Sobs) at (delays, alpha, rho) for a problem in GPCC_METHOD_STATESPACE, the distribution of
+ * gpcc_fit_state_sample, in O(N) time and memory: the kernel's SDE recurrence over the merged, delay-shifted times, run as a
+ * parallel scan on the problem's first device.  out_f[nsamples][N] is in the problem's input order.  Deviates: d process
+ * deviates then 1 noise deviate per point (d = 1, 2, 3 for OU, matern32, matern52), [nsamples][N][d+1]; the d process
+ * deviates of point i drive the step of the recurrence that arrives at i.  z_in (may be NULL) supplies them, and seed is
+ * then ignored; otherwise they come from Philox-4x32-10 + Box-Muller and depend only on (seed, sample, point), so a draw
+ * does not depend on nsamples and the same seed gives common random numbers across delays.  out_z (may be NULL) receives
+ * the deviates used.  Bitwise reproducible.  Returns < 0 as gpcc_ss_state_create does (-1 NULL, -2 alpha <= 0, -3
+ * non-finite delay, -4 rho <= 0, -5 problem not in GPCC_METHOD_STATESPACE), -7 for nsamples < 1 and -8 for a non-finite
+ * value in z_in.                                                                                                        */
+int gpcc_ss_sample(gpcc_problem* p, const double* delays, const double* alpha, double rho, unsigned long long seed,
+                   int nsamples, const double* z_in, double* out_f, double* out_z);
 
 /* Fill `opt` with the reference defaults (seed-independent part of :46, :112, :205).               */
 int gpcc_fit_options_default(gpcc_fit_options* opt);
