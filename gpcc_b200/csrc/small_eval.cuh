@@ -12,7 +12,7 @@
 //   * assembly is fused: every thread evaluates its 64 kernel entries from the shifted times in smem;
 //   * one symmetric Gauss-Jordan "sweep" per index k (k = 0..N-1): A_ij -= A_ik A_kj / A_kk for
 //     i,j != k, A_ik <- A_ik/A_kk, A_kk <- -1/A_kk.  Per step a thread does 64 independent DFMAs on its
-//     tile from 16 values broadcast through shared memory (8 LDS.128) and ONE __syncthreads: the
+//     tile from 16 values broadcast through shared memory (16 LDS.64) and ONE __syncthreads: the
 //     owners publish column k+1 (double buffered) as soon as their slice of it is updated.
 //     The pivots are exactly the Cholesky pivots L_kk^2, so logdet = sum log(pivot) and the
 //     leading-minor `info` follow LAPACK dpotrf; the border row gives a = K~^-1 r and the corner
@@ -44,23 +44,21 @@ __device__ int gpcc_prof_block;
 constexpr int TS = SMALL_TILE;  // 8
 constexpr double LOG2PI = 1.8378770664093454835606594728112;
 
-// Chunked layout of the per-point vectors in shared memory: [pair-of-rows part (4)][tile (<=32)][2], with a
-// compile-time part stride so that every address in the sweep loop is "per-thread base + immediate".
-constexpr int CS = 64;          // doubles per part (>= 2*SMALL_MAX_T)
-constexpr int VLEN = 4 * CS;    // doubles per vector
-__device__ __forceinline__ int cidx(int i) { return ((i & 7) >> 1) * CS + ((i >> 3) << 1) + (i & 1); }
+// Chunked layout of the per-point vectors in shared memory: [in-tile index (8)][tile (<=32)], with a compile-time part
+// stride so that every address in the sweep loop is "per-thread base + immediate".  No two values that one thread reads
+// are adjacent, so every access is a 64-bit LDS/STS: a 128-bit access needs an aligned quad of destination registers,
+// which ptxas cannot find among the 128 accumulator registers of the tile, and it lands the quad in scratch registers
+// and copies the values out (14-59 moves per sweep step with the former [pair of rows][tile][2] layout).
+constexpr int CS = 32;          // doubles per part (>= SMALL_MAX_T)
+constexpr int VLEN = 8 * CS;    // doubles per vector
+__device__ __forceinline__ int cidx(int i) { return (i & 7) * CS + (i >> 3); }
 __device__ __forceinline__ void load8(const double* buf, int tile, double (&out)[8]) {
 #pragma unroll
-    for (int part = 0; part < 4; ++part) {
-        const double2 v = *reinterpret_cast<const double2*>(buf + part * CS + 2 * tile);
-        out[2 * part] = v.x;
-        out[2 * part + 1] = v.y;
-    }
+    for (int r = 0; r < 8; ++r) out[r] = buf[r * CS + tile];
 }
 __device__ __forceinline__ void store8(double* buf, int tile, const double (&in)[8]) {
 #pragma unroll
-    for (int part = 0; part < 4; ++part)
-        *reinterpret_cast<double2*>(buf + part * CS + 2 * tile) = make_double2(in[2 * part], in[2 * part + 1]);
+    for (int r = 0; r < 8; ++r) buf[r * CS + tile] = in[r];
 }
 
 // shared-memory footprint of one evaluation (doubles, then Np ints)
@@ -132,20 +130,20 @@ __device__ __forceinline__ void publish(const double (&A)[8][8], int ti, int tj,
                                         double prn, bool fwd) {
     const bool pc = (tj == tkn), prw = (ti == tkn) && (!fwd || pc);   // forward-only mode: the row part is never read again
     if (pc) {
-        double* dst = nb + 2 * ti;
+        double* dst = nb + ti;
         if (prw) {  // diagonal tile: below the diagonal from the column, above it from the row
 #pragma unroll
-            for (int r = 0; r < 8; ++r) dst[(r >> 1) * CS + (r & 1)] = (r >= KKN) ? A[r][KKN] : A[KKN][r];
+            for (int r = 0; r < 8; ++r) dst[r * CS] = (r >= KKN) ? A[r][KKN] : A[KKN][r];
             *pivslot = A[KKN][KKN];
             *pslot = prn;
         } else {
 #pragma unroll
-            for (int r = 0; r < 8; ++r) dst[(r >> 1) * CS + (r & 1)] = A[r][KKN];
+            for (int r = 0; r < 8; ++r) dst[r * CS] = A[r][KKN];
         }
     } else if (prw) {
-        double* dst = nb + 2 * tj;
+        double* dst = nb + tj;
 #pragma unroll
-        for (int c = 0; c < 8; ++c) dst[(c >> 1) * CS + (c & 1)] = A[KKN][c];
+        for (int c = 0; c < 8; ++c) dst[c * CS] = A[KKN][c];
     }
 }
 
@@ -176,14 +174,14 @@ __device__ __forceinline__ void sweep_step(double (&A)[8][8], int ti, int tj, in
         for (int pp = 0; pp < 4; ++pp) {
             constexpr int P0 = KKN >> 1;
             const int part = (pp + P0) & 3;          // compile-time after unrolling
-            double2 x = *reinterpret_cast<const double2*>(cb + part * CS + 2 * ti);
+            double x0 = cb[2 * part * CS + ti], x1 = cb[(2 * part + 1) * CS + ti];
             if (part == (KK >> 1) && own_row) {      // row k of its owners becomes c/d
-                if (KK & 1) x.y -= 1.0; else x.x -= 1.0;
+                if (KK & 1) x1 -= 1.0; else x0 -= 1.0;
             }
 #pragma unroll
             for (int c = 0; c < 8; ++c) {
-                A[2 * part][c] = fma(-x.x, v[c], A[2 * part][c]);
-                A[2 * part + 1][c] = fma(-x.y, v[c], A[2 * part + 1][c]);
+                A[2 * part][c] = fma(-x0, v[c], A[2 * part][c]);
+                A[2 * part + 1][c] = fma(-x1, v[c], A[2 * part + 1][c]);
             }
             if (pp == 0) prn = fast_rcp(A[KKN][KKN]);   // final for this step; only the owner of the next pivot publishes it
         }
