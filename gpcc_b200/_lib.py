@@ -15,7 +15,7 @@ EXPORTS = [
     "gpcc_fit_state_predict", "gpcc_fit_state_predict_loglik", "gpcc_fit_state_factorisations",
     "gpcc_comm_unique_id", "gpcc_ctx_comm_init_rank", "gpcc_fit_state_sample", "gpcc_problem_set_method",
     "gpcc_ss_state_create", "gpcc_ss_state_destroy", "gpcc_ss_state_predict", "gpcc_ss_state_predict_loglik",
-    "gpcc_ss_sample",
+    "gpcc_ss_sample", "gpcc_ss_state_sample",
 ]
 
 
@@ -82,6 +82,7 @@ def load():
     lib.gpcc_ss_state_predict.argtypes = [vp, ip, dp, dp, dp]
     lib.gpcc_ss_state_predict_loglik.argtypes = [vp, ip, dp, dp, dp, dp, ip]
     lib.gpcc_ss_sample.argtypes = [vp, dp, dp, C.c_double, C.c_ulonglong, C.c_int, dp, dp, dp]
+    lib.gpcc_ss_state_sample.argtypes = [vp, ip, dp, C.c_ulonglong, C.c_int, dp, dp, dp]
     lib.gpcc_comm_unique_id.argtypes = [C.c_char_p]
     lib.gpcc_ctx_comm_init_rank.argtypes = [vp, C.c_int, C.c_int, C.c_char_p]
     for name in EXPORTS:

@@ -406,7 +406,8 @@ class StateSpaceFitState:
     """Fit state of the state-space method on the device (gpcc_ss_state_*): the filtered moments and the backward-pass adjoint
     of the N merged training points at (delays, alpha, rho), O(N) memory.  Answers the per-point form of `pred` (means and
     standard deviations) and the test log-likelihood; the full predictive covariance needs the dense `fit_state`.  The
-    state owns its data: it stays usable after its problem is closed."""
+    state owns its data: it stays usable after its problem is closed.  `sample` draws the test values jointly from the
+    predictive distribution, the route to any derived quantity without the full covariance."""
 
     def __init__(self, problem, delays, alpha, rho):
         self.problem = problem              # keeps the context alive
@@ -434,6 +435,32 @@ class StateSpaceFitState:
         ll, info = C.c_double(), C.c_int()
         check(_lib.load().gpcc_ss_state_predict_loglik(self._h, _i(nt), _d(tt), _d(yt), _d(st), C.byref(ll), C.byref(info)))
         return ll.value, info.value
+
+    def sample(self, ttest_per_band, seed, nsamples=1, z=None, return_z=False):
+        """Exact joint draws of the test values given the training data (gpcc_ss_state_sample), shape (nsamples, NT) with
+        the bands concatenated as `predict` returns them: distributed as N(mu, Sigma) of the dense pred(::Vector{Vector})
+        (:259-289), jitter included, in O(N + NT) per draw.  z (nsamples, (N+NT)(d+1) + L), d = 1, 2, 3 for OU, matern32,
+        matern52: per sample, the d process deviates and the noise deviate of every training point (input order) and
+        every test point (in the order of ttest_per_band), then the L shift deviates; used instead of the generator (seed
+        is then ignored).  return_z=True also returns the deviates used, in the same shape."""
+        nt, tt = self.problem._pack_test(ttest_per_band)
+        NT, ns = int(nt.sum()), int(nsamples)
+        d = {OU.kid: 1, matern32.kid: 2, matern52.kid: 3}.get(self.problem.kernel_id, 1)
+        zp, K = (self.problem.N + NT) * (d + 1), (self.problem.N + NT) * (d + 1) + self.L
+        zc = None
+        if z is not None:
+            z = _f64(z)
+            if z.shape != (ns, K):
+                raise GpccError(f"z must have shape (nsamples, (N+NT)(d+1) + L) = {(ns, K)}")
+            zc = _f64(np.concatenate([z[:, :zp].ravel(), z[:, zp:].ravel()]))
+        f = np.empty((max(ns, 0), NT))
+        zo = np.empty(max(ns, 0) * K) if return_z else None
+        check(_lib.load().gpcc_ss_state_sample(self._h, _i(nt), _d(tt), int(seed) & (2 ** 64 - 1), ns, _d(zc), _d(f),
+                                               _d(zo)))
+        if not return_z:
+            return f
+        zo = np.concatenate([zo[:ns * zp].reshape(ns, zp), zo[ns * zp:].reshape(ns, self.L)], axis=1)
+        return f, zo
 
     def pred(self, ttest, ytest=None, stest=None):
         """The reference's `pred` forms (:259-343) except the full covariance (Vector{Vector} form, and the nearestposdef

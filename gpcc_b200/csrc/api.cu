@@ -423,7 +423,7 @@ int fit_all(gpcc_problem* p, int M, const double* delays, int P, const double* t
 // =====================================================================================================
 extern "C" {
 
-int gpcc_version(void) { return 103; }   // 103: gpcc_ss_state_*, then gpcc_ss_sample (additive, same number); 102: gpcc_problem_set_method; 101: gpcc_stats grew by n_tau_cache and assembly_bytes
+int gpcc_version(void) { return 103; }   // 103: gpcc_ss_state_*, then gpcc_ss_sample and gpcc_ss_state_sample (additive, same number); 102: gpcc_problem_set_method; 101: gpcc_stats grew by n_tau_cache and assembly_bytes
 const char* gpcc_last_error(void) { return gpcc::last_error().c_str(); }
 
 int gpcc_fit_options_default(gpcc_fit_options* o) {
@@ -958,6 +958,8 @@ struct gpcc_ss_state {
     int dev = 0, kernel_id = 0, N = 0, L = 0, D = 0;
     SSProblem prior;                    // N, L, band_start, mu_b, Sigma_b of the training problem (no data pointers)
     std::vector<double> tr_t, tr_r, tr_s2;   // training data, each band sorted by t: merged with the test points of a call
+    std::vector<int> tr_ord;            // input index of every sorted training point (the deviates of gpcc_ss_state_sample)
+    std::vector<double> h_hyp;          // host copy of hyp
     double ll_train = 0.0;
     Stream stream;
     DevArray<double> hyp;               // delays [L], alpha [L], rho
@@ -967,6 +969,12 @@ struct gpcc_ss_state {
     // scratch of the calls, kept between calls
     DevArray<double> tt, mu, sd, mt, mr, ms2, ll;
     DevArray<int> bt, info;
+    // gpcc_ss_state_sample: the per-step records, built by its first call and kept (N (d^2 + D + 3) doubles + N ints), and
+    // the scratch of its calls (the prior sampler over the merged problem, one chunk of the mean passes)
+    DevArray<double> ps_rec;
+    DevArray<int> ps_in;
+    DevArray<double> ps_f, ps_z, ps_bs, ps_dv, ps_mbuf, ps_lbuf, ps_tw, ps_out, ps_step, ps_aggA, ps_aggc;
+    DevArray<int> ps_perm, ps_ints, ps_need, ps_mpos, ps_lpos, ps_tstep;
     ~gpcc_ss_state() { cudaSetDevice(dev); }
 };
 
@@ -981,13 +989,14 @@ int ss_state_create(gpcc_problem* p, const double* delays, const double* alpha, 
     s->dev = pd.dev; s->kernel_id = p->kernel_id; s->N = N; s->L = L; s->D = (int)D;
     s->prior = pd.ssp;
     s->prior.t = s->prior.r = s->prior.s2 = nullptr;
-    sort_bands(p, s->tr_t, s->tr_r, s->tr_s2);
+    sort_bands(p, s->tr_t, s->tr_r, s->tr_s2, &s->tr_ord);
     CUDA_TRY(create_stream(s->stream, 0));
     cudaStream_t st = s->stream.get();
     std::vector<double> h(2 * L + 1);
     std::memcpy(h.data(), delays, L * sizeof(double));
     std::memcpy(h.data() + L, alpha, L * sizeof(double));
     h[2 * L] = rho;
+    s->h_hyp = h;
     CUDA_TRY(s->hyp.reserve(h.size()));
     CUDA_TRY(s->st_t.reserve(N));
     CUDA_TRY(s->st_band.reserve(N));
@@ -1072,6 +1081,150 @@ int ss_test_points(const gpcc_ss_state* s, const int* ntest_per_band, const doub
             if (!std::isfinite(ttest[k])) return fail(-3, "non-finite test time");
             bt[k] = l;
         }
+    return 0;
+}
+
+// Records of gpcc_ss_state_sample (first call): the sorted training data go to the device for the rank and record kernels
+// only; the state keeps the records.
+int ss_post_records(gpcc_ss_state* s) {
+    const size_t N = (size_t)s->N;
+    cudaStream_t st = s->stream.get();
+    DevArray<double> t, r, s2;
+    DevArray<int> perm, order;
+    CUDA_TRY(t.reserve(N));
+    CUDA_TRY(r.reserve(N));
+    CUDA_TRY(s2.reserve(N));
+    CUDA_TRY(perm.reserve(N));
+    CUDA_TRY(order.reserve(N));
+    CUDA_TRY(s->ps_rec.reserve(N * statespace_post_record_width(s->kernel_id, s->L)));
+    CUDA_TRY(s->ps_in.reserve(N));
+    CUDA_TRY(cudaMemcpyAsync(t.d, s->tr_t.data(), N * sizeof(double), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(r.d, s->tr_r.data(), N * sizeof(double), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(s2.d, s->tr_s2.data(), N * sizeof(double), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(perm.d, s->tr_ord.data(), N * sizeof(int), cudaMemcpyHostToDevice, st));
+    SSProblem q = s->prior;
+    q.t = t.d; q.r = r.d; q.s2 = s2.d;
+    CUDA_TRY(statespace_post_records_launch(s->kernel_id, q, s->hyp.d, s->h_hyp.data(), s->st, perm.d, order.d, s->ps_rec.d,
+                                            s->ps_in.d, st));
+    CUDA_TRY(cudaStreamSynchronize(st));      // before the temporaries are freed
+    return 0;
+}
+
+constexpr size_t PS_CHUNK_BYTES = size_t(1) << 30;   // scratch of one chunk of samples of gpcc_ss_state_sample
+constexpr unsigned PS_STREAM_TAG = 0x53535053u;      // "SSPS": apart from gpcc_ss_sample's "SSMP" and the dense "GPCC"
+
+// gpcc_ss_state_sample after its checks.  The merged problem of the prior draw: per band the sorted training points and the
+// sorted test points, training first on ties (as gpcc_ss_state_predict_loglik merges them), test points with sigma^2 = 1e-8;
+// its input indices are the training input order, then N + the test input order.
+int ss_state_sample(gpcc_ss_state* s, const int* ntest_per_band, const double* ttest, const std::vector<int>& bt,
+                    unsigned long long seed, int nsamples, const double* z_in, double* out_f, double* out_z) {
+    const int L = s->L, N = s->N, NT = (int)bt.size(), NM = N + NT;
+    const int d = s->kernel_id == GPCC_KERNEL_OU ? 1 : s->kernel_id == GPCC_KERNEL_MATERN32 ? 2 : 3, D = d + L;
+    const size_t zp = (size_t)NM * (d + 1);             // point deviates per sample
+    std::vector<double> mt(NM), ms2(NM);
+    std::vector<int> mperm(NM);
+    SSProblem q = s->prior;
+    q.N = NM;
+    std::vector<size_t> ord;
+    size_t k = 0, first = 0;
+    for (int l = 0; l < L; ++l) {
+        const size_t nt = (size_t)ntest_per_band[l];
+        ord.resize(nt);
+        for (size_t i = 0; i < nt; ++i) ord[i] = first + i;
+        std::stable_sort(ord.begin(), ord.end(), [&](size_t a, size_t b) { return ttest[a] < ttest[b]; });
+        q.band_start[l] = (int)k;
+        size_t a = s->prior.band_start[l], b = 0;
+        const size_t ae = s->prior.band_start[l + 1];
+        while (a < ae || b < nt) {
+            if (b == nt || (a < ae && s->tr_t[a] <= ttest[ord[b]])) {
+                mt[k] = s->tr_t[a]; ms2[k] = s->tr_s2[a]; mperm[k] = s->tr_ord[a]; ++a;
+            } else {
+                const size_t j = ord[b++];
+                mt[k] = ttest[j]; ms2[k] = 1e-8; mperm[k] = N + (int)j;
+            }
+            ++k;
+        }
+        first += nt;
+    }
+    q.band_start[L] = (int)k;
+
+    CUDA_TRY(cudaSetDevice(s->dev));
+    cudaStream_t st = s->stream.get();
+    if (!s->ps_rec.d) {
+        int rc = ss_post_records(s);
+        if (rc) return rc;
+    }
+    // samples per chunk: the per-sample scratch of the prior draw and of the mean passes within PS_CHUNK_BYTES
+    const size_t tiles = ((size_t)NM + 63) / 64;
+    const size_t per = (size_t)NM + (z_in || out_z ? zp + L : 0) + L + (size_t)N + 2 * (size_t)NT * D + NT + tiles * d;
+    const int C = (int)std::max<size_t>(1, std::min<size_t>((size_t)nsamples, PS_CHUNK_BYTES / (per * sizeof(double))));
+    size_t n_step, n_aggA, n_aggc;
+    statespace_sample_scratch(s->kernel_id, NM, C, n_step, n_aggA, n_aggc);
+    CUDA_TRY(s->mt.reserve(NM));
+    CUDA_TRY(s->ms2.reserve(NM));
+    CUDA_TRY(s->ps_perm.reserve(NM));
+    CUDA_TRY(s->ps_ints.reserve(2 * (size_t)NM));
+    CUDA_TRY(s->ps_step.reserve(n_step));
+    CUDA_TRY(s->ps_aggA.reserve(n_aggA));
+    CUDA_TRY(s->ps_aggc.reserve(n_aggc));
+    CUDA_TRY(s->ps_f.reserve((size_t)C * NM));
+    if (z_in || out_z) CUDA_TRY(s->ps_z.reserve((size_t)C * (zp + L)));
+    CUDA_TRY(s->ps_bs.reserve((size_t)C * L));
+    CUDA_TRY(s->ps_dv.reserve((size_t)C * N));
+    CUDA_TRY(s->ps_mbuf.reserve((size_t)C * NT * D));
+    CUDA_TRY(s->ps_lbuf.reserve((size_t)C * NT * D));
+    CUDA_TRY(s->ps_out.reserve((size_t)C * NT));
+    CUDA_TRY(s->ps_tw.reserve((size_t)NT * 2 * D));
+    CUDA_TRY(s->ps_tstep.reserve(NT));
+    CUDA_TRY(s->ps_need.reserve(N));
+    CUDA_TRY(s->ps_mpos.reserve(N));
+    CUDA_TRY(s->ps_lpos.reserve(N));
+    CUDA_TRY(s->tt.reserve(NT));
+    CUDA_TRY(s->bt.reserve(NT));
+    CUDA_TRY(cudaMemcpyAsync(s->mt.d, mt.data(), NM * sizeof(double), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(s->ms2.d, ms2.data(), NM * sizeof(double), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(s->ps_perm.d, mperm.data(), NM * sizeof(int), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(s->tt.d, ttest, NT * sizeof(double), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(s->bt.d, bt.data(), NT * sizeof(int), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemsetAsync(s->ps_need.d, 0, N * sizeof(int), st));
+    q.t = s->mt.d; q.s2 = s->ms2.d; q.r = nullptr;
+    CUDA_TRY(statespace_post_locate_launch(s->kernel_id, s->prior, s->hyp.d, s->st, NT, s->tt.d, s->bt.d, s->ps_tstep.d,
+                                           s->ps_tw.d, s->ps_need.d, st));
+    SSSampleArgs sa;
+    for (int l = 0; l < L; ++l) { sa.tau[l] = s->h_hyp[l]; sa.alpha[l] = s->h_hyp[L + l]; }
+    sa.rho = s->h_hyp[2 * L]; sa.seed = seed; sa.tag = PS_STREAM_TAG; sa.perm = s->ps_perm.d; sa.f = s->ps_f.d;
+    SSSampleScratch sc{s->ps_ints.d, s->ps_ints.d + NM, s->ps_step.d, s->ps_aggA.d, s->ps_aggc.d};
+    SSPostArgs pa;
+    pa.N = N; pa.NT = NT; pa.NM = NM; pa.L = L; pa.seed = seed; pa.tag = PS_STREAM_TAG;
+    for (int l = 0; l < L; ++l) { pa.mub[l] = s->prior.mub[l]; pa.sqrt_sigmab[l] = std::sqrt(s->prior.Sigmab[l]); }
+    pa.rec = s->ps_rec.d; pa.in = s->ps_in.d; pa.band = s->st.band;
+    pa.tstep = s->ps_tstep.d; pa.tw = s->ps_tw.d; pa.bt = s->bt.d; pa.need = s->ps_need.d;
+    pa.mpos = s->ps_mpos.d; pa.lpos = s->ps_lpos.d; pa.f = s->ps_f.d; pa.bs = s->ps_bs.d; pa.dv = s->ps_dv.d;
+    pa.mbuf = s->ps_mbuf.d; pa.lbuf = s->ps_lbuf.d; pa.out = s->ps_out.d;
+    for (int s0 = 0; s0 < nsamples; s0 += C) {
+        const int c = std::min(C, nsamples - s0);
+        double* zb = (z_in || out_z) ? s->ps_z.d + (size_t)c * zp : nullptr;    // [c][L] after the [c][NM][d+1] points
+        if (z_in) {
+            CUDA_TRY(cudaMemcpyAsync(s->ps_z.d, z_in + (size_t)s0 * zp, (size_t)c * zp * sizeof(double), cudaMemcpyHostToDevice, st));
+            CUDA_TRY(cudaMemcpyAsync(zb, z_in + (size_t)nsamples * zp + (size_t)s0 * L, (size_t)c * L * sizeof(double),
+                                     cudaMemcpyHostToDevice, st));
+        }
+        sa.nsamples = c; sa.sample0 = s0;
+        sa.zin = z_in ? s->ps_z.d : nullptr;
+        sa.zout = out_z && !z_in ? s->ps_z.d : nullptr;
+        CUDA_TRY(statespace_sample_launch(s->kernel_id, q, sa, sc, st));
+        pa.C = c; pa.sample0 = s0;
+        pa.zin_b = z_in ? zb : nullptr;
+        pa.zout_b = out_z && !z_in ? zb : nullptr;
+        CUDA_TRY(statespace_post_chunk_launch(s->kernel_id, pa, st));
+        CUDA_TRY(cudaMemcpyAsync(out_f + (size_t)s0 * NT, s->ps_out.d, (size_t)c * NT * sizeof(double), cudaMemcpyDeviceToHost, st));
+        if (out_z) {
+            CUDA_TRY(cudaMemcpyAsync(out_z + (size_t)s0 * zp, s->ps_z.d, (size_t)c * zp * sizeof(double), cudaMemcpyDeviceToHost, st));
+            CUDA_TRY(cudaMemcpyAsync(out_z + (size_t)nsamples * zp + (size_t)s0 * L, zb, (size_t)c * L * sizeof(double),
+                                     cudaMemcpyDeviceToHost, st));
+        }
+    }
+    CUDA_TRY(cudaStreamSynchronize(st));
     return 0;
 }
 
@@ -1180,6 +1333,26 @@ int gpcc_ss_state_predict_loglik(gpcc_ss_state* s, const int* ntest_per_band, co
     *out_ll = info ? -std::numeric_limits<double>::infinity() : ll - s->ll_train;
     if (out_info) *out_info = info;
     return 0;
+}
+
+int gpcc_ss_state_sample(gpcc_ss_state* s, const int* ntest_per_band, const double* ttest, unsigned long long seed, int nsamples,
+                         const double* z_in, double* out_f, double* out_z) {
+    std::vector<int> bt;
+    int rc = ss_test_points(s, ntest_per_band, ttest, bt);
+    if (rc) return rc;
+    if (nsamples < 1) return fail(-7, "nsamples < 1");
+    const size_t NT = bt.size();
+    if (NT == 0) return 0;
+    if (!out_f) return fail(-1, "NULL argument");
+    const size_t NM = (size_t)s->N + NT;
+    if (NM > (size_t)std::numeric_limits<int>::max()) return fail(-7, "too many test points for one call");
+    if (z_in) {
+        const size_t d = s->kernel_id == GPCC_KERNEL_OU ? 1 : s->kernel_id == GPCC_KERNEL_MATERN32 ? 2 : 3;
+        const size_t nz = (size_t)nsamples * (NM * (d + 1) + s->L);
+        for (size_t k = 0; k < nz; ++k)
+            if (!std::isfinite(z_in[k])) return fail(-8, "non-finite deviate in z_in");
+    }
+    return ss_state_sample(s, ntest_per_band, ttest, bt, seed, nsamples, z_in, out_f, out_z);
 }
 
 int gpcc_ss_sample(gpcc_problem* p, const double* delays, const double* alpha, double rho, unsigned long long seed, int nsamples,

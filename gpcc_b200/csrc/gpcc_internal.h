@@ -166,6 +166,8 @@ struct SSSampleArgs {
     double tau[MAX_BANDS] = {0}, alpha[MAX_BANDS] = {0}, rho = 0;
     unsigned long long seed = 0;
     int nsamples = 0;
+    int sample0 = 0;              // generator counter of sample s: sample0 + s (a caller that draws in chunks of samples)
+    unsigned tag = 0x53534D50u;   // generator stream: "SSMP" (gpcc_ss_sample), apart from the dense sampler's "GPCC" (predict.cu)
     const int* perm = nullptr;    // [N] input index of the point at each position of p's sorted per-band copy
     const double* zin = nullptr;  // [nsamples][N][d+1] deviates in input order, or NULL: Philox from (seed, sample, point)
     double* zout = nullptr;       // [nsamples][N][d+1] or NULL: the deviates used
@@ -183,6 +185,43 @@ void statespace_sample_scratch(int kernel_id, int N, int nsamples, size_t& n_ste
 // Five launches on `stream`: merged ranks, per-step factors, tile aggregates, scan of the aggregates, tile re-run.
 cudaError_t statespace_sample_launch(int kernel_id, const SSProblem& p, const SSSampleArgs& a, const SSSampleScratch& s,
                                      cudaStream_t stream);
+// order[k] = the sorted position (in p) of merged step k: the filter's merge at delays tau (host, [L]).
+cudaError_t statespace_rank_launch(const SSProblem& p, const double* tau, int* order, cudaStream_t stream);
+
+// ---- exact O(N) posterior draws of the state-space fit state (ss_post_sample.cu): pathwise conditioning ----
+// Doubles per merged training step of the records: A (d x d), gain k (D = d + L), 1 / S, alpha_l, residual.
+int statespace_post_record_width(int kernel_id, int L);
+// The records rec [N][width] and the input index in [N] of every merged training step, from the stored moments st of the fit
+// state at hyp (device) / h_tau (host delays).  p: the training problem, each band sorted, on the device; perm: its input
+// indices; order: [N] scratch.
+cudaError_t statespace_post_records_launch(int kernel_id, const SSProblem& p, const double* hyp, const double* h_tau,
+                                           const SSStore& st, const int* perm, int* order, double* rec, int* in,
+                                           cudaStream_t stream);
+// Per test point: tstep = the last training step at or before it (-1: none), tw [NT][2 D] = the weights c1, w of
+// ss::point_mean_weights; need[step] |= 1 (a test point reads its m), 2 (... its adjoint).  need must be zeroed before.
+cudaError_t statespace_post_locate_launch(int kernel_id, const SSProblem& p, const double* hyp, const SSStore& st, int NT,
+                                          const double* tt, const int* bt, int* tstep, double* tw, int* need,
+                                          cudaStream_t stream);
+struct SSPostArgs {               // one chunk of C samples (global indices sample0 ..), all pointers on the device
+    int N = 0, NT = 0, NM = 0, L = 0;    // training steps, test points, N + NT (the merged problem of the prior draw), bands
+    int C = 0, sample0 = 0;
+    unsigned long long seed = 0;
+    unsigned tag = 0;                    // generator stream of the shift deviates (counter word 3 = 2)
+    double mub[MAX_BANDS] = {0}, sqrt_sigmab[MAX_BANDS] = {0};
+    const double* rec = nullptr;  const int* in = nullptr;     // records (statespace_post_records_launch)
+    const int* band = nullptr;                                 // [N] band of every merged training step (SSStore::band)
+    const int* tstep = nullptr;   const double* tw = nullptr;  const int* bt = nullptr;   // statespace_post_locate_launch
+    const int* need = nullptr;
+    int* mpos = nullptr;  int* lpos = nullptr;   // [N] slot of each flagged step (written by the chunk with sample0 = 0)
+    const double* f = nullptr;    // [C][NM] prior draw of the merged problem, input order (training, then test points)
+    const double* zin_b = nullptr;  double* zout_b = nullptr;  // [C][L] shift deviates in / out, or NULL
+    double* bs = nullptr;         // [C][L] shift draws
+    double* dv = nullptr;         // [N][C] pseudo-residuals, then innovations
+    double* mbuf = nullptr;  double* lbuf = nullptr;          // [<= NT slots][D][C] m and lam~ at flagged steps
+    double* out = nullptr;        // [C][NT] draws, test input order
+};
+// Shift draws, pseudo-residuals, forward and backward mean passes, test points: five launches on `stream`.
+cudaError_t statespace_post_chunk_launch(int kernel_id, const SSPostArgs& a, cudaStream_t stream);
 
 // ---- posterior over candidates (posterior.cu): src/getprobabilities.jl:10-20 --------------------
 cudaError_t posterior_launch(int M, const double* d_ll, const double* d_logprior, double* d_out, cudaStream_t stream,

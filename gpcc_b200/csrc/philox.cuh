@@ -17,4 +17,14 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
     return c;
 }
 
+// Two standard normals from one Philox output (Box-Muller on two 53-bit uniforms in (0, 1)): the state-space samplers.
+__device__ __forceinline__ double2 box_muller(uint4 r) {
+    const double u1 = ((double)(((unsigned long long)(r.x >> 5) << 26) | (r.y >> 6)) + 0.5) * (1.0 / 9007199254740992.0);
+    const double u2 = ((double)(((unsigned long long)(r.z >> 5) << 26) | (r.w >> 6)) + 0.5) * (1.0 / 9007199254740992.0);
+    const double rad = sqrt(-2.0 * log(u1));
+    double sn, cs;
+    sincospi(2.0 * u2, &sn, &cs);
+    return make_double2(rad * cs, rad * sn);
+}
+
 }  // namespace gpcc

@@ -308,5 +308,37 @@ GPCC_HD inline void point_moments(const Coef<Dim<KID>::d>& c, int l, double a, d
     var -= wLw;
 }
 
+// The mean of point_moments as a linear function of the data, for the posterior draws of ss_post_sample.cu: with m and lam
+// as there (m the filtered mean of step i, lam the adjoint of step i+1; neither is read here), mean = c1'm - w'lam, where
+// c1 = T1'h (T1: A over dt1 on the f-block, identity on the b-block) and w = T2 P1 h (P1: P predicted over dt1, T2: A over
+// dt2); w = 0 when later is false.  c1 and w depend on the covariances only, so one pair serves every sample.  P is
+// overwritten with P1.
+template <int KID, int L>
+GPCC_HD inline void point_mean_weights(const Coef<Dim<KID>::d>& c, int l, double a,
+                                       double (&P)[(Dim<KID>::d + L) * (Dim<KID>::d + L + 1) / 2], double dt1, bool later,
+                                       double dt2, double (&c1)[Dim<KID>::d + L], double (&w)[Dim<KID>::d + L]) {
+    constexpr int d = Dim<KID>::d, D = d + L;
+    double A[d][d], Q[d][d], dA[d][d], dQ[d][d];
+    for (int i = 0; i < D; ++i) c1[i] = i < d ? (i == 0 ? a : 0.0) : (i == d + l ? 1.0 : 0.0);
+    if (dt1 > 0.0) {
+        step<KID, false>(c, dt1, A, Q, dA, dQ);
+        double m0[D];
+        for (int i = 0; i < D; ++i) m0[i] = 0.0;
+        predict_moments<d, D>(A, Q, m0, P);
+        for (int i = 0; i < d; ++i) c1[i] = a * A[0][i];
+    }
+    double u[D];
+    for (int i = 0; i < D; ++i) u[i] = fma(a, P[sym<D>(i, 0)], P[sym<D>(i, d + l)]);
+    for (int i = 0; i < D; ++i) w[i] = 0.0;
+    if (!later) return;
+    step<KID, false>(c, dt2, A, Q, dA, dQ);
+    for (int i = 0; i < D; ++i) {
+        double s = i < d ? 0.0 : u[i];
+        if (i < d)
+            for (int q = 0; q < d; ++q) s = fma(A[i][q], u[q], s);
+        w[i] = s;
+    }
+}
+
 }  // namespace ss
 }  // namespace gpcc

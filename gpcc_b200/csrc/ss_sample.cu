@@ -8,9 +8,9 @@
 // ss_model.h; C_k is ss::noise_factor (D_k = 0 gives C_k = 0: a tie adds no process noise).
 //
 // Deviates: point i (input order) of sample s owns d process deviates (they drive the step that arrives at i) and one noise
-// deviate, [s][i][d+1].  They come from the caller (z_in) or from Philox-4x32-10 with counter (i, s, "SSMP", call) and key =
-// seed, two Box-Muller normals per call: a draw depends only on (seed, s, i), not on the launch geometry, on nsamples or on
-// the delays (common random numbers across delays).
+// deviate, [s][i][d+1].  They come from the caller (z_in) or from Philox-4x32-10 with counter (i, sample0 + s, tag, call)
+// and key = seed, two Box-Muller normals per call: a draw depends only on (seed, sample, i), not on the launch geometry, on
+// nsamples or on the delays (common random numbers across delays).  gpcc_ss_sample uses the tag "SSMP" and sample0 = 0.
 //
 // The recurrence is a composition of affine maps (A_k, c_k = C_k w_k), evaluated as an inclusive scan per sample in three
 // kernels with a fixed association, so every draw is bitwise reproducible:
@@ -31,7 +31,6 @@ namespace {
 
 constexpr int TILE = 64;                      // merged steps per tile (phases 1 and 3); fixed, so results never depend on the card
 constexpr int SCAN = 256;                     // threads of the aggregate scan (phase 2)
-constexpr unsigned STREAM_TAG = 0x53534D50u;  // "SSMP": a counter stream apart from the dense sampler's "GPCC" (predict.cu)
 
 template <int KID> struct Rec {               // layout of one stored step: A (d x d), packed lower C, alpha, sigma
     static constexpr int d = ss::Dim<KID>::d, NC = d * (d + 1) / 2, W = d * d + NC + 2;
@@ -68,14 +67,9 @@ __device__ __forceinline__ void deviates(const SSSampleArgs& a, int N, int s, in
     const uint2 key = make_uint2((unsigned)a.seed, (unsigned)(a.seed >> 32));
 #pragma unroll
     for (int c = 0; 2 * c < DD; ++c) {
-        const uint4 r = philox4x32_10(make_uint4((unsigned)i, (unsigned)s, STREAM_TAG, (unsigned)c), key);
-        const double u1 = ((double)(((unsigned long long)(r.x >> 5) << 26) | (r.y >> 6)) + 0.5) * (1.0 / 9007199254740992.0);
-        const double u2 = ((double)(((unsigned long long)(r.z >> 5) << 26) | (r.w >> 6)) + 0.5) * (1.0 / 9007199254740992.0);
-        const double rad = sqrt(-2.0 * log(u1));
-        double sn, cs;
-        sincospi(2.0 * u2, &sn, &cs);
-        w[2 * c] = rad * cs;
-        if (2 * c + 1 < DD) w[2 * c + 1] = rad * sn;
+        const double2 g = box_muller(philox4x32_10(make_uint4((unsigned)i, (unsigned)(a.sample0 + s), a.tag, (unsigned)c), key));
+        w[2 * c] = g.x;
+        if (2 * c + 1 < DD) w[2 * c + 1] = g.y;
     }
 }
 
@@ -323,6 +317,14 @@ cudaError_t launch(const SSProblem& p, const SSSampleArgs& a, const SSSampleScra
 int state_dim(int kernel_id) { return kernel_id == K_OU ? 1 : kernel_id == K_M32 ? 2 : 3; }
 
 }  // namespace
+
+cudaError_t statespace_rank_launch(const SSProblem& p, const double* tau, int* order, cudaStream_t stream) {
+    if (p.N <= 0) return cudaSuccess;
+    SSSampleArgs a;
+    for (int l = 0; l < p.L; ++l) a.tau[l] = tau[l];
+    ss_rank_kernel<<<(p.N + 255) / 256, 256, 0, stream>>>(p, a, order);
+    return cudaGetLastError();
+}
 
 void statespace_sample_scratch(int kernel_id, int N, int nsamples, size_t& n_step, size_t& n_aggA, size_t& n_aggc) {
     const size_t d = (size_t)state_dim(kernel_id), tiles = ((size_t)N + TILE - 1) / TILE;

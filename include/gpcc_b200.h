@@ -84,8 +84,8 @@ typedef struct gpcc_stats {
                                    tiles imported from the last-band cache count read + written); pairs with ms_assembly      */
 } gpcc_stats;
 
-int         gpcc_version(void);   /* 103.  102 -> 103: gpcc_ss_state_* (additive); gpcc_ss_sample was added later under the same
-                                      number (additive: a caller that needs it looks the symbol up).  101 -> 102: gpcc_problem_set_method (additive).
+int         gpcc_version(void);   /* 103.  102 -> 103: gpcc_ss_state_* (additive); gpcc_ss_sample and gpcc_ss_state_sample were
+                                      added later under the same number (additive: a caller that needs one looks the symbol up).  101 -> 102: gpcc_problem_set_method (additive).
                                       100 -> 101: gpcc_stats grew by n_tau_cache and assembly_bytes (appended at the end);
                                       a caller built against 100 must be rebuilt before it calls gpcc_ctx_get_stats                */
 const char* gpcc_last_error(void);
@@ -130,8 +130,10 @@ int gpcc_problem_get_prior(const gpcc_problem* p, double* mub, double* Sigmab);
  *     Cholesky factor of K + Sobs;
  *   - gpcc_ss_state_create builds the O(N) fit state of this method (see below): predictive means, standard deviations
  *     and the test log-likelihood without a factorisation;
- *   - gpcc_ss_sample draws from N(0, K + Sobs) in O(N), the O(N) form of gpcc_fit_state_sample.
- * The full predictive covariance has no O(N) form and stays dense.
+ *   - gpcc_ss_sample draws from N(0, K + Sobs) in O(N), the O(N) form of gpcc_fit_state_sample;
+ *   - gpcc_ss_state_sample draws the test values jointly from the predictive distribution N(mu_pred, Sigma_pred) in
+ *     O(N + NT) per draw.
+ * The full predictive covariance has no O(N) form and stays dense; its joint draws do not need it.
  * Returns < 0 for a NULL problem, an unknown method, or rbf with GPCC_METHOD_STATESPACE.                              */
 int gpcc_problem_set_method(gpcc_problem* p, int method);
 
@@ -233,6 +235,20 @@ int gpcc_ss_state_predict(gpcc_ss_state* s, const int* ntest_per_band, const dou
  * for negative counts, non-finite times or values, or sigmatest < 0; NT = 0 gives out_ll = 0.                         */
 int gpcc_ss_state_predict_loglik(gpcc_ss_state* s, const int* ntest_per_band, const double* ttest, const double* ytest,
                                  const double* sigmatest, double* out_ll, int* out_info);
+/* Exact joint draws of the test values g*_j = alpha_l f(t*_j - tau_l) + b_l + eta_j (eta_j ~ N(0, 1e-8), the jitter) given
+ * the training data: out_f[nsamples][NT] ~ N(mu_pred, Sigma_pred) of pred(::Vector{Vector}) (:259-289), test points in the
+ * order of ttest (bands concatenated, any order within a band), in O(N + NT) time and memory per draw and no N x N or
+ * NT x NT matrix.  Pathwise conditioning: a joint prior draw over the N training and NT test times (the recurrence of
+ * gpcc_ss_sample over their merge) and of the shifts, corrected by the smoother mean of the residual of that draw with the
+ * state's own gains.  Deviates, one array [nsamples][N+NT][d+1] then [nsamples][L]: per sample the d process deviates and the
+ * noise deviate of every point (the training points in the problem's input order, then the test points in the order of
+ * ttest), then the L shift deviates (b_l = mu_b,l + sqrt(Sigma_b,l) zeta_l in the prior draw).  z_in (may be NULL) supplies
+ * them, and seed is then ignored; otherwise they come from Philox-4x32-10 + Box-Muller in a stream of their own and depend
+ * only on (seed, sample, slot), so a draw does not depend on nsamples.  out_z (may be NULL) receives the deviates used.
+ * Bitwise reproducible.  Returns -1 for a NULL argument, -3 for a non-finite test time, -5 for a negative count, -7 for
+ * nsamples < 1 or too many points, -8 for a non-finite value in z_in; NT = 0 writes nothing.                            */
+int gpcc_ss_state_sample(gpcc_ss_state* s, const int* ntest_per_band, const double* ttest, unsigned long long seed,
+                         int nsamples, const double* z_in, double* out_f, double* out_z);
 
 /* Exact draws f ~ N(0, K + Sobs) at (delays, alpha, rho) for a problem in GPCC_METHOD_STATESPACE, the distribution of
  * gpcc_fit_state_sample, in O(N) time and memory: the kernel's SDE recurrence over the merged, delay-shifted times, run as a
